@@ -2,6 +2,7 @@
 """bench.py — VB Gaussian-mixture hot path on B200: VB iterations/s as N*K point*components per second.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--config c2] [--scaling strong|weak] [--impl reference]
+                    [--dump-outputs DIR]
 
 One "step" = one VB iteration of `gaussianmixture.LearnModel.update_posterior` (reference
 _gaussianmixture.py:863-869): M-step + q(pi) update + E-step/statistics pass over all rows + ELBO + convergence
@@ -17,6 +18,7 @@ from the oracle/_ref archive that oracle/build_ref.py packs from /root/reference
 archive is missing) on the host cores, on a bounded sample of the same workload.
 """
 import argparse
+import atexit
 import contextlib
 import io
 import json
@@ -31,6 +33,7 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True      # the benchmark leaves the tree as the build left it (it may be read-only)
 
 METRIC = "VB iters/sec (N*K points*comps/s) GMM"
 UNIT = "point*comps/s"
@@ -119,6 +122,7 @@ class ClockSampler:
             self.proc = subprocess.Popen(
                 ["nvidia-smi", f"--query-gpu={self.Q}", "--format=csv,noheader,nounits", "-lms", "100",
                  "-i", str(self.gpu_index)], stdout=open(self.path, "w"), stderr=subprocess.DEVNULL)
+            atexit.register(self.proc.kill)     # a run that fails before stop() must not leave the sampler running
         except Exception:
             self.proc = None
 
@@ -239,6 +243,40 @@ def run_reference_arm(args):
         "gpu_launches": 0,
     }
     print(json.dumps(line), flush=True)
+
+
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def engine_outputs(eng, n_hist):
+    """What one timed step hands its caller, read back after the step: the posterior hyperparameters the M-step produced
+    (under LearnModel's attribute names), the statistics of the pass, the ELBO terms and the ELBO history of the run."""
+    p = eng.fetch_params()
+    o = eng.off["vlhist"]
+    return {"hn_alpha_vec": p["alpha"], "hn_m_vecs": p["m"], "hn_kappas": p["kappa"], "hn_nus": p["nu"],
+            "hn_w_mats": p["w"], "hn_w_mats_inv": p["winv"], "e_ln_pi_vec": p["e_ln_pi"],
+            "e_ln_lambda_dets": p["e_ln_lambda_dets"], "ln_b_hn_w_nus": p["ln_b"], "ns": p["ns"], "x_bar_vecs": p["x_bar"],
+            "s_mats": p["s_mats"], "vl_terms": p["vl_terms"], "vl_history": eng.state[o:o + n_hist].cpu().numpy()}
+
+
+def dump_plan(eng, n_hist, count):
+    """Which of `count` output sets shaped like `eng`'s (one per restart) --dump-outputs writes: all of them, or a fixed,
+    seeded sample of them when all would exceed DUMP_LIMIT_BYTES.  Decided from shapes alone, before the timed steps, so
+    every rank gets the same answer and an impossible dump fails before any timing."""
+    one = sum(np.asarray(a, dtype=np.float64).nbytes for a in engine_outputs(eng, n_hist).values())
+    fit = DUMP_LIMIT_BYTES // one
+    if fit < 1:
+        raise RuntimeError(f"--dump-outputs: one output set takes {one} bytes, over the {DUMP_LIMIT_BYTES}-byte limit")
+    if count <= fit:
+        return list(range(count))
+    return sorted(np.random.default_rng(0).choice(count, size=fit, replace=False).tolist())
+
+
+def dump_outputs(dirname, arrays):
+    """Writes every array as DIR/<name>.npy in float64."""
+    os.makedirs(dirname, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(dirname, name + ".npy"), np.ascontiguousarray(a, dtype=np.float64))
 
 
 def _rel(a, b):
@@ -407,6 +445,7 @@ def bench_restarts(args, world, rank, local_rank, device, group):
            for _ in range(args.steps)]
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     launches0 = sum(e.kernel_launches for e in members)
+    dumped = dump_plan(lead, warmup + args.steps, r_total) if args.dump_outputs else []
     barrier()
     e0.record()
     for s in range(args.steps):
@@ -415,6 +454,15 @@ def bench_restarts(args, world, rank, local_rank, device, group):
     e1.record()
     launches = sum(e.kernel_launches for e in members) - launches0
     barrier()
+    if args.dump_outputs:
+        outs = {f"restart{i}_{name}": a for i, e in zip(mine, members) if i in dumped
+                for name, a in engine_outputs(e, warmup + args.steps).items()}
+        if world > 1:                                   # every rank's restarts: the dump does not depend on the GPU count
+            parts = [None] * world if rank == 0 else None
+            dist.gather_object(outs, parts, dst=0)
+            outs = {k: v for part in parts for k, v in part.items()} if rank == 0 else None
+        if rank == 0:
+            dump_outputs(args.dump_outputs, outs)
     ms_total = torch.tensor([e0.elapsed_time(e1)], device=device, dtype=torch.float64)
     pass_ms = torch.tensor([np.mean([sum(a.elapsed_time(b) for a, b in step) for step in evs])], device=device,
                            dtype=torch.float64)                   # all sweeps of one step on this rank
@@ -518,7 +566,14 @@ def main():
                     help="restart mode (C5): this many restarts spread over the GPUs, X replicated (default 64 for --config c5)")
     ap.add_argument("--no-batch", action="store_true", help="restart mode: one sweep per restart (no bgmm_pass_batched)")
     ap.add_argument("--variant", default="auto", choices=["auto", "simple", "dmma", "f32", "large", "tf32", "direct"])
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last one computed as DIR/<name>.npy (float64); the inputs "
+                         "are seeded, so two builds run with the same arguments can be compared output for output")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of the device path; it does not apply to --impl reference")
     args.warmup = max(args.warmup, 0)
     if args.impl == "reference":
         run_reference_arm(args)
@@ -603,6 +658,8 @@ def main():
     pass_ev = [(torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)) for _ in range(args.steps)]
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     launches0 = eng.kernel_launches
+    if args.dump_outputs:
+        dump_plan(eng, warmup + args.steps, 1)
     barrier()
     e0.record()
     for i in range(args.steps):
@@ -614,6 +671,8 @@ def main():
     e1.record()
     launches = eng.kernel_launches - launches0
     barrier()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, engine_outputs(eng, warmup + args.steps))
     ms_total = torch.tensor([e0.elapsed_time(e1)], device=device, dtype=torch.float64)
     pass_ms = torch.tensor([np.mean([a.elapsed_time(b) for a, b in pass_ev])], device=device, dtype=torch.float64)
     if world > 1:

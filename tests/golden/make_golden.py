@@ -21,6 +21,8 @@ import scipy
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, os.path.dirname(os.path.dirname(HERE)))
+sys.path.insert(0, os.path.dirname(HERE))
+from conftest import save_golden  # noqa: E402
 from oracle.ref_loader import load_reference_gaussianmixture  # noqa: E402
 
 gm = load_reference_gaussianmixture()
@@ -129,8 +131,7 @@ def run_case(name, x, k, d, seed, fit_kwargs, prior_kwargs=None, latent_x=None, 
         payload["latent_onehot"] = model.estimate_latent_vars(latent_x, loss="0-1")
         payload["latent_r"] = np.array(model.estimate_latent_vars(latent_x, loss="squared"))
         payload["latent_ns_after"] = np.array(model.ns)
-    path = os.path.join(HERE, name + ".npz")
-    np.savez_compressed(path, **payload)
+    path = save_golden(name, payload)
     print(f"{name}: {len(rec.states)} states, {os.path.getsize(path) / 1024:.0f} KiB")
 
 

@@ -11,10 +11,16 @@ def _params():
 
 
 def test_host_gen_sample_and_gen_params_follow_the_reference_stream():
-    from oracle.ref_loader import load_reference_gaussianmixture, reference_available
-    if not reference_available():
-        pytest.skip("reference not available")
     from bayesml_b200 import gaussianmixture
+    from conftest import load_golden
+    from oracle.ref_loader import load_reference_gaussianmixture, reference_available
+    # stored: the c1_readme fixture's input rows are the reference GenModel's own sample (make_golden.py)
+    g = load_golden("c1_readme")
+    x, z = gaussianmixture.GenModel(c_num_classes=3, c_degree=2, mu_vecs=np.array([[-5., -5.], [0., 0.], [5., 5.]]),
+                                    seed=0).gen_sample(1000)
+    assert np.array_equal(x, g["x"]) and z.shape == (1000, 3)
+    if not reference_available():
+        return
     ref = load_reference_gaussianmixture()
     for seed in (0, 5):
         a, b = gaussianmixture.GenModel(3, 2, seed=seed, **_params()), ref.GenModel(3, 2, seed=seed, **_params())

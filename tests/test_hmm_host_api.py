@@ -61,8 +61,28 @@ def test_broadcast_and_overwrite():
     assert np.array_equal(m.hn_zeta_vecs, m.h0_zeta_vecs)
 
 
-@pytest.mark.skipif(not reference_available(), reason="/root/reference not present (GPU box)")
 def test_host_features_and_estimates_equal_reference(tmp_path):
+    # stored: priors, final hyperparameters, features and predictive parameters the reference produced (make_golden_hmm.py)
+    from conftest import load_golden
+    from test_hmm_oracle_golden import CASES, PRIOR
+    hn = ("hn_eta_vec", "hn_zeta_vecs", "hn_m_vecs", "hn_kappas", "hn_nus", "hn_w_mats")
+    pred = ("p_a_mat", "p_mu_vecs", "p_nus", "p_lambda_mats")
+    for name in CASES:
+        g = load_golden(name)
+        mine = hiddenmarkovnormal.LearnModel(int(g["K"]), int(g["D"]), **{f: g[f] for f in PRIOR})
+        for f in pred:                                   # prior-based, as the reference left them after its fit
+            assert np.allclose(getattr(mine, f), g["stale_" + f], rtol=1e-13, atol=1e-15), (name, f)
+        mine.set_hn_params(**{f: g["final_" + f] for f in hn})
+        # hn_w_mats_inv is inv(hn_w_mats) here but the M-step's own matrix in the fixture: it and its log-determinant
+        # terms are defined to cond * eps
+        w_rtol = max(1e-13, 16 * np.finfo(float).eps * float(np.max(np.linalg.cond(g["final_hn_w_mats"]))))
+        for f in ("hn_w_mats_inv", "_e_ln_lambda_dets", "_ln_b_hn_w_nus", "_ln_pi_tilde_vec", "_ln_a_tilde_mat"):
+            rtol = w_rtol if f in ("hn_w_mats_inv", "_e_ln_lambda_dets", "_ln_b_hn_w_nus") else 1e-13
+            assert np.allclose(getattr(mine, f), g["final_" + f], rtol=rtol, atol=1e-15), (name, f)
+        for f in pred:
+            assert np.allclose(getattr(mine, f), g["pred_" + f], rtol=1e-13, atol=1e-15), (name, f)
+    if not reference_available():
+        return
     hm = load_reference_module("hiddenmarkovnormal")
     rng = np.random.default_rng(2)
     a = rng.normal(size=(3, 2, 2))
