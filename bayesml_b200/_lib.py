@@ -101,6 +101,14 @@ def load():
     lib.bgmm_hmm_pass.argtypes = [vp, i64, i32, i32, vp, vp, vp, vp, vp, vp, vp, vp, vp, i32, i32, vp]
     lib.bgmm_hmm_viterbi.restype = i32
     lib.bgmm_hmm_viterbi.argtypes = [i64, i32, vp, vp, vp, vp, vp, vp, vp]
+    lib.bgmm_hmm_seq_plan.restype = i64
+    lib.bgmm_hmm_seq_plan.argtypes = [i64, i64, vp, vp, i64]
+    lib.bgmm_hmm_seq_workspace_doubles.restype = i64
+    lib.bgmm_hmm_seq_workspace_doubles.argtypes = [i32, i64, i64]
+    lib.bgmm_hmm_pass_seqs.restype = i32
+    lib.bgmm_hmm_pass_seqs.argtypes = [vp, i64, i32, i32, vp, vp, vp, vp, vp, vp, vp, vp, vp, i32, i32, vp, vp, vp]
+    lib.bgmm_hmm_viterbi_seqs.restype = i32
+    lib.bgmm_hmm_viterbi_seqs.argtypes = [i64, i32, vp, vp, vp, vp, vp, vp, vp, i64, vp]
     lib.bgmm_hmm_small.restype = i32
     lib.bgmm_hmm_small.argtypes = [i32, i32, vp, vp, i32, i32, f64, i32, vp]
     if lib.bgmm_abi_version() != ABI_VERSION:

@@ -18,10 +18,13 @@
 // Phase A costs K times phase C (N K^3 flops); everything is FP64 CUDA-core work on small per-state vectors: a group
 // of KP = 2^ceil(log2 K) lanes owns one chunk (32 / KP chunks per warp), state vectors are exchanged through a per-warp
 // shared-memory line (one STS + K/2 broadcast LDS.128 per step).  All sums are in a fixed order (deterministic).
+// Several independent sequences (bgmm_hmm_pass_seqs): every sequence is cut into its own chunks (ScanPlan.coff), so no
+// recursion meets a restart inside a chunk; phase B is segmented per sequence and the windows are clamped to it.
 #include "bgmm_common.cuh"
 #include "bgmm_mma.cuh"
 #include <math.h>
 #include <stdlib.h>
+#include <type_traits>
 
 namespace bgmm {
 
@@ -36,6 +39,7 @@ struct ScanPlan {
     int K, L, nch;
     int window_cap;      // longest warm-up window the mixing mode may use (0 disables it); env BGMM_HMM_WINDOW_CAP
 };
+
 
 // Chunk length: <= 4096 chunks (the length of the sequential phase B), at least 32 elements each.
 __host__ __device__ inline int hmm_chunk_len(int64_t n) {
@@ -97,6 +101,46 @@ struct ScanBufs {
     double* seq2;          // two-level sweep: group matrices [72][K][K], log scales [72][K], boundary vectors [72][K]
 };
 
+// Several sequences (bgmm_hmm_pass_seqs): chunk c covers elements [coff[c], coff[c+1]) of the sequence [sst[c], sen[c]);
+// chunks never cross a sequence start.  The scan kernels take it as a trailing argument of type SeqArg<SEQS>, empty for
+// one sequence (chunk c = [cL, min(cL + L, n))), so the one-sequence instantiations keep the single-sequence arguments.
+struct SeqTable {
+    const int64_t* coff;
+    const int64_t* sst;
+    const int64_t* sen;
+    double* pg0;           // [nch][K] gamma at the first element of chunks that start a sequence
+};
+struct NoSeqTable {};
+template <bool SEQS> using SeqArg = typename std::conditional<SEQS, SeqTable, NoSeqTable>::type;
+
+struct ChunkInfo {
+    int64_t i0, i1;      // the chunk's elements [i0, i1)
+    int64_t s0, s1;      // its sequence's elements [s0, s1)
+};
+// The scan kernels are instantiated twice: SEQS = false is the one-sequence code (chunk c = [cL, min(cL + L, n)), the
+// expressions of the single-sequence path), SEQS = true reads the chunk table through chunk_info.
+__device__ __forceinline__ ChunkInfo chunk_info(const ScanPlan& sp, const SeqTable& T, int c) {
+    ChunkInfo ci;
+    if (c >= sp.nch) c = sp.nch - 1;                 // idle lane groups past the last chunk: the table ends there
+    ci.i0 = T.coff[c];
+    ci.i1 = T.coff[c + 1];
+    ci.s0 = T.sst[c];
+    ci.s1 = T.sen[c];
+    return ci;
+}
+// steps a warp's recursion loop runs: the chunk length, or (several sequences) the longest live chunk of the warp
+__device__ __forceinline__ int warp_steps(bool live, const ChunkInfo& ci) {
+    return (int)__reduce_max_sync(0xffffffffu, live ? (unsigned)(ci.i1 - ci.i0) : 0u);
+}
+// pi~ = exp(ln pi~ - max) (:849), component kk
+__device__ __forceinline__ double pi_tilde(const double* st, const Layout& L, int K, int kk) {
+    const volatile int* ctrl = reinterpret_cast<const volatile int*>(st + L.ctrl);
+    const double* Pc = st + L.params[ctrl[BGMM_CTRL_CUR]];
+    double pmax = -INFINITY;
+    for (int k = 0; k < K; ++k) pmax = fmax(pmax, Pc[L.p_elnpi + k]);
+    return kk < K ? exp(Pc[L.p_elnpi + kk] - pmax) : 0.0;
+}
+
 __device__ __forceinline__ const double* current_at(const double* st, const Layout& L, const double* hst, const HmmLayout& H) {
     const volatile int* ctrl = reinterpret_cast<const volatile int*>(st + L.ctrl);
     return hst + H.set[ctrl[BGMM_CTRL_CUR]] + H.s_at;
@@ -127,10 +171,10 @@ __device__ __forceinline__ int hmm_window(const double* st, const Layout& L, con
 }
 
 // MODE 0: phase C (exact recursion from the boundary vector);  1: phase A (K basis runs per chunk; skipped in mixing mode)
-template <int KP, int MODE>
+template <int KP, int MODE, bool SEQS>
 __global__ void __launch_bounds__(HT) hmm_fwd_kernel(const ScanPlan sp, const double* __restrict__ st, const Layout L,
                                                      const double* __restrict__ hst, const HmmLayout H, const int force,
-                                                     const ScanBufs B) {
+                                                     const ScanBufs B, const SeqArg<SEQS> T) {
     __shared__ __align__(16) double lines[HW][2][32];
     const volatile int* ctrl = reinterpret_cast<const volatile int*>(st + L.ctrl);
     if (!force && ctrl[BGMM_CTRL_DONE]) return;
@@ -144,18 +188,26 @@ __global__ void __launch_bounds__(HT) hmm_fwd_kernel(const ScanPlan sp, const do
     const int64_t nitems = MODE == 1 ? (int64_t)(sp.nch - 1) * K : sp.nch;
     const int c = MODE == 1 ? (int)(item / K) : (int)item;
     const int j0 = MODE == 1 ? (int)(item - (int64_t)c * K) : 0;
-    const bool live = item < nitems, mine = live && kk < K;
+    ChunkInfo ci{};
+    if constexpr (SEQS) ci = chunk_info(sp, T, c);
+    // basis runs only for chunks followed by another chunk of the same sequence
+    const bool live = item < nitems && !(SEQS && MODE == 1 && ci.i1 == ci.s1), mine = live && kk < K;
+    if (SEQS && !__any_sync(0xffffffffu, live)) return;
     double acol[KP];
 #pragma unroll
     for (int j = 0; j < KP; ++j) acol[j] = (mine && j < K) ? at[j * K + kk] : 0.0;
     double a = 0.0;
-    if (mine) a = MODE == 1 ? (kk == j0 ? 1.0 : 0.0) : B.vb[(int64_t)c * K + kk];
-    const int64_t i0 = (int64_t)c * sp.L;
+    if (SEQS && MODE == 0 && ci.i0 == ci.s0) a = mine ? pi_tilde(st, L, K, kk) : 0.0;   // a sequence starts
+    else if (mine) a = MODE == 1 ? (kk == j0 ? 1.0 : 0.0) : B.vb[(int64_t)c * K + kk];
+    const int64_t i0 = SEQS ? ci.i0 : (int64_t)c * sp.L;
+    const int nst = SEQS ? warp_steps(live, ci) : sp.L;
     double slog = 0.0;
     // emission values are fetched two steps ahead of the dependent chain (which runs through `a` only)
-    auto RH = [&](int64_t i, int s) { return (mine && s < sp.L && i < sp.n) ? rhohat[i * K + kk] : 0.0; };
+    auto RH = [&](int64_t i, int s) {
+        return (mine && (SEQS ? i < ci.i1 : (s < sp.L && i < sp.n))) ? rhohat[i * K + kk] : 0.0;
+    };
     double rho_c = RH(i0, 0), rho_n = RH(i0 + 1, 1);
-    for (int s = 0; s < sp.L; ++s) {
+    for (int s = 0; s < nst; ++s) {
         const int64_t i = i0 + s;
         const double rho = rho_c;
         rho_c = rho_n;
@@ -163,11 +215,11 @@ __global__ void __launch_bounds__(HT) hmm_fwd_kernel(const ScanPlan sp, const do
         double* line = lines[warp][s & 1];
         publish<KP>(line, lane, a);
         const double dot = group_dot<KP>(line, grp * KP, acol);
-        const double u = rho * (i == 0 ? a : dot);                 // :1000 — the first element has no transition
+        const double u = rho * ((SEQS ? i == ci.s0 : i == 0) ? a : dot);   // :1000 — the first element has no transition
         if (BASIS) {
             // rhohat <= 1 with row maximum 1, so the vector shrinks by at most min(A~) per step: it is renormalised
             // every 8 steps only (and at the end: phase B relies on rows of T summing to one)
-            if ((s & 7) == 7 || s == sp.L - 1) {
+            if ((s & 7) == 7 || s == nst - 1) {
                 const double sum = group_sum<KP>(u);
                 if (live) {
                     if (!(sum > 0.0)) {
@@ -185,7 +237,7 @@ __global__ void __launch_bounds__(HT) hmm_fwd_kernel(const ScanPlan sp, const do
             }
         } else {
             const double sum = group_sum<KP>(u);                   // chat_i; c_i, 1 / chat_i and sum ln c_i: hmm_cs_kernel
-            if (live && i < sp.n) {
+            if (live && i < (SEQS ? ci.i1 : sp.n)) {
                 a = u / sum;
                 if (mine) B.alpha[i * K + kk] = a;
                 if (kk == 0) B.chat[i] = sum;
@@ -200,13 +252,17 @@ __global__ void __launch_bounds__(HT) hmm_fwd_kernel(const ScanPlan sp, const do
 
 // c_i = chat_i e^{max_i} (:1001-1004), 1 / chat_i and the chunk's sum of ln c_i (for -E ln q(z), :909): element-wise, kept
 // out of the sequential recursions.  One CTA per chunk, fixed-order block sum.
+template <bool SEQS>
 __global__ void __launch_bounds__(128) hmm_cs_kernel(const ScanPlan sp, const double* __restrict__ st, const Layout L,
-                                                     const int force, const ScanBufs B) {
+                                                     const int force, const ScanBufs B, const SeqArg<SEQS> T) {
     __shared__ double red[40];
     const volatile int* ctrl = reinterpret_cast<const volatile int*>(st + L.ctrl);
     if (!force && ctrl[BGMM_CTRL_DONE]) return;
     const int c = blockIdx.x;
-    const int64_t i0 = (int64_t)c * sp.L, i1 = i0 + sp.L < sp.n ? i0 + sp.L : sp.n;
+    ChunkInfo ci{};
+    if constexpr (SEQS) ci = chunk_info(sp, T, c);
+    const int64_t i0 = SEQS ? ci.i0 : (int64_t)c * sp.L;
+    const int64_t i1 = SEQS ? ci.i1 : (i0 + sp.L < sp.n ? i0 + sp.L : sp.n);
     double acc = 0.0;
     for (int64_t i = i0 + threadIdx.x; i < i1; i += 128) {
         const double ch = B.chat[i], mx = B.rowmax[i];
@@ -247,6 +303,12 @@ struct SeqLevel {
     double* lsg;           // [ngroups][K]    mode 1 output
     const double* vbg;     // [ngroups][K]    mode 3 input: the vector at the start of every group
 };
+// several sequences: the swept chunk range (a trailing kernel argument, empty for one sequence)
+struct SeqRange {
+    int cbase;             // modes 0, 1, 3: chunk index of the first chunk of the swept range
+    const int64_t* segs;   // mode 0: CTA b sweeps chunks [segs[2b], segs[2b] + segs[2b+1]) (cbase, nsteps unused); or NULL
+};
+template <bool SEQS> using SeqRangeArg = typename std::conditional<SEQS, SeqRange, NoSeqTable>::type;
 __device__ __forceinline__ void cp_async16(double* smem_dst, const double* gsrc) {
     const unsigned d = (unsigned)__cvta_generic_to_shared(smem_dst);
     asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"(d), "l"(gsrc) : "memory");
@@ -261,10 +323,10 @@ __host__ __device__ inline int seq_batch(int K) {
     return b > 64 ? 64 : (b < 1 ? 1 : b);
 }
 
-template <int KP, bool FWD>
+template <int KP, bool FWD, bool SEQS>
 __global__ void __launch_bounds__(SEQ_T) hmm_seq_kernel(const ScanPlan sp, const double* __restrict__ st, const Layout L,
                                                         const double* __restrict__ hst, const HmmLayout H,
-                                                        const int force, const SeqLevel lv) {
+                                                        const int force, const SeqLevel lv, const SeqRangeArg<SEQS> R) {
     extern __shared__ __align__(16) double sq[];
     __shared__ __align__(16) double lines[2][32];
     const volatile int* ctrl = reinterpret_cast<const volatile int*>(st + L.ctrl);
@@ -273,16 +335,31 @@ __global__ void __launch_bounds__(SEQ_T) hmm_seq_kernel(const ScanPlan sp, const
     const int K = sp.K, KK = K * K, tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
     const int nb_chunk = seq_batch(K);
     const int stride = KK + K + 8;                       // per chunk: matrix [K][K] | e [K] | {exp(max), ...}
+    int cb = 0, nsteps_all = lv.nsteps;                  // the swept chunk range: [cb, cb + nsteps_all]
+    if constexpr (SEQS) {
+        cb = R.cbase;
+        if (R.segs != nullptr) {                         // segmented sweep: one sequence per CTA
+            cb = (int)R.segs[2 * blockIdx.x];
+            nsteps_all = (int)R.segs[2 * blockIdx.x + 1] - 1;
+        }
+    }
     // this CTA's range of sequential positions [s_lo, s_lo + nsteps): everything (modes 0, 2) or one group (modes 1, 3)
     const int grp = (lv.mode == 1 || lv.mode == 3) ? (int)blockIdx.x : 0;
     const int s_lo = grp * SEQ_GLEN;
-    const int nsteps = (lv.mode == 1 || lv.mode == 3) ? min(SEQ_GLEN, lv.nsteps - s_lo) : lv.nsteps;
+    const int nsteps = (lv.mode == 1 || lv.mode == 3) ? min(SEQ_GLEN, (SEQS ? nsteps_all : lv.nsteps) - s_lo)
+                                                      : (SEQS ? nsteps_all : lv.nsteps);
     const int nbatch = (nsteps + nb_chunk - 1) / nb_chunk;
-    const int n_items = lv.nsteps + 1;                   // chunks (modes 0, 1, 3) or groups + 1 (mode 2) along the sweep
+    const int n_items = (SEQS ? nsteps_all : lv.nsteps) + 1;   // chunks (modes 0, 1, 3) or groups + 1 (mode 2) along the sweep
     const bool mine = lane < K;
     // item (chunk / group) handled at sequential position s, and the item whose vector that step produces
-    auto chunk_of = [&](int s) { return (FWD || lv.mode == 2) ? s : n_items - 1 - s; };
-    auto out_of = [&](int s) { return (FWD || lv.mode == 2) ? s + 1 : n_items - 2 - s; };
+    auto chunk_of = [&](int s) {
+        const int q = (FWD || lv.mode == 2) ? s : n_items - 1 - s;
+        return SEQS ? cb + q : q;
+    };
+    auto out_of = [&](int s) {
+        const int q = (FWD || lv.mode == 2) ? s + 1 : n_items - 2 - s;
+        return SEQS ? cb + q : q;
+    };
     double a = 0.0, lsacc = 0.0;
     if (warp == 0) {
         if (lv.mode == 1) {
@@ -422,10 +499,10 @@ __global__ void __launch_bounds__(SEQ_T) hmm_seq_kernel(const ScanPlan sp, const
 // Otherwise (phase C'): from the boundary vector w[c]; gamma, the xi sum S[j][k] = sum_i alpha_{i-1}[j] rho_i[k]
 // beta_i[k] / c_i (A~ is applied once at the end), sum gamma ln rho, gamma_0, optionally beta.
 // MODE as in hmm_fwd_kernel (0: phase C', 1: phase A')
-template <int KP, int MODE>
+template <int KP, int MODE, bool SEQS>
 __global__ void __launch_bounds__(HT) hmm_bwd_kernel(const ScanPlan sp, const double* __restrict__ st, const Layout L,
                                                      double* __restrict__ hst, const HmmLayout H, const int force,
-                                                     const ScanBufs B) {
+                                                     const ScanBufs B, const SeqArg<SEQS> T) {
     __shared__ __align__(16) double lines[HW][2][32];
     const volatile int* ctrl = reinterpret_cast<const volatile int*>(st + L.ctrl);
     if (!force && ctrl[BGMM_CTRL_DONE]) return;
@@ -442,7 +519,11 @@ __global__ void __launch_bounds__(HT) hmm_bwd_kernel(const ScanPlan sp, const do
     const int64_t nitems = MODE == 1 ? (int64_t)(sp.nch - 1) * K : sp.nch;
     const int c = MODE == 1 ? 1 + (int)(item / K) : (int)item;          // basis runs: chunks 1 .. nch-1
     const int j0 = MODE == 1 ? (int)(item % K) : 0;
-    const bool live = item < nitems, mine = live && kk < K;
+    ChunkInfo ci{};
+    if constexpr (SEQS) ci = chunk_info(sp, T, c);
+    // basis runs only for chunks preceded by another chunk of the same sequence
+    const bool live = item < nitems && !(SEQS && MODE == 1 && ci.i0 == ci.s0), mine = live && kk < K;
+    if (SEQS && !__any_sync(0xffffffffu, live)) return;
     double arow[KP], srow[BASIS ? 1 : KP];
 #pragma unroll
     for (int k = 0; k < KP; ++k) arow[k] = (mine && k < K) ? at[kk * K + k] : 0.0;
@@ -450,10 +531,12 @@ __global__ void __launch_bounds__(HT) hmm_bwd_kernel(const ScanPlan sp, const do
 #pragma unroll
         for (int k = 0; k < KP; ++k) srow[k] = 0.0;
     }
-    const int64_t i0 = (int64_t)c * sp.L;
-    const int64_t i1 = (i0 + sp.L < sp.n ? i0 + sp.L : sp.n) - 1;        // last element of the chunk
+    const int64_t i0 = SEQS ? ci.i0 : (int64_t)c * sp.L;
+    const int64_t i1 = (SEQS ? ci.i1 : (i0 + sp.L < sp.n ? i0 + sp.L : sp.n)) - 1;   // last element of the chunk
+    const int nst = SEQS ? warp_steps(live, ci) : sp.L;
     double b = 0.0;
-    if (mine) b = MODE == 1 ? (kk == j0 ? 1.0 : 0.0) : B.vb[(int64_t)c * K + kk];
+    if (SEQS && MODE == 0 && ci.i1 == ci.s1) b = mine ? 1.0 : 0.0;       // a sequence ends (:939)
+    else if (mine) b = MODE == 1 ? (kk == j0 ? 1.0 : 0.0) : B.vb[(int64_t)c * K + kk];
     double slog = 0.0, gl = 0.0;
     // loads run two steps ahead, exp / reciprocal one step ahead of the dependent chain (which runs through b only)
     auto LR = [&](int64_t i) { return (!BASIS && mine && i >= i0) ? lnrho[i * K + kk] : 0.0; };
@@ -463,7 +546,7 @@ __global__ void __launch_bounds__(HT) hmm_bwd_kernel(const ScanPlan sp, const do
     double lr_c = LR(i1), rho_c = RH(i1), inv_c = CI(i1);
     double lr_n = LR(i1 - 1), rho_n = RH(i1 - 1), ci_n = CI(i1 - 1);
     double al_c = AL(i1), al_p = AL(i1 - 1), al_pp = AL(i1 - 2);
-    for (int s = 0; s < sp.L; ++s) {
+    for (int s = 0; s < nst; ++s) {
         const int64_t i = i1 - s;
         const bool in = live && i >= i0, on = mine && i >= i0;
         const double lr = lr_c, rho = rho_c, inv = inv_c, al = al_c, aprev = al_p;
@@ -476,13 +559,18 @@ __global__ void __launch_bounds__(HT) hmm_bwd_kernel(const ScanPlan sp, const do
             B.gamma[i * K + kk] = g;
             if (B.beta_out != nullptr) B.beta_out[i * K + kk] = b;
             gl = fma(g, lr, gl);
-            if (i == 0) hst[H.g0 + kk] = g;
+            if constexpr (!SEQS) {
+                if (i == 0) hst[H.g0 + kk] = g;
+            } else {
+                if (i == ci.s0) T.pg0[(int64_t)c * K + kk] = g;        // summed over sequence starts: hmm_reduce_kernel
+            }
         }
         double* line = lines[warp][s & 1];
         publish<KP>(line, lane, rb);
         const double dot = group_dot<KP>(line, grp * KP, arow);        // (A~ (rho o beta))[kk]
         if constexpr (!BASIS) {
-            const double f = (on && i >= 1) ? aprev * inv : 0.0;       // alpha_{i-1}[kk] / c_i   (:1017-1018)
+            // alpha_{i-1}[kk] / c_i (:1017-1018); xi = 0 at a (sequence) start
+            const double f = (on && (SEQS ? i > ci.s0 : i >= 1)) ? aprev * inv : 0.0;
             const double2* p = reinterpret_cast<const double2*>(line + grp * KP);
 #pragma unroll
             for (int k2 = 0; k2 < KP / 2; ++k2) {
@@ -535,10 +623,10 @@ __global__ void __launch_bounds__(HT) hmm_bwd_kernel(const ScanPlan sp, const do
 // The vector form above does the same 2 K^3 flops per element as K dependent mat-vec chains through shared memory
 // (12.4 of h2's 16.6 ms); this one is bound by the DMMA pipe.  Rows are renormalised every 8 steps (and at the end of a
 // forward chunk: phase B relies on rows summing to one), with the same zero-row rule as the vector kernels.
-template <int KP, bool FWD>
+template <int KP, bool FWD, bool SEQS>
 __global__ void __launch_bounds__(HT, KP >= 32 ? 1 : 4) hmm_basis_mma_kernel(const ScanPlan sp, const double* __restrict__ st, const Layout L,
                                                               const double* __restrict__ hst, const HmmLayout H,
-                                                              const int force, const ScanBufs B) {
+                                                              const int force, const ScanBufs B, const SeqArg<SEQS> T) {
     constexpr int NB = KP / 8;
     const volatile int* ctrl = reinterpret_cast<const volatile int*>(st + L.ctrl);
     if (!force && ctrl[BGMM_CTRL_DONE]) return;
@@ -547,6 +635,9 @@ __global__ void __launch_bounds__(HT, KP >= 32 ? 1 : 4) hmm_basis_mma_kernel(con
     const int64_t item = (int64_t)blockIdx.x * HW + warp;
     if (item >= sp.nch - 1) return;                               // whole warps only: no block barrier below
     const int c = FWD ? (int)item : 1 + (int)item;                // forward: chunks 0 .. nch-2, backward: 1 .. nch-1
+    ChunkInfo ci{};
+    if constexpr (SEQS) ci = chunk_info(sp, T, c);
+    if (SEQS && (FWD ? ci.i1 == ci.s1 : ci.i0 == ci.s0)) return;           // the sequence ends / starts here: no neighbour to feed
     const double* at = current_at(st, L, hst, H);
     const double* __restrict__ rhohat = B.rhohat;
     const double* __restrict__ ichat = B.ichat;
@@ -573,8 +664,8 @@ __global__ void __launch_bounds__(HT, KP >= 32 ? 1 : 4) hmm_basis_mma_kernel(con
                 sm[mb][nb][e] = (row == col && row < K) ? 1.0 : 0.0;
             }
     }
-    const int64_t i0 = (int64_t)c * sp.L;
-    const int64_t i1 = (i0 + sp.L < sp.n ? i0 + sp.L : sp.n) - 1;
+    const int64_t i0 = SEQS ? ci.i0 : (int64_t)c * sp.L;
+    const int64_t i1 = (SEQS ? ci.i1 : (i0 + sp.L < sp.n ? i0 + sp.L : sp.n)) - 1;
     const int nsteps = (int)(i1 - i0 + 1);
     // emission values (this lane's 2 NB columns) two steps ahead of the dependent chain
     auto load_rho = [&](int s, double (&dst)[NB][2]) {
@@ -599,7 +690,7 @@ __global__ void __launch_bounds__(HT, KP >= 32 ? 1 : 4) hmm_basis_mma_kernel(con
 #pragma unroll
             for (int e = 0; e < 2; ++e) { rho[nb][e] = rc[nb][e]; rc[nb][e] = rn[nb][e]; }
         load_rho(s + 2, rn);
-        const bool no_transition = FWD && i0 + s == 0;            // :1000 — the first element has no transition
+        const bool no_transition = FWD && i0 + s == (SEQS ? ci.s0 : 0);   // :1000 — the first element has no transition
 #pragma unroll
         for (int mb = 0; mb < NB; ++mb) {
             if (!FWD) {
@@ -667,10 +758,10 @@ __global__ void __launch_bounds__(HT, KP >= 32 ? 1 : 4) hmm_basis_mma_kernel(con
 //         reaches element 0, where the first element has no transition: then it is the exact recursion);
 //   !FWD: w[c] = beta at the last element e of chunk c, un-normalised run from ones over [e+1, e+W] (exact when the
 //         window reaches element N-1, where beta = 1, :939).
-template <int KP, bool FWD>
+template <int KP, bool FWD, bool SEQS>
 __global__ void __launch_bounds__(HT) hmm_window_kernel(const ScanPlan sp, const double* __restrict__ st, const Layout L,
                                                         double* hst, const HmmLayout H,
-                                                        const int force, const ScanBufs B) {
+                                                        const int force, const ScanBufs B, const SeqArg<SEQS> T) {
     __shared__ __align__(16) double lines[HW][2][32];
     const volatile int* ctrl = reinterpret_cast<const volatile int*>(st + L.ctrl);
     if (!force && ctrl[BGMM_CTRL_DONE]) return;
@@ -684,6 +775,14 @@ __global__ void __launch_bounds__(HT) hmm_window_kernel(const ScanPlan sp, const
     const double* __restrict__ chat = B.ichat;             // 1 / chat_i
     const int c = (int)(((int64_t)blockIdx.x * HW + warp) * G + grp);
     const bool live = c < sp.nch, mine = live && kk < K;
+    ChunkInfo ci{};
+    if constexpr (SEQS) ci = chunk_info(sp, T, c);
+    // a chunk that starts (FWD) / ends (!FWD) its sequence takes the exact vector there, pi~ / ones: no window to run
+    const bool edge = SEQS ? (FWD ? ci.i0 == ci.s0 : ci.i1 == ci.s1) : (FWD && c == 0);
+    if (SEQS && !__any_sync(0xffffffffu, live && !edge)) {
+        if (mine) B.vb[(int64_t)c * K + kk] = FWD ? pi_tilde(st, L, K, kk) : 1.0;
+        return;
+    }
     double av[KP];                                          // FWD: column kk of A~;  !FWD: row kk
 #pragma unroll
     for (int j = 0; j < KP; ++j) av[j] = (mine && j < K) ? (FWD ? at[j * K + kk] : at[kk * K + j]) : 0.0;
@@ -695,10 +794,11 @@ __global__ void __launch_bounds__(HT) hmm_window_kernel(const ScanPlan sp, const
         double pmax = -INFINITY;
         for (int k = 0; k < K; ++k) pmax = fmax(pmax, Pc[L.p_elnpi + k]);
         const double pt = (kk < K) ? exp(Pc[L.p_elnpi + kk] - pmax) : 0.0;      // pi~ (:849)
-        const int64_t end = (int64_t)c * sp.L - 1;          // last element before chunk c
-        const int64_t first = end - 8 * (int64_t)WB + 1;    // first element of the window (may be < 0)
-        double a = mine ? (first <= 0 ? pt : 1.0) : 0.0;
-        auto RH = [&](int64_t i) { return (mine && i >= 0 && i <= end) ? rhohat[i * K + kk] : 0.0; };
+        const int64_t S = SEQS ? ci.s0 : 0;                 // the window is clamped to the chunk's sequence
+        const int64_t end = (SEQS ? ci.i0 : (int64_t)c * sp.L) - 1;   // last element before chunk c
+        const int64_t first = end - 8 * (int64_t)WB + 1;    // first element of the window (may be < S)
+        double a = mine ? (first <= S ? pt : 1.0) : 0.0;
+        auto RH = [&](int64_t i) { return (mine && i >= S && i <= end) ? rhohat[i * K + kk] : 0.0; };
         double rc[8], rn[8];
 #pragma unroll
         for (int t = 0; t < 8; ++t) rn[t] = RH(first + t);
@@ -716,8 +816,8 @@ __global__ void __launch_bounds__(HT) hmm_window_kernel(const ScanPlan sp, const
                 double* line = lines[warp][t & 1];
                 publish<KP>(line, lane, a);
                 const double dot = group_dot<KP>(line, grp * KP, av);
-                const double u = rc[t] * (i == 0 ? a : dot);
-                const bool on = live && i >= 0;
+                const double u = rc[t] * (i == S ? a : dot);
+                const bool on = live && i >= S;
                 if (t == 7) {
                     const double sum = group_sum<KP>(u);
                     if (on) a = u / sum;
@@ -726,13 +826,14 @@ __global__ void __launch_bounds__(HT) hmm_window_kernel(const ScanPlan sp, const
                 }
             }
         }
-        if (mine) B.vb[(int64_t)c * K + kk] = (c == 0) ? pt : a;
+        if (mine) B.vb[(int64_t)c * K + kk] = edge ? pt : a;
     } else {
-        const int64_t e = ((int64_t)(c + 1) * sp.L < sp.n ? (int64_t)(c + 1) * sp.L : sp.n) - 1;   // last element of chunk c
-        const int64_t top = e + 8 * (int64_t)WB;            // first element visited (may be > N-1)
+        const int64_t e = (SEQS ? ci.i1 : ((int64_t)(c + 1) * sp.L < sp.n ? (int64_t)(c + 1) * sp.L : sp.n)) - 1;   // last element of chunk c
+        const int64_t S1 = SEQS ? ci.s1 : sp.n;             // end of its sequence: the window is clamped there
+        const int64_t top = e + 8 * (int64_t)WB;            // first element visited (may be > S1-1)
         double b = mine ? 1.0 : 0.0;
-        auto RH = [&](int64_t i) { return (mine && i > e && i < sp.n) ? rhohat[i * K + kk] : 0.0; };
-        auto CI = [&](int64_t i) { return (live && i > e && i < sp.n) ? chat[i] : 1.0; };
+        auto RH = [&](int64_t i) { return (mine && i > e && i < S1) ? rhohat[i * K + kk] : 0.0; };
+        auto CI = [&](int64_t i) { return (live && i > e && i < S1) ? chat[i] : 1.0; };
         double rc[8], rn[8], ic[8], cn[8];
 #pragma unroll
         for (int t = 0; t < 8; ++t) { rn[t] = RH(top - t); cn[t] = CI(top - t); }
@@ -747,7 +848,7 @@ __global__ void __launch_bounds__(HT) hmm_window_kernel(const ScanPlan sp, const
 #pragma unroll
             for (int t = 0; t < 8; ++t) {
                 const int64_t i = ib - t;
-                const bool on = live && i > e && i < sp.n;
+                const bool on = live && i > e && i < S1;
                 double* line = lines[warp][t & 1];
                 publish<KP>(line, lane, on ? rc[t] * b : 0.0);
                 const double dot = group_dot<KP>(line, grp * KP, av);
@@ -759,9 +860,11 @@ __global__ void __launch_bounds__(HT) hmm_window_kernel(const ScanPlan sp, const
 }
 
 // ms[j][k] = A~[j][k] * sum_c S_c[j][k] (:839 with :1017), sc[0] = sum_i ln c_i, sc[1] = sum gamma ln rho; fixed order.
+// SEQS: also G0 = sum over the sequence starts of gamma there.
+template <bool SEQS>
 __global__ void __launch_bounds__(256) hmm_reduce_kernel(const ScanPlan sp, const double* __restrict__ st, const Layout L,
                                                          double* __restrict__ hst, const HmmLayout H, const int force,
-                                                         const ScanBufs B) {
+                                                         const ScanBufs B, const SeqArg<SEQS> T) {
     __shared__ double part[8][32];
     const volatile int* ctrl = reinterpret_cast<const volatile int*>(st + L.ctrl);
     if (!force && ctrl[BGMM_CTRL_DONE]) return;
@@ -774,6 +877,11 @@ __global__ void __launch_bounds__(256) hmm_reduce_kernel(const ScanPlan sp, cons
         for (int c = sl; c < sp.nch; c += 8) acc += B.plc[c];
     } else if (e == KK + 1) {
         for (int c = sl; c < sp.nch; c += 8) acc += B.pgl[c];
+    } else if (SEQS && e < KK + 2 + sp.K) {
+        if constexpr (SEQS) {
+            for (int c = sl; c < sp.nch; c += 8)
+                if (T.coff[c] == T.sst[c]) acc += T.pg0[(int64_t)c * sp.K + (e - KK - 2)];
+        }
     }
     part[sl][threadIdx.x & 31] = acc;
     __syncthreads();
@@ -783,12 +891,11 @@ __global__ void __launch_bounds__(256) hmm_reduce_kernel(const ScanPlan sp, cons
         if (e < KK) hst[H.ms + e] = at[e] * t;
         else if (e == KK) hst[H.sc + 0] = t;
         else if (e == KK + 1) hst[H.sc + 1] = t;
+        else if (SEQS && e < KK + 2 + sp.K) hst[H.g0 + (e - KK - 2)] = t;
     }
 }
 
-static int64_t scan_ws_doubles(int K, int64_t n) {
-    const int L = hmm_chunk_len(n);
-    const int64_t nch = (n + L - 1) / L;
+static int64_t scan_ws_doubles(int K, int64_t n, int64_t nch) {
     const int64_t KK = (int64_t)K * K;
     // transfer matrices + log scales + boundary vectors + S partials + the two scalar partial arrays
     // + rhohat [n][K], row max [n], chat [n]
@@ -797,40 +904,68 @@ static int64_t scan_ws_doubles(int K, int64_t n) {
 }
 
 // Phase B of one direction: the single-CTA sweep, or (>= 4 groups of SEQ_GLEN steps) group matrices -> group sweep -> expansion
-template <int KP, bool FWD>
-static void launch_seq(const ScanPlan& sp, double* st, const Layout& L, double* hst, const HmmLayout& H, int force,
-                       const ScanBufs& B, size_t smem_seq, cudaStream_t stream) {
-    const int K = sp.K, nsteps = sp.nch - 1;
-    const int ngroups = (nsteps + SEQ_GLEN - 1) / SEQ_GLEN;
+static int hmm_two_level() {
     static const int two_level = [] { const char* e = getenv("BGMM_HMM_TWO_LEVEL"); return (e == nullptr || atoi(e) != 0) ? 1 : 0; }();
+    return two_level;
+}
+
+// the sweep over chunks [cbase, cbase + nsteps] (cbase = 0 unless SEQS)
+template <int KP, bool FWD, bool SEQS>
+static void launch_seq(const ScanPlan& sp, double* st, const Layout& L, double* hst, const HmmLayout& H, int force,
+                       const ScanBufs& B, size_t smem_seq, cudaStream_t stream, int cbase, int nsteps) {
+    const int K = sp.K;
+    const int ngroups = (nsteps + SEQ_GLEN - 1) / SEQ_GLEN;
+    const int two_level = hmm_two_level();
     SeqLevel lv{0, nsteps, ngroups, B.tf, B.ls, B.vb, nullptr, nullptr, nullptr};
+    SeqRangeArg<SEQS> R{};
+    if constexpr (SEQS) R = SeqRange{cbase, nullptr};
     if (!two_level || ngroups < 4) {
-        hmm_seq_kernel<KP, FWD><<<1, SEQ_T, smem_seq, stream>>>(sp, st, L, hst, H, force, lv);
+        hmm_seq_kernel<KP, FWD, SEQS><<<1, SEQ_T, smem_seq, stream>>>(sp, st, L, hst, H, force, lv, R);
         return;
     }
     double* tg = B.seq2;                                   // [ngroups][K][K]
     double* lsg = tg + (int64_t)72 * K * K;                // [ngroups][K]
     double* vbg = lsg + (int64_t)72 * K;                   // [ngroups + 1][K]
     lv.mode = 1; lv.tg = tg; lv.lsg = lsg;
-    hmm_seq_kernel<KP, FWD><<<dim3(ngroups, K), SEQ_T, smem_seq, stream>>>(sp, st, L, hst, H, force, lv);
-    SeqLevel l2{2, ngroups - 1, ngroups, tg, lsg, vbg, nullptr, nullptr, nullptr};      // the last group's matrix is not needed
-    hmm_seq_kernel<KP, FWD><<<1, SEQ_T, smem_seq, stream>>>(sp, st, L, hst, H, force, l2);
+    hmm_seq_kernel<KP, FWD, SEQS><<<dim3(ngroups, K), SEQ_T, smem_seq, stream>>>(sp, st, L, hst, H, force, lv, R);
+    SeqLevel l2{2, ngroups - 1, ngroups, tg, lsg, vbg, nullptr, nullptr, nullptr};   // the last group's matrix is not needed
+    hmm_seq_kernel<KP, FWD, SEQS><<<1, SEQ_T, smem_seq, stream>>>(sp, st, L, hst, H, force, l2, SeqRangeArg<SEQS>{});   // group level: cbase 0
     lv.mode = 3; lv.tg = nullptr; lv.lsg = nullptr; lv.vbg = vbg;
-    hmm_seq_kernel<KP, FWD><<<ngroups, SEQ_T, smem_seq, stream>>>(sp, st, L, hst, H, force, lv);
+    hmm_seq_kernel<KP, FWD, SEQS><<<ngroups, SEQ_T, smem_seq, stream>>>(sp, st, L, hst, H, force, lv, R);
 }
 
-template <int KP>
+// Phase B of one direction over several sequences: sequences of one chunk need none; the others are swept in parallel
+// (one CTA each, segmented), except those long enough for the two-level sweep, which get it one after another.
+// plan: see bgmm_hmm_seq_plan.
+template <int KP, bool FWD>
+static void launch_seq_segs(const ScanPlan& sp, double* st, const Layout& L, double* hst, const HmmLayout& H, int force,
+                            const ScanBufs& B, size_t smem_seq, cudaStream_t stream, const int64_t* plan,
+                            const int64_t* segs_dev) {
+    const int64_t nshort = plan[4], nlong = plan[5];
+    const int64_t* segs = plan + 8 + 3 * plan[3] + 1;
+    if (nshort > 0) {
+        SeqLevel lv{0, 0, 0, B.tf, B.ls, B.vb, nullptr, nullptr, nullptr};
+        hmm_seq_kernel<KP, FWD, true><<<(unsigned)nshort, SEQ_T, smem_seq, stream>>>(sp, st, L, hst, H, force, lv,
+                                                                                     SeqRange{0, segs_dev});
+    }
+    for (int64_t q = nshort; q < nshort + nlong; ++q)
+        launch_seq<KP, FWD, true>(sp, st, L, hst, H, force, B, smem_seq, stream, (int)segs[2 * q], (int)segs[2 * q + 1] - 1);
+}
+
+// plan: NULL for one sequence, else the host copy of bgmm_hmm_seq_plan's table (segs_dev: its segment list on the device)
+template <int KP, bool SEQS>
 static int launch_scan(const ScanPlan& sp, double* st, const Layout& L, double* hst, const HmmLayout& H, int force,
-                       const ScanBufs& B, cudaStream_t stream) {
+                       const ScanBufs& B, const SeqArg<SEQS>& T, cudaStream_t stream, const int64_t* plan,
+                       const int64_t* segs_dev) {
     constexpr int G = 32 / KP;
     const int per_cta = HW * G;
     const int64_t nbasis = (int64_t)(sp.nch - 1) * sp.K;
     const unsigned gb = (unsigned)((nbasis + per_cta - 1) / per_cta), gc = (unsigned)((sp.nch + per_cta - 1) / per_cta);
     const size_t smem_seq = (size_t)2 * seq_batch(sp.K) * (sp.K * sp.K + sp.K + 8) * sizeof(double);
     {   // per launch: the attribute is per device
-        cudaError_t e = cudaFuncSetAttribute(hmm_seq_kernel<KP, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 208 * 1024);
+        cudaError_t e = cudaFuncSetAttribute(hmm_seq_kernel<KP, true, SEQS>, cudaFuncAttributeMaxDynamicSharedMemorySize, 208 * 1024);
         if (e == cudaSuccess)
-            e = cudaFuncSetAttribute(hmm_seq_kernel<KP, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 208 * 1024);
+            e = cudaFuncSetAttribute(hmm_seq_kernel<KP, false, SEQS>, cudaFuncAttributeMaxDynamicSharedMemorySize, 208 * 1024);
         if (e != cudaSuccess) return check_cuda(e, "cudaFuncSetAttribute(hmm_seq)");
     }
     // boundary vectors: either {basis runs, sequential sweep} or {one warm-up window per chunk}; the device decides
@@ -838,22 +973,27 @@ static int launch_scan(const ScanPlan& sp, double* st, const Layout& L, double* 
     const char* env_mma = getenv("BGMM_HMM_BASIS_MMA");                    // 0: the vector basis runs (tests compare the two)
     const int basis_mma = (env_mma == nullptr || atoi(env_mma) != 0) ? 1 : 0;
     const unsigned gm = (unsigned)((sp.nch - 1 + HW - 1) / HW);          // tensor-pipe basis runs: one warp per chunk
-    if (sp.nch > 1) {
-        if (KP >= 2 && basis_mma) hmm_basis_mma_kernel<(KP >= 8 ? KP : 8), true><<<gm, HT, 0, stream>>>(sp, st, L, hst, H, force, B);
-        else hmm_fwd_kernel<KP, 1><<<gb, HT, 0, stream>>>(sp, st, L, hst, H, force, B);
+    // basis runs and sweeps only where a sequence has more than one chunk
+    const bool multi = plan == nullptr ? sp.nch > 1 : plan[4] + plan[5] > 0;
+    if (multi) {
+        if (KP >= 2 && basis_mma) hmm_basis_mma_kernel<(KP >= 8 ? KP : 8), true, SEQS><<<gm, HT, 0, stream>>>(sp, st, L, hst, H, force, B, T);
+        else hmm_fwd_kernel<KP, 1, SEQS><<<gb, HT, 0, stream>>>(sp, st, L, hst, H, force, B, T);
     }
-    launch_seq<KP, true>(sp, st, L, hst, H, force, B, smem_seq, stream);
-    hmm_window_kernel<KP, true><<<gc, HT, 0, stream>>>(sp, st, L, hst, H, force, B);
-    hmm_fwd_kernel<KP, 0><<<gc, HT, 0, stream>>>(sp, st, L, hst, H, force, B);
-    hmm_cs_kernel<<<sp.nch, 128, 0, stream>>>(sp, st, L, force, B);
-    if (sp.nch > 1) {
-        if (KP >= 2 && basis_mma) hmm_basis_mma_kernel<(KP >= 8 ? KP : 8), false><<<gm, HT, 0, stream>>>(sp, st, L, hst, H, force, B);
-        else hmm_bwd_kernel<KP, 1><<<gb, HT, 0, stream>>>(sp, st, L, hst, H, force, B);
+    if (plan == nullptr) launch_seq<KP, true, false>(sp, st, L, hst, H, force, B, smem_seq, stream, 0, sp.nch - 1);
+    else launch_seq_segs<KP, true>(sp, st, L, hst, H, force, B, smem_seq, stream, plan, segs_dev);
+    hmm_window_kernel<KP, true, SEQS><<<gc, HT, 0, stream>>>(sp, st, L, hst, H, force, B, T);
+    hmm_fwd_kernel<KP, 0, SEQS><<<gc, HT, 0, stream>>>(sp, st, L, hst, H, force, B, T);
+    hmm_cs_kernel<SEQS><<<sp.nch, 128, 0, stream>>>(sp, st, L, force, B, T);
+    if (multi) {
+        if (KP >= 2 && basis_mma) hmm_basis_mma_kernel<(KP >= 8 ? KP : 8), false, SEQS><<<gm, HT, 0, stream>>>(sp, st, L, hst, H, force, B, T);
+        else hmm_bwd_kernel<KP, 1, SEQS><<<gb, HT, 0, stream>>>(sp, st, L, hst, H, force, B, T);
     }
-    launch_seq<KP, false>(sp, st, L, hst, H, force, B, smem_seq, stream);
-    hmm_window_kernel<KP, false><<<gc, HT, 0, stream>>>(sp, st, L, hst, H, force, B);
-    hmm_bwd_kernel<KP, 0><<<gc, HT, 0, stream>>>(sp, st, L, hst, H, force, B);
-    hmm_reduce_kernel<<<(sp.K * sp.K + 2 + 31) / 32, 256, 0, stream>>>(sp, st, L, hst, H, force, B);
+    if (plan == nullptr) launch_seq<KP, false, false>(sp, st, L, hst, H, force, B, smem_seq, stream, 0, sp.nch - 1);
+    else launch_seq_segs<KP, false>(sp, st, L, hst, H, force, B, smem_seq, stream, plan, segs_dev);
+    hmm_window_kernel<KP, false, SEQS><<<gc, HT, 0, stream>>>(sp, st, L, hst, H, force, B, T);
+    hmm_bwd_kernel<KP, 0, SEQS><<<gc, HT, 0, stream>>>(sp, st, L, hst, H, force, B, T);
+    const int nred = sp.K * sp.K + 2 + (SEQS ? sp.K : 0);
+    hmm_reduce_kernel<SEQS><<<(nred + 31) / 32, 256, 0, stream>>>(sp, st, L, hst, H, force, B, T);
     return check_cuda(cudaGetLastError(), "hmm scan launch");
 }
 
@@ -1059,7 +1199,84 @@ __global__ void __launch_bounds__(SEQ_T) hmm_viterbi_back_kernel(const int64_t n
     }
 }
 
+// Viterbi over several sequences: one warp per sequence (lane k owns state k and column k of ln a~), the recursion in the
+// same operation order as hmm_viterbi_fwd_kernel, restarted at every sequence start (omega = ln rho + ln pi~, phi = 0),
+// then lane 0 traces the path back from argmax omega at the sequence's last element.  Sequences run in parallel.
+template <int KP>
+__global__ void __launch_bounds__(128) hmm_viterbi_seqs_kernel(const int64_t n, const int K, const int64_t n_seqs,
+                                                               const int64_t* __restrict__ starts,
+                                                               const double* __restrict__ lnrho,
+                                                               const double* __restrict__ lnpi,
+                                                               const double* __restrict__ lna, double* __restrict__ omega,
+                                                               int32_t* __restrict__ phi, int32_t* __restrict__ path) {
+    __shared__ __align__(16) double lines[4][2][32];
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    const int64_t q = (int64_t)blockIdx.x * 4 + warp;
+    if (q >= n_seqs) return;
+    const int64_t s0 = starts[q], s1 = q + 1 < n_seqs ? starts[q + 1] : n;
+    const bool mine = lane < K;
+    double acol[KP];
+#pragma unroll
+    for (int j = 0; j < KP; ++j) acol[j] = (mine && j < K) ? lna[j * K + lane] : -INFINITY;
+    // ln rho two steps ahead of the dependent chain
+    auto LR = [&](int64_t i) { return (mine && i < s1) ? lnrho[i * K + lane] : 0.0; };
+    double lr_c = LR(s0), lr_n = LR(s0 + 1);
+    double om = mine ? lr_c + lnpi[lane] : -INFINITY;                   // :1469
+    if (mine) { omega[s0 * K + lane] = om; phi[s0 * K + lane] = 0; }
+    for (int64_t i = s0 + 1; i < s1; ++i) {
+        lr_c = lr_n;
+        lr_n = LR(i + 1);
+        double* line = lines[warp][i & 1];
+        line[lane] = om;
+        __syncwarp();
+        double best = -INFINITY;
+        int arg = 0;
+#pragma unroll
+        for (int j = 0; j < KP; ++j) {
+            if (j < K) {
+                const double cand = acol[j] + line[j];                   // ln a~[j][k] + omega_{i-1}[j]   (:1471-1472)
+                if (j == 0 || cand > best) { best = cand; arg = j; }
+            }
+        }
+        om = lr_c + best;
+        if (mine) { omega[i * K + lane] = om; phi[i * K + lane] = arg; }
+    }
+    __syncwarp();                                                       // phi of the whole sequence is visible to lane 0
+    if (lane == 0) {                                                    // :1474-1479
+        const double* o = omega + (s1 - 1) * K;
+        int z = 0;
+        double bv = o[0];
+        for (int k = 1; k < K; ++k)
+            if (o[k] > bv) { bv = o[k]; z = k; }
+        path[s1 - 1] = z;
+        for (int64_t i = s1 - 2; i >= s0; --i) {
+            z = phi[(i + 1) * K + z];
+            path[i] = z;
+        }
+    }
+}
+
 }  // namespace bgmm
+
+extern "C" int bgmm_hmm_viterbi_seqs(int64_t n, int K, const double* lnrho, const double* lnpi, const double* lna,
+                                     double* omega, int32_t* phi, int32_t* path, const int64_t* seq_starts, int64_t n_seqs,
+                                     void* stream) {
+    using namespace bgmm;
+    if (n <= 0 || K < 1 || K > 32 || n_seqs < 1 || n_seqs > n || lnrho == nullptr || lnpi == nullptr || lna == nullptr ||
+        omega == nullptr || phi == nullptr || path == nullptr || seq_starts == nullptr) {
+        set_error("bgmm_hmm_viterbi_seqs: bad argument (n=%lld K=%d n_seqs=%lld, K <= 32, 1 <= n_seqs <= n)", (long long)n,
+                  K, (long long)n_seqs);
+        return BGMM_EINVAL;
+    }
+    cudaStream_t s = (cudaStream_t)stream;
+    const unsigned g = (unsigned)((n_seqs + 3) / 4);
+    if (K <= 2) hmm_viterbi_seqs_kernel<2><<<g, 128, 0, s>>>(n, K, n_seqs, seq_starts, lnrho, lnpi, lna, omega, phi, path);
+    else if (K <= 4) hmm_viterbi_seqs_kernel<4><<<g, 128, 0, s>>>(n, K, n_seqs, seq_starts, lnrho, lnpi, lna, omega, phi, path);
+    else if (K <= 8) hmm_viterbi_seqs_kernel<8><<<g, 128, 0, s>>>(n, K, n_seqs, seq_starts, lnrho, lnpi, lna, omega, phi, path);
+    else if (K <= 16) hmm_viterbi_seqs_kernel<16><<<g, 128, 0, s>>>(n, K, n_seqs, seq_starts, lnrho, lnpi, lna, omega, phi, path);
+    else hmm_viterbi_seqs_kernel<32><<<g, 128, 0, s>>>(n, K, n_seqs, seq_starts, lnrho, lnpi, lna, omega, phi, path);
+    return check_cuda(cudaGetLastError(), "viterbi_seqs launch");
+}
 
 extern "C" int bgmm_hmm_viterbi(int64_t n, int K, const double* lnrho, const double* lnpi, const double* lna, double* omega,
                                 int32_t* phi, int32_t* path, void* stream) {
@@ -1092,17 +1309,86 @@ extern "C" int bgmm_hmm_viterbi(int64_t n, int K, const double* lnrho, const dou
 
 extern "C" int64_t bgmm_hmm_scan_workspace_doubles(int K, int64_t n) {
     if (K <= 0 || K > 32 || n <= 0) return 0;
-    return bgmm::scan_ws_doubles(K, n);
+    const int L = bgmm::hmm_chunk_len(n);
+    return bgmm::scan_ws_doubles(K, n, (n + L - 1) / L);
+}
+
+// Several sequences: every sequence is cut into chunks of hmm_chunk_len(n), the last one shorter, so there are at most
+// ceil(n / L) + n_seqs chunks; plus G0's per-chunk partials.
+extern "C" int64_t bgmm_hmm_seq_workspace_doubles(int K, int64_t n, int64_t n_seqs) {
+    if (K <= 0 || K > 32 || n <= 0 || n_seqs < 1 || n_seqs > n) return 0;
+    const int L = bgmm::hmm_chunk_len(n);
+    const int64_t nch = (n + L - 1) / L + n_seqs;
+    return bgmm::scan_ws_doubles(K, n, nch) + nch * K;
+}
+
+// The chunk table of bgmm_hmm_pass_seqs (int64):
+//   [0] n  [1] n_seqs  [2] L  [3] nch  [4] nshort  [5] nlong  [6] size  [7] 0
+//   coff[nch + 1] | sst[nch] | sen[nch] | segs[nshort + nlong][2] | starts[n_seqs]
+// chunk c = elements [coff[c], coff[c+1]) of the sequence [sst[c], sen[c]); segs = (first chunk, chunk count) of every
+// sequence with more than one chunk, those swept by one CTA (nshort) before those long enough for the two-level sweep.
+extern "C" int64_t bgmm_hmm_seq_plan(int64_t n, int64_t n_seqs, const int64_t* seq_starts, int64_t* plan, int64_t cap) {
+    using namespace bgmm;
+    if (n <= 0 || n_seqs < 1 || seq_starts == nullptr) {
+        set_error("bgmm_hmm_seq_plan: bad argument (n=%lld n_seqs=%lld)", (long long)n, (long long)n_seqs);
+        return BGMM_EINVAL;
+    }
+    if (seq_starts[0] != 0) { set_error("bgmm_hmm_seq_plan: seq_starts[0] must be 0"); return BGMM_EINVAL; }
+    const int64_t L = hmm_chunk_len(n);
+    int64_t nch = 0, nseg = 0;
+    for (int64_t q = 0; q < n_seqs; ++q) {
+        const int64_t a = seq_starts[q], b = q + 1 < n_seqs ? seq_starts[q + 1] : n;
+        if (!(b > a) || b > n) {
+            set_error("bgmm_hmm_seq_plan: seq_starts must increase strictly and stay below n (index %lld)", (long long)q);
+            return BGMM_EINVAL;
+        }
+        const int64_t m = (b - a + L - 1) / L;
+        nch += m;
+        nseg += m > 1;
+    }
+    const int64_t size = 8 + 3 * nch + 1 + 2 * nseg + n_seqs;
+    if (plan == nullptr || cap < size) return size;
+    int64_t* coff = plan + 8;
+    int64_t* sst = coff + nch + 1;
+    int64_t* sen = sst + nch;
+    int64_t* segs = sen + nch;
+    int64_t* starts = segs + 2 * nseg;
+    int64_t c = 0, ns = 0, nl = 0, nshort = 0;
+    const int two_level = hmm_two_level();
+    for (int64_t q = 0; q < n_seqs; ++q) {
+        const int64_t m = ((q + 1 < n_seqs ? seq_starts[q + 1] : n) - seq_starts[q] + L - 1) / L;
+        nshort += m > 1 && !(two_level && (m - 1 + SEQ_GLEN - 1) / SEQ_GLEN >= 4);
+    }
+    for (int64_t q = 0; q < n_seqs; ++q) {
+        const int64_t a = seq_starts[q], b = q + 1 < n_seqs ? seq_starts[q + 1] : n, m = (b - a + L - 1) / L;
+        if (m > 1) {
+            const bool lng = two_level && (m - 1 + SEQ_GLEN - 1) / SEQ_GLEN >= 4;
+            int64_t* sg = segs + 2 * (lng ? nshort + nl++ : ns++);
+            sg[0] = c;
+            sg[1] = m;
+        }
+        for (int64_t j = 0; j < m; ++j, ++c) {
+            coff[c] = a + j * L;
+            sst[c] = a;
+            sen[c] = b;
+        }
+        starts[q] = a;
+    }
+    coff[nch] = n;
+    plan[0] = n; plan[1] = n_seqs; plan[2] = L; plan[3] = nch; plan[4] = nshort; plan[5] = nseg - nshort;
+    plan[6] = size; plan[7] = 0;
+    return size;
 }
 
 extern "C" int bgmm_hmm_supported(int K, int D) {
     return (K >= 1 && K <= 32 && bgmm::large_supported(K, D, BGMM_F64)) ? 1 : 0;
 }
 
-extern "C" int bgmm_hmm_pass(const void* x, int64_t n, int K, int D, double* state, double* hst, double* workspace,
-                             double* scan_ws, double* lnrho, double* alpha, double* gamma, double* cs, double* beta_out,
-                             int mode, int force, void* stream) {
-    using namespace bgmm;
+namespace bgmm {
+// plan / plan_dev: NULL (one sequence), or bgmm_hmm_seq_plan's table on the host and the same table on the device
+static int hmm_pass(const void* x, int64_t n, int K, int D, double* state, double* hst, double* workspace, double* scan_ws,
+                    double* lnrho, double* alpha, double* gamma, double* cs, double* beta_out, int mode, int force,
+                    void* stream, const int64_t* plan, const int64_t* plan_dev) {
     if (!bgmm_hmm_supported(K, D)) {
         set_error("bgmm_hmm_pass: unsupported shape K=%d D=%d (float64, K <= 32, D <= 128)", K, D);
         return BGMM_ENOSUP;
@@ -1136,6 +1422,7 @@ extern "C" int bgmm_hmm_pass(const void* x, int64_t n, int K, int D, double* sta
     if (mode == BGMM_HMM_FULL) {
         ScanPlan sp;
         sp.n = n; sp.K = K; sp.L = hmm_chunk_len(n); sp.nch = (int)((n + sp.L - 1) / sp.L);
+        if (plan != nullptr) sp.nch = (int)plan[3];
         const char* wc = getenv("BGMM_HMM_WINDOW_CAP");          // tests / experiments: 0 forces the basis + sweep path
         sp.window_cap = wc != nullptr ? atoi(wc) : 16384;
         const int64_t KK = (int64_t)K * K, nch = sp.nch;
@@ -1149,6 +1436,13 @@ extern "C" int bgmm_hmm_pass(const void* x, int64_t n, int K, int D, double* sta
         B.rowmax = rmx;
         B.ichat = rmx + n;
         B.seq2 = reinterpret_cast<double*>((reinterpret_cast<uintptr_t>(B.ichat + n) + 15) & ~uintptr_t(15));   // cp.async 16
+        SeqTable T{nullptr, nullptr, nullptr, nullptr};
+        if (plan != nullptr) {
+            T.coff = plan_dev + 8;
+            T.sst = T.coff + sp.nch + 1;
+            T.sen = T.sst + sp.nch;
+            T.pg0 = B.seq2 + 72 * (KK + 2 * K);
+        }
         a.rhohat_out = rh; a.rowmax_out = rmx;
         rc = launch_emit_small(x, n, K, D, state, L, force, lnrho, rh, rmx, s);
         if (rc == -1) {
@@ -1156,15 +1450,40 @@ extern "C" int bgmm_hmm_pass(const void* x, int64_t n, int K, int D, double* sta
             rc = launch_pass_large_part(a, K, D, BGMM_F64, 1, s);
         }
         if (rc) return rc;
-        if (K <= 2) rc = launch_scan<2>(sp, state, L, hst, H, force, B, s);
-        else if (K <= 4) rc = launch_scan<4>(sp, state, L, hst, H, force, B, s);
-        else if (K <= 8) rc = launch_scan<8>(sp, state, L, hst, H, force, B, s);
-        else if (K <= 16) rc = launch_scan<16>(sp, state, L, hst, H, force, B, s);
-        else rc = launch_scan<32>(sp, state, L, hst, H, force, B, s);
+        const int64_t* segs_dev = plan != nullptr ? plan_dev + 8 + 3 * plan[3] + 1 : nullptr;
+#define BGMM_SCAN(KP) (plan != nullptr ? launch_scan<KP, true>(sp, state, L, hst, H, force, B, T, s, plan, segs_dev) \
+                                        : launch_scan<KP, false>(sp, state, L, hst, H, force, B, NoSeqTable{}, s, nullptr, nullptr))
+        if (K <= 2) rc = BGMM_SCAN(2);
+        else if (K <= 4) rc = BGMM_SCAN(4);
+        else if (K <= 8) rc = BGMM_SCAN(8);
+        else if (K <= 16) rc = BGMM_SCAN(16);
+        else rc = BGMM_SCAN(32);
+#undef BGMM_SCAN
         if (rc) return rc;
     }
     a.lnrho_only = 0;
     a.lnrho_out = nullptr;
     a.r_out = gamma;
     return launch_pass_large_part(a, K, D, BGMM_F64, 2, s);
+}
+}  // namespace bgmm
+
+extern "C" int bgmm_hmm_pass(const void* x, int64_t n, int K, int D, double* state, double* hst, double* workspace,
+                             double* scan_ws, double* lnrho, double* alpha, double* gamma, double* cs, double* beta_out,
+                             int mode, int force, void* stream) {
+    return bgmm::hmm_pass(x, n, K, D, state, hst, workspace, scan_ws, lnrho, alpha, gamma, cs, beta_out, mode, force, stream,
+                          nullptr, nullptr);
+}
+
+extern "C" int bgmm_hmm_pass_seqs(const void* x, int64_t n, int K, int D, double* state, double* hst, double* workspace,
+                                  double* scan_ws, double* lnrho, double* alpha, double* gamma, double* cs, double* beta_out,
+                                  int mode, int force, const int64_t* plan, const int64_t* plan_dev, void* stream) {
+    using namespace bgmm;
+    if (plan == nullptr || plan_dev == nullptr || plan[0] != n || plan[1] < 1 || plan[3] < plan[1] ||
+        plan[6] != 8 + 3 * plan[3] + 1 + 2 * (plan[4] + plan[5]) + plan[1] || plan[2] != hmm_chunk_len(n)) {
+        set_error("bgmm_hmm_pass_seqs: plan is NULL or not bgmm_hmm_seq_plan's table for n=%lld", (long long)n);
+        return BGMM_EINVAL;
+    }
+    return hmm_pass(x, n, K, D, state, hst, workspace, scan_ws, lnrho, alpha, gamma, cs, beta_out, mode, force, stream,
+                    plan, plan_dev);
 }

@@ -516,7 +516,10 @@ class HMMEngine(VBEngine):
 
     Reference call sites replaced (bayesml/hiddenmarkovnormal/_hiddenmarkovnormal.py): the VB loop :1102-1113 —
     `_update_q_mu_lambda`/`_update_q_pi`/`_update_q_a` -> bgmm_hmm_small, `_update_q_z` -> bgmm_hmm_pass, `_calc_vl`
-    and the convergence test -> bgmm_hmm_small; one sequence on one GPU (the recursions couple all elements)."""
+    and the convergence test -> bgmm_hmm_small; on one GPU (the recursions couple all elements of a sequence).
+
+    The loaded rows are one sequence, or (`set_sequences`) several independent sequences, concatenated, that share the
+    posterior: then the E-step and the Viterbi decode run through bgmm_hmm_pass_seqs / bgmm_hmm_viterbi_seqs."""
 
     def __init__(self, K, D, device=None):
         super().__init__(K, D, device=device, precision="float64", group=None, variant=_lib.PASS_LARGE)
@@ -526,6 +529,7 @@ class HMMEngine(VBEngine):
         self.hoff = _lib.hmm_layout(self.K)
         self.hst = torch.zeros(self.hoff["total"], dtype=torch.float64, device=self.device)
         self.lnrho_buf = self.alpha_buf = self.gamma_buf = self.cs_buf = self.beta_buf = self.scan_ws = None
+        self.seq_starts = self.plan = self.plan_dev = None
 
     def _hview(self, name, length, which=None):
         o = self.hoff[name] if which is None else self.hoff[f"set{which}"] + self.hoff[name]
@@ -540,7 +544,34 @@ class HMMEngine(VBEngine):
                 self.lnrho_buf, self.alpha_buf, self.gamma_buf, self.cs_buf = mk(n, K), mk(n, K), mk(n, K), mk(n)
                 self.scan_ws = mk(int(self.lib.bgmm_hmm_scan_workspace_doubles(K, n)))
             self.beta_buf = None
+        self.seq_starts = self.plan = self.plan_dev = None
         return self
+
+    def set_sequences(self, seq_starts):
+        """The loaded rows are the sequences starting at rows `seq_starts` (sorted, first 0), concatenated; None: one
+        sequence.  Builds the chunk table (bgmm_hmm_seq_plan) on the host and keeps a device copy for the E-steps."""
+        self.seq_starts = self.plan = self.plan_dev = None
+        if seq_starts is None:
+            return self
+        n, K = self.n_local, self.K
+        starts = np.ascontiguousarray(seq_starts, dtype=np.int64)
+        size = int(self.lib.bgmm_hmm_seq_plan(n, starts.size, starts.ctypes.data, None, 0))
+        if size < 0:
+            _lib.check(size, "bgmm_hmm_seq_plan")
+        plan = np.zeros(size, dtype=np.int64)
+        _lib.check(int(self.lib.bgmm_hmm_seq_plan(n, starts.size, starts.ctypes.data, plan.ctypes.data, size)) - size,
+                   "bgmm_hmm_seq_plan")
+        with torch.cuda.device(self.device):
+            self.plan_dev = torch.from_numpy(plan).to(self.device)
+            need = int(self.lib.bgmm_hmm_seq_workspace_doubles(K, n, starts.size))
+            if self.scan_ws.numel() < need:
+                self.scan_ws = torch.empty(need, dtype=torch.float64, device=self.device)
+        self.seq_starts, self.plan = starts, plan
+        return self
+
+    def _seq_starts_dev(self):
+        nch, nseg = int(self.plan[3]), int(self.plan[4] + self.plan[5])
+        return self.plan_dev[8 + 3 * nch + 1 + 2 * nseg:]
 
     def set_hmm_prior(self, eta0, zeta0, m0, kappa0, nu0, w0inv, ln_b_h0, ln_c_h0_eta, ln_c_h0_zeta_sum):
         self.set_prior(eta0, m0, kappa0, nu0, w0inv, ln_b_h0, ln_c_h0_eta)
@@ -560,6 +591,21 @@ class HMMEngine(VBEngine):
 
     def _pass(self, mode=_lib.HMM_FULL, force=0, beta_out=None):
         ptr = lambda t: 0 if t is None else t.data_ptr()  # noqa: E731
+        if self.plan is not None:
+            _lib.check(self.lib.bgmm_hmm_pass_seqs(self.x.data_ptr(), self.n_local, self.K, self.D, self.state.data_ptr(),
+                                                   self.hst.data_ptr(), self.workspace.data_ptr(), ptr(self.scan_ws),
+                                                   ptr(self.lnrho_buf), ptr(self.alpha_buf), ptr(self.gamma_buf),
+                                                   ptr(self.cs_buf), ptr(beta_out), mode, force, self.plan.ctypes.data,
+                                                   self.plan_dev.data_ptr(), self._stream()), "bgmm_hmm_pass_seqs")
+            self.passes += 1
+            # emission (3) + per direction {window, chunk kernel} + c + reduction + statistics (2); with sequences of more
+            # than one chunk also the basis runs and the sweeps: one segmented launch for the short sequences, a
+            # two-level sweep (3 launches) for every long one
+            nshort, nlong = int(self.plan[4]), int(self.plan[5])
+            sweeps = (1 if nshort else 0) + 3 * nlong
+            multi = 2 + 2 * sweeps if nshort + nlong else 0
+            self.kernel_launches += (11 + multi) if mode == _lib.HMM_FULL else 2
+            return
         _lib.check(self.lib.bgmm_hmm_pass(self.x.data_ptr(), self.n_local, self.K, self.D, self.state.data_ptr(),
                                           self.hst.data_ptr(), self.workspace.data_ptr(), ptr(self.scan_ws),
                                           ptr(self.lnrho_buf), ptr(self.alpha_buf), ptr(self.gamma_buf), ptr(self.cs_buf),
@@ -581,7 +627,8 @@ class HMMEngine(VBEngine):
                 gamma, ms = init
                 self.gamma_buf.copy_(torch.as_tensor(np.ascontiguousarray(gamma, dtype=np.float64)))
                 self._put(self._hview("ms", self.K * self.K), ms)
-                self._put(self._hview("g0", self.K), gamma[0])
+                g0 = gamma[0] if self.seq_starts is None else gamma[self.seq_starts].sum(axis=0)
+                self._put(self._hview("g0", self.K), g0)
                 self._hview("sc", 8).zero_()
                 self._pass(mode=_lib.HMM_STATS_FROM_GAMMA, force=1)
             else:
@@ -621,7 +668,8 @@ class HMMEngine(VBEngine):
     def viterbi(self, ln_pi_tilde, ln_a_tilde):
         """Most probable state path of the loaded sequence under the current parameter set (:1466-1480): the emission log
         densities (bgmm_hmm_pass, emission-only mode), then the max-plus recursion and the back-tracking on the device
-        (bgmm_hmm_viterbi).  -> (path [n] int64 numpy, omega [n][K] device tensor, phi [n][K] int32 device tensor)."""
+        (bgmm_hmm_viterbi; bgmm_hmm_viterbi_seqs per sequence, in parallel, after set_sequences).
+        -> (path [n] int64 numpy, omega [n][K] device tensor, phi [n][K] int32 device tensor)."""
         n, K = self.n_local, self.K
         with torch.cuda.device(self.device):
             _lib.check(self.lib.bgmm_hmm_pass(self.x.data_ptr(), n, K, self.D, self.state.data_ptr(), self.hst.data_ptr(),
@@ -632,6 +680,13 @@ class HMMEngine(VBEngine):
             omega = torch.empty((n, K), dtype=torch.float64, device=self.device)
             phi = torch.empty((n, K), dtype=torch.int32, device=self.device)
             path = torch.empty(n, dtype=torch.int32, device=self.device)
+            if self.plan is not None:
+                _lib.check(self.lib.bgmm_hmm_viterbi_seqs(n, K, self.lnrho_buf.data_ptr(), lnpi.data_ptr(), lna.data_ptr(),
+                                                          omega.data_ptr(), phi.data_ptr(), path.data_ptr(),
+                                                          self._seq_starts_dev().data_ptr(), self.seq_starts.size,
+                                                          self._stream()), "bgmm_hmm_viterbi_seqs")
+                self.kernel_launches += 4
+                return path.cpu().numpy().astype(np.int64), omega, phi
             _lib.check(self.lib.bgmm_hmm_viterbi(n, K, self.lnrho_buf.data_ptr(), lnpi.data_ptr(), lna.data_ptr(),
                                                  omega.data_ptr(), phi.data_ptr(), path.data_ptr(), self._stream()),
                        "bgmm_hmm_viterbi")

@@ -13,7 +13,14 @@ Viterbi path of `estimate_latent_vars` (max-plus recursion + back-tracking) also
 The per-element arrays (`_ln_rho`, `_rho`, `alpha_vecs`, `beta_vecs`, `gamma_vecs`, `_cs`, `xi_mats`) stay on the
 GPU until the attribute is read; `xi_mats` (N x K x K) is formed on the host from them on first access.
 
-Additive, defaulted option (does not exist in the reference): `device`.
+Several independent sequences (`lengths=` of `update_posterior` / `estimate_latent_vars`, keyword only): the rows of x
+are the sequences concatenated in order, and they share one posterior.  The recursions restart at every sequence start
+(forward from pi~, backward from ones at every sequence end), xi is zero at every start (so `ms` counts only transitions
+inside a sequence), E ln p(z) / E ln q(z) take gamma summed over the sequence starts, and the Viterbi path is decoded per
+sequence.  The per-element arrays keep their (N, K) / (N,) shapes over the concatenated rows.  `lengths=None` and
+`lengths=[N]` are the single-sequence path.
+
+Additive, defaulted options (they do not exist in the reference): `device`, `lengths`.
 """
 import warnings
 
@@ -99,6 +106,7 @@ class LearnModel(base.Posterior, base.PredictiveMixin):
 
         # per-element quantities of the forward-backward pass (:554-561), device resident until read
         self._length = 0
+        self._starts = None                             # first rows of the sequences (several sequences), else None
         for name in _LAZY:
             setattr(self, "_lazy_" + name.lstrip("_"), _LazyDeviceArray())
         self._rho_host = None
@@ -177,6 +185,8 @@ class LearnModel(base.Posterior, base.PredictiveMixin):
                 xi[1:] = (self.alpha_vecs[:-1, :, np.newaxis] * self._rho[1:, np.newaxis, :]
                           * self._a_tilde_mat[np.newaxis, :, :] * self.beta_vecs[1:, np.newaxis, :])
                 xi[1:] /= self._cs[1:, np.newaxis, np.newaxis]
+            if self._starts is not None:
+                xi[self._starts] = 0.0                 # no transition into the first element of a sequence
             self._xi_host = xi
         return self._xi_host
 
@@ -298,6 +308,24 @@ class LearnModel(base.Posterior, base.PredictiveMixin):
         _check.shape_consistency(x.shape[-1], "x.shape[-1]", self.c_degree, "self.c_degree", DataFormatError)
         return x.reshape(-1, self.c_degree)
 
+    @staticmethod
+    def _seq_starts(lengths, n):
+        """First rows of the sequences given by `lengths` (int64), or None for one sequence (lengths None or [n])."""
+        if lengths is None:
+            return None
+        arr = np.asarray(lengths)
+        if arr.ndim != 1 or arr.size == 0 or arr.dtype.kind not in "iu":
+            raise DataFormatError("lengths must be a non-empty 1-dimensional sequence of positive ints.")
+        if np.any(arr <= 0):
+            raise DataFormatError(f"lengths must be positive: lengths = {arr}")
+        if int(arr.sum()) != n:
+            raise DataFormatError(f"lengths must sum to the number of rows of x: sum(lengths) = {int(arr.sum())}, rows = {n}")
+        if arr.size == 1:
+            return None
+        starts = np.zeros(arr.size, dtype=np.int64)
+        np.cumsum(arr[:-1], out=starts[1:])
+        return starts
+
     def _push_prior(self, eng):
         eng.set_hmm_prior(self.h0_eta_vec, self.h0_zeta_vecs, self.h0_m_vecs, self.h0_kappas, self.h0_nus,
                           self.h0_w_mats_inv, self._ln_b_h0_w_nus, self._ln_c_h0_eta_vec, self._ln_c_h0_zeta_vecs_sum)
@@ -337,18 +365,33 @@ class LearnModel(base.Posterior, base.PredictiveMixin):
         self.s_mats[:] = s["s_mats"]
 
     # ------------------------------------------------------------------ initialisations (host: they consume self.rng)
-    def _init_random_responsibility(self, n):
-        """Random xi / gamma (:944-952) -> (gamma [n][K], ms [K][K]); the statistics are computed on the device."""
+    def _init_random_responsibility(self, n, starts=None):
+        """Random xi / gamma (:944-952) -> (gamma [n][K], ms [K][K]); the statistics are computed on the device.
+
+        Several sequences (`starts`, their first rows): the same single draw `rng.dirichlet(np.ones(K**2), n)`; every
+        row gets gamma = xi.sum(axis=1), then at every sequence start s, gamma_s = xi_{s+1}.sum(axis=1) (row sums of the
+        K x K matrix) when that sequence is longer than 1, or the row sums of its own drawn xi_s for a sequence of
+        length 1; then xi_s = 0.  With one sequence this is the reference's rule."""
         K = self.c_num_classes
         gamma = np.ones([n, K]) / K
         xi_sum = np.zeros([K, K])
         if n == 1:
             gamma[0] = self.rng.dirichlet(np.ones(K))
-        else:
+        elif starts is None:
             xi = self.rng.dirichlet(np.ones(K ** 2), n).reshape(n, K, K)
             xi[0] = 0.0
             gamma[:] = xi.sum(axis=1)
             gamma[0] = xi[1].sum(axis=1)
+            xi_sum = xi.sum(axis=0)
+        else:
+            xi = self.rng.dirichlet(np.ones(K ** 2), n).reshape(n, K, K)
+            gamma[:] = xi.sum(axis=1)
+            ends = np.append(starts[1:], n)
+            single = ends - starts == 1
+            longer = starts[~single]
+            gamma[longer] = xi[longer + 1].sum(axis=2)           # the row sums of xi_{s+1}, as gamma[0] above
+            gamma[starts[single]] = xi[starts[single]].sum(axis=2)
+            xi[starts] = 0.0
             xi_sum = xi.sum(axis=0)
         return gamma, xi_sum
 
@@ -365,23 +408,30 @@ class LearnModel(base.Posterior, base.PredictiveMixin):
         self._calc_q_lambda_features()
 
     # ------------------------------------------------------------------ the fit (:1028-1134)
-    def update_posterior(self, x, max_itr=100, num_init=10, tolerance=1.0E-8, init_type='subsampling'):
+    def update_posterior(self, x, max_itr=100, num_init=10, tolerance=1.0E-8, init_type='subsampling', *, lengths=None):
         """Update the posterior hyperparameters by variational Bayes with `num_init` restarts (:1028-1134).
 
         Parameters
         ----------
-        x : numpy.ndarray, shape (..., c_degree) — one sequence, in time order
+        x : numpy.ndarray, shape (..., c_degree) — one sequence in time order, or the sequences of `lengths` concatenated
         max_itr : int, maximum number of VB iterations per restart (default 100)
         num_init : int, number of restarts (default 10)
         tolerance : float, relative ELBO change that stops a restart (default 1e-8)
         init_type : 'subsampling' | 'random_responsibility'
+        lengths : optional (extension, keyword only) 1-D sequence of positive ints summing to the number of rows of x:
+            x holds that many independent sequences that share the posterior (see the module docstring).  'subsampling'
+            draws rows from all of x, as for one sequence; 'random_responsibility' is described in
+            `_init_random_responsibility`.  `make_prediction` / `pred_and_update` continue from the last element of
+            the last sequence.
 
         Nothing else consumes `self.rng` between the restarts (:1087-1100), so all initial states are drawn first (the
         same random stream as the reference's sequential loop) while x is uploaded; the restarts then run one after the
         other on the device and the reference's selection rule (:1114) and progress text are applied in order.
         """
         x = self._check_x(x)
+        starts = self._seq_starts(lengths, x.shape[0])
         self._length = x.shape[0]
+        self._starts = starts
         eng = self._engine()
         eng.load_data_begin(x)
         self._clear_elementwise()
@@ -395,7 +445,7 @@ class LearnModel(base.Posterior, base.PredictiveMixin):
             if init_type == 'subsampling':
                 self._init_subsampling(x)
             elif init_type == 'random_responsibility':
-                init = self._init_random_responsibility(x.shape[0])
+                init = self._init_random_responsibility(x.shape[0], starts)
             else:
                 raise ValueError(
                     f'init_type={init_type} is unsupported. '
@@ -403,6 +453,7 @@ class LearnModel(base.Posterior, base.PredictiveMixin):
                     + '"subsampling" and "random_responsibility"')
             inits.append(({name: np.array(getattr(self, name)) for name in _HN_NAMES}, init))
         eng.load_data_finish()
+        eng.set_sequences(starts)
         self._push_prior(eng)
 
         never_converged = True
@@ -582,9 +633,13 @@ class LearnModel(base.Posterior, base.PredictiveMixin):
         return prediction
 
     # ------------------------------------------------------------------ latent variables (:1425-1558)
-    def estimate_latent_vars(self, x, loss='0-1', viterbi=True):
+    def estimate_latent_vars(self, x, loss='0-1', viterbi=True, *, lengths=None):
         """Hidden-state estimates of the sequence x (:1425-1499): the jointly most probable path (`viterbi=True`,
         loss "0-1" only) or the per-element marginals gamma ("squared"/"KL") / their arg-max ("0-1").
+
+        `lengths` (extension, keyword only): x holds that many independent sequences, concatenated; the path is decoded
+        per sequence (the sequences in parallel on the device), `phi_vecs` is zero at every sequence start, and the
+        marginals are those of the multi-sequence model (see the module docstring).
 
         Everything runs on the device: the emission log densities, the max-plus recursion and back-tracking of the
         Viterbi path (in the reference's operation order), or (for `viterbi=False`) the whole forward-backward pass.
@@ -595,6 +650,7 @@ class LearnModel(base.Posterior, base.PredictiveMixin):
                 "x.shape[-1] must be self.c_degree: "
                 + f"x.shape[-1]={x.shape[-1]}, self.c_degree={self.c_degree}")
         x = x.reshape(-1, self.c_degree)
+        starts = self._seq_starts(lengths, x.shape[0])
         if viterbi and loss != '0-1':
             raise CriteriaError(f"loss=\"{loss}\" is unsupported. "
                                 + "When viterbi == True, this function supports only \"0-1\".")
@@ -605,6 +661,7 @@ class LearnModel(base.Posterior, base.PredictiveMixin):
         self._length = n
         eng = self._engine()
         eng.load_data(x)
+        eng.set_sequences(starts)
         self._push_prior(eng)
         if viterbi:
             # only the emission densities are evaluated (the reference fills _ln_rho / _rho here and nothing else); the
@@ -612,12 +669,14 @@ class LearnModel(base.Posterior, base.PredictiveMixin):
             self._push_hn(eng)
             path, omega, phi = eng.viterbi(self._ln_pi_tilde_vec, self._ln_a_tilde_mat)
             self._rho_host = None                   # alpha / beta / gamma / xi keep their values, as in the reference
+            # (and so does the sequence split they belong to, `_starts`, which xi_mats uses)
             self._lazy_ln_rho.set_device(eng.lnrho_buf)
             self._lazy_omega_vecs.set_device(omega)
             self._lazy_phi_vecs.set_device(phi)
             z_hat = np.zeros([n, K], dtype=int)
             z_hat[np.arange(n), path] = 1
             return z_hat
+        self._starts = starts                       # the per-element arrays below are those of this x and split
         self._final_e_step(eng)
         if loss == "squared" or loss == "KL":
             return self.gamma_vecs

@@ -303,6 +303,27 @@ int bgmm_hmm_small(int K, int D, double* state, double* hst, int mode, int max_i
 int bgmm_hmm_viterbi(int64_t n, int K, const double* lnrho, const double* lnpi, const double* lna, double* omega,
                      int32_t* phi, int32_t* path, void* stream);
 
+/* ---- several independent sequences sharing one posterior (`lengths=`) ---------------------------------------------
+ * x[n][D] holds the sequences concatenated in order; seq_starts[n_seqs] (int64, seq_starts[0] == 0, strictly increasing,
+ * < n) are their first rows.  The recursions restart at every sequence start (forward from pi~, backward from ones), xi
+ * is zero there (MS counts transitions inside sequences only) and G0 = sum over sequence starts of gamma there.
+ *
+ * bgmm_hmm_seq_plan (host): the chunk table bgmm_hmm_pass_seqs runs on (every sequence is cut into chunks of the
+ * single-sequence chunk length; no chunk crosses a sequence start).  Returns the table's length in int64 (and fills
+ * `plan` when cap is at least that), or BGMM_EINVAL for a bad argument.  The caller copies it to the device once. */
+int64_t bgmm_hmm_seq_plan(int64_t n, int64_t n_seqs, const int64_t* seq_starts, int64_t* plan, int64_t cap);
+/* doubles of scratch bgmm_hmm_pass_seqs needs (0 for a bad argument) */
+int64_t bgmm_hmm_seq_workspace_doubles(int K, int64_t n, int64_t n_seqs);
+/* bgmm_hmm_pass over several sequences: `plan` the host table from bgmm_hmm_seq_plan, `plan_dev` the same on the device;
+ * `scan_ws`: bgmm_hmm_seq_workspace_doubles(K, n, n_seqs). */
+int bgmm_hmm_pass_seqs(const void* x, int64_t n, int K, int D, double* state, double* hst, double* workspace,
+                       double* scan_ws, double* lnrho, double* alpha, double* gamma, double* cs, double* beta_out, int mode,
+                       int force, const int64_t* plan, const int64_t* plan_dev, void* stream);
+/* bgmm_hmm_viterbi per sequence (seq_starts: device), the sequences decoded in parallel; phi is 0 at every sequence start.
+ * Bit-identical to the numpy recursion run sequence by sequence. */
+int bgmm_hmm_viterbi_seqs(int64_t n, int K, const double* lnrho, const double* lnpi, const double* lna, double* omega,
+                          int32_t* phi, int32_t* path, const int64_t* seq_starts, int64_t n_seqs, void* stream);
+
 #ifdef __cplusplus
 }
 #endif

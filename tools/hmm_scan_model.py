@@ -4,6 +4,8 @@ Design aid + executable specification: tests/test_hmm_scan_model.py checks it ag
 the oracle.  Phase A: per chunk, the recursion is run from the K unit vectors (normalised, log scale kept) -> chunk
 transfer matrix.  Phase B: one sequential sweep over chunk matrices -> the vector at every chunk boundary.
 Phase C: per chunk, the exact recursion from its boundary vector (what the reference computes, up to rounding).
+The *_seqs functions model several independent sequences (bgmm_hmm_pass_seqs): chunks aligned to sequence starts,
+phase B segmented per sequence, windows clamped to their sequence (tests/test_hmm_seqs_scan_model.py).
 """
 import numpy as np
 
@@ -116,6 +118,115 @@ def backward_boundaries_window(rho, cs, a_t, L, W):
         e = min((c + 1) * L, n) - 1
         b = np.ones(K)
         for i in range(min(e + W, n - 1), e, -1):
+            b = a_t @ (rho[i] * b / cs[i])
+        w[c] = b
+    return w
+
+
+# ---- several independent sequences (bgmm_hmm_pass_seqs): every sequence is cut into its own chunks ----------------------
+def seq_chunks(starts, n, L):
+    """[(i0, i1, s0, s1)]: chunk [i0, i1) of the sequence [s0, s1); chunks of L elements, the last of a sequence shorter."""
+    ends = list(starts[1:]) + [n]
+    return [(i0, min(i0 + L, b), a, b) for a, b in zip(starts, ends) for i0 in range(a, b, L)]
+
+
+def forward_seqs(rho, pi_t, a_t, chunks):
+    """Phase A only for chunks followed by a chunk of the same sequence; phase B segmented per sequence (a chunk that
+    starts a sequence takes pi~); phase C restarts (no transition) at every sequence start.  -> alpha, cs, v."""
+    n, K = rho.shape
+    nch = len(chunks)
+    T = np.zeros((nch, K, K)); ls = np.zeros((nch, K))
+    for c, (i0, i1, s0, s1) in enumerate(chunks):
+        if i1 == s1:
+            continue
+        for j in range(K):
+            t = np.zeros(K); t[j] = 1.0; s_log = 0.0
+            for i in range(i0, i1):
+                t = (t if i == s0 else t @ a_t) * rho[i]
+                s = t.sum(); t = t / s; s_log += np.log(s)
+            T[c, j], ls[c, j] = t, s_log
+    v = np.zeros((nch, K))
+    for c, (i0, i1, s0, s1) in enumerate(chunks):
+        if i0 == s0:
+            v[c] = pi_t
+        else:
+            w = v[c - 1] * np.exp(ls[c - 1] - ls[c - 1].max())
+            nv = w @ T[c - 1]
+            v[c] = nv / nv.sum()
+    alpha = np.empty((n, K)); cs = np.empty(n)
+    for c, (i0, i1, s0, s1) in enumerate(chunks):
+        a = v[c]
+        for i in range(i0, i1):
+            u = (a if i == s0 else a @ a_t) * rho[i]
+            cs[i] = u.sum(); a = u / cs[i]; alpha[i] = a
+    return alpha, cs, v
+
+
+def backward_seqs(rho, cs, alpha, a_t, chunks):
+    """Phase A' only for chunks preceded by a chunk of the same sequence; phase B' segmented (a chunk that ends a sequence
+    takes ones); phase C' with xi = 0 at every sequence start.  -> beta, gamma, S, G0 (gamma summed over the starts), w."""
+    n, K = rho.shape
+    nch = len(chunks)
+    U = np.zeros((nch, K, K)); ls = np.zeros((nch, K))
+    for c, (i0, i1, s0, s1) in enumerate(chunks):
+        if i0 == s0:
+            continue
+        for j in range(K):
+            b = np.zeros(K); b[j] = 1.0; s_log = 0.0
+            for i in range(i1 - 1, i0 - 1, -1):
+                b = a_t @ (rho[i] * b / cs[i])
+                s = b.sum(); b = b / s; s_log += np.log(s)
+            U[c, j], ls[c, j] = b, s_log
+    w = np.zeros((nch, K))
+    for c in range(nch - 1, -1, -1):
+        i0, i1, s0, s1 = chunks[c]
+        if i1 == s1:
+            w[c] = 1.0
+        else:
+            acc = np.zeros(K)
+            for j in range(K):
+                if w[c + 1, j] > 0:
+                    acc += np.exp(ls[c + 1, j] + np.log(w[c + 1, j])) * U[c + 1, j]
+            w[c] = acc
+    beta = np.empty((n, K)); gamma = np.empty((n, K)); S = np.zeros((K, K)); G0 = np.zeros(K)
+    for c, (i0, i1, s0, s1) in enumerate(chunks):
+        b = w[c]
+        for i in range(i1 - 1, i0 - 1, -1):
+            beta[i] = b; gamma[i] = alpha[i] * b
+            wv = rho[i] * b / cs[i]
+            if i > s0:
+                S += np.outer(alpha[i - 1], wv)
+            else:
+                G0 += gamma[i]
+            b = a_t @ wv
+    return beta, gamma, S, G0, w
+
+
+def forward_boundaries_window_seqs(rho, pi_t, a_t, chunks, W):
+    """v[c] from a run over the W elements before chunk c, clamped to its sequence (from pi~ when it reaches the start)."""
+    K = rho.shape[1]
+    v = np.zeros((len(chunks), K))
+    for c, (i0, i1, s0, s1) in enumerate(chunks):
+        if i0 == s0:
+            v[c] = pi_t
+            continue
+        end, first = i0 - 1, i0 - W
+        t = np.array(pi_t) if first <= s0 else np.ones(K)
+        for i in range(max(first, s0), end + 1):
+            t = (t if i == s0 else t @ a_t) * rho[i]
+            t = t / t.sum()
+        v[c] = t
+    return v
+
+
+def backward_boundaries_window_seqs(rho, cs, a_t, chunks, W):
+    """w[c] from an un-normalised run from ones over the W elements after chunk c, clamped to its sequence."""
+    K = rho.shape[1]
+    w = np.zeros((len(chunks), K))
+    for c, (i0, i1, s0, s1) in enumerate(chunks):
+        e = i1 - 1
+        b = np.ones(K)
+        for i in range(min(e + W, s1 - 1), e, -1):
             b = a_t @ (rho[i] * b / cs[i])
         w[c] = b
     return w
