@@ -2,9 +2,9 @@
 //
 // Replaces, in /root/reference/bayesml/hiddenmarkovnormal/_hiddenmarkovnormal.py, `_update_q_z` :1020-1026 =
 //   _calc_rho :988-997          ln rho[n][k] (emission log density under q)        -> e_large_kernel, ln-rho-only mode
-//   _forward :999-1006          alpha_i = rho_i o (alpha_{i-1} A~) / c_i            -> fwd_basis / fwd_seq / fwd_chunk
-//   _backward :1008-1011        beta_i = A~ (rho_{i+1} o beta_{i+1}) / c_{i+1}       -> bwd_basis / bwd_seq / bwd_chunk
-//   _update_gamma :1013-1014    gamma = alpha o beta                                 -> bwd_chunk
+//   _forward :999-1006          alpha_i = rho_i o (alpha_{i-1} A~) / c_i            -> hmm_basis_mma / hmm_seq / hmm_fwd
+//   _backward :1008-1011        beta_i = A~ (rho_{i+1} o beta_{i+1}) / c_{i+1}       -> hmm_basis_mma / hmm_seq / hmm_bwd
+//   _update_gamma :1013-1014    gamma = alpha o beta                                 -> hmm_bwd
 //   _update_xi :1016-1018       xi_i = alpha_{i-1} rho_i A~ beta_i / c_i; only sum_i xi_i (= ms, :839) is formed
 //   _calc_n_m_x_bar_s :837-845  N_k, x_bar_k, S_k with gamma as weights              -> m_large_kernel + reduction
 //
@@ -15,7 +15,8 @@
 //   B  (one warp, sequential over chunks): propagate the boundary vector through the transfer matrices;
 //   C  (parallel over chunks): the reference's exact recursion from the chunk's boundary vector, writing alpha, c
 //      (forward) or gamma, sum xi, sum gamma ln rho (backward).
-// Phase A costs K times phase C (N K^3 flops); everything is FP64 CUDA-core work on small per-state vectors: a group
+// Phase A costs K times phase C (N K^3 flops) and runs on the FP64 tensor pipe (hmm_basis_mma_kernel: the K runs of a
+// chunk as one matrix recursion).  Phases B and C are FP64 CUDA-core work on small per-state vectors; in phase C a group
 // of KP = 2^ceil(log2 K) lanes owns one chunk (32 / KP chunks per warp), state vectors are exchanged through a per-warp
 // shared-memory line (one STS + K/2 broadcast LDS.128 per step).  All sums are in a fixed order (deterministic).
 // Several independent sequences (bgmm_hmm_pass_seqs): every sequence is cut into its own chunks (ScanPlan.coff), so no
@@ -79,9 +80,6 @@ __device__ __forceinline__ double group_dot(const double* line, int gbase, const
 }
 
 // ---------------------------------------------------------------------------------------------------------------
-// forward recursion over one chunk from a given start vector.  BASIS: start = unit vector j, keep the normalised end
-// vector and its log scale (phase A).  Otherwise: start = boundary vector v[c]; write alpha, c, sum ln c (phase C).
-// Lane kk of a group owns state kk and column kk of A~.
 struct ScanBufs {
     const double* lnrho;   // [n][K]
     const double* rhohat;  // [n][K] exp(ln rho - row max): what the recursions multiply by (rho_i / c_i = rhohat_i / chat_i)
@@ -170,8 +168,9 @@ __device__ __forceinline__ int hmm_window(const double* st, const Layout& L, con
     return w < 8.0 ? 8 : (int)w;
 }
 
-// MODE 0: phase C (exact recursion from the boundary vector);  1: phase A (K basis runs per chunk; skipped in mixing mode)
-template <int KP, int MODE, bool SEQS>
+// Phase C, forward: the exact recursion over one chunk from its boundary vector v[c] (pi~ where a sequence starts);
+// writes alpha and chat.  Lane kk of a group owns state kk and column kk of A~.
+template <int KP, bool SEQS>
 __global__ void __launch_bounds__(HT) hmm_fwd_kernel(const ScanPlan sp, const double* __restrict__ st, const Layout L,
                                                      const double* __restrict__ hst, const HmmLayout H, const int force,
                                                      const ScanBufs B, const SeqArg<SEQS> T) {
@@ -180,28 +179,22 @@ __global__ void __launch_bounds__(HT) hmm_fwd_kernel(const ScanPlan sp, const do
     if (!force && ctrl[BGMM_CTRL_DONE]) return;
     constexpr int G = 32 / KP;
     const int K = sp.K, lane = threadIdx.x & 31, warp = threadIdx.x >> 5, kk = lane % KP, grp = lane / KP;
-    constexpr bool BASIS = (MODE != 0);                     // renormalise sparsely, no per-element outputs
-    if (MODE == 1 && hmm_window(st, L, hst, H, sp) > 0) return;
     const double* at = current_at(st, L, hst, H);
     const double* __restrict__ rhohat = B.rhohat;
     const int64_t item = ((int64_t)blockIdx.x * HW + warp) * G + grp;
-    const int64_t nitems = MODE == 1 ? (int64_t)(sp.nch - 1) * K : sp.nch;
-    const int c = MODE == 1 ? (int)(item / K) : (int)item;
-    const int j0 = MODE == 1 ? (int)(item - (int64_t)c * K) : 0;
+    const int c = (int)item;
     ChunkInfo ci{};
     if constexpr (SEQS) ci = chunk_info(sp, T, c);
-    // basis runs only for chunks followed by another chunk of the same sequence
-    const bool live = item < nitems && !(SEQS && MODE == 1 && ci.i1 == ci.s1), mine = live && kk < K;
+    const bool live = item < sp.nch, mine = live && kk < K;
     if (SEQS && !__any_sync(0xffffffffu, live)) return;
     double acol[KP];
 #pragma unroll
     for (int j = 0; j < KP; ++j) acol[j] = (mine && j < K) ? at[j * K + kk] : 0.0;
     double a = 0.0;
-    if (SEQS && MODE == 0 && ci.i0 == ci.s0) a = mine ? pi_tilde(st, L, K, kk) : 0.0;   // a sequence starts
-    else if (mine) a = MODE == 1 ? (kk == j0 ? 1.0 : 0.0) : B.vb[(int64_t)c * K + kk];
+    if (SEQS && ci.i0 == ci.s0) a = mine ? pi_tilde(st, L, K, kk) : 0.0;   // a sequence starts
+    else if (mine) a = B.vb[(int64_t)c * K + kk];
     const int64_t i0 = SEQS ? ci.i0 : (int64_t)c * sp.L;
     const int nst = SEQS ? warp_steps(live, ci) : sp.L;
-    double slog = 0.0;
     // emission values are fetched two steps ahead of the dependent chain (which runs through `a` only)
     auto RH = [&](int64_t i, int s) {
         return (mine && (SEQS ? i < ci.i1 : (s < sp.L && i < sp.n))) ? rhohat[i * K + kk] : 0.0;
@@ -216,37 +209,12 @@ __global__ void __launch_bounds__(HT) hmm_fwd_kernel(const ScanPlan sp, const do
         publish<KP>(line, lane, a);
         const double dot = group_dot<KP>(line, grp * KP, acol);
         const double u = rho * ((SEQS ? i == ci.s0 : i == 0) ? a : dot);   // :1000 — the first element has no transition
-        if (BASIS) {
-            // rhohat <= 1 with row maximum 1, so the vector shrinks by at most min(A~) per step: it is renormalised
-            // every 8 steps only (and at the end: phase B relies on rows of T summing to one)
-            if ((s & 7) == 7 || s == nst - 1) {
-                const double sum = group_sum<KP>(u);
-                if (live) {
-                    if (!(sum > 0.0)) {
-                        // the start state of this basis run is impossible (its emission value underflowed to exactly
-                        // 0): its response is exactly zero — not 0/0 — and weighs nothing in phase B (log scale -inf)
-                        a = 0.0;
-                        slog = -INFINITY;
-                    } else {
-                        a = u / sum;
-                        slog += log(sum);
-                    }
-                }
-            } else if (live) {
-                a = u;
-            }
-        } else {
-            const double sum = group_sum<KP>(u);                   // chat_i; c_i, 1 / chat_i and sum ln c_i: hmm_cs_kernel
-            if (live && i < (SEQS ? ci.i1 : sp.n)) {
-                a = u / sum;
-                if (mine) B.alpha[i * K + kk] = a;
-                if (kk == 0) B.chat[i] = sum;
-            }
+        const double sum = group_sum<KP>(u);                       // chat_i; c_i, 1 / chat_i and sum ln c_i: hmm_cs_kernel
+        if (live && i < (SEQS ? ci.i1 : sp.n)) {
+            a = u / sum;
+            if (mine) B.alpha[i * K + kk] = a;
+            if (kk == 0) B.chat[i] = sum;
         }
-    }
-    if (MODE == 1) {
-        if (mine) B.tf[((int64_t)c * K + j0) * K + kk] = a;
-        if (live && kk == 0) B.ls[(int64_t)c * K + j0] = slog;
     }
 }
 
@@ -494,12 +462,10 @@ __global__ void __launch_bounds__(SEQ_T) hmm_seq_kernel(const ScanPlan sp, const
 }
 
 // ---------------------------------------------------------------------------------------------------------------
-// backward recursion over one chunk (descending i).  Lane kk owns state kk and ROW kk of A~.
-// BASIS (phase A'): from unit vector j at the chunk's last element to the previous chunk's last element.
-// Otherwise (phase C'): from the boundary vector w[c]; gamma, the xi sum S[j][k] = sum_i alpha_{i-1}[j] rho_i[k]
-// beta_i[k] / c_i (A~ is applied once at the end), sum gamma ln rho, gamma_0, optionally beta.
-// MODE as in hmm_fwd_kernel (0: phase C', 1: phase A')
-template <int KP, int MODE, bool SEQS>
+// Phase C', backward: the recursion over one chunk (descending i) from its boundary vector w[c] (ones where a sequence
+// ends); gamma, the xi sum S[j][k] = sum_i alpha_{i-1}[j] rho_i[k] beta_i[k] / c_i (A~ is applied once at the end),
+// sum gamma ln rho, gamma_0, optionally beta.  Lane kk owns state kk and ROW kk of A~.
+template <int KP, bool SEQS>
 __global__ void __launch_bounds__(HT) hmm_bwd_kernel(const ScanPlan sp, const double* __restrict__ st, const Layout L,
                                                      double* __restrict__ hst, const HmmLayout H, const int force,
                                                      const ScanBufs B, const SeqArg<SEQS> T) {
@@ -507,8 +473,6 @@ __global__ void __launch_bounds__(HT) hmm_bwd_kernel(const ScanPlan sp, const do
     const volatile int* ctrl = reinterpret_cast<const volatile int*>(st + L.ctrl);
     if (!force && ctrl[BGMM_CTRL_DONE]) return;
     constexpr int G = 32 / KP;
-    constexpr bool BASIS = (MODE != 0);                     // no per-element outputs
-    if (MODE == 1 && hmm_window(st, L, hst, H, sp) > 0) return;
     const int K = sp.K, lane = threadIdx.x & 31, warp = threadIdx.x >> 5, kk = lane % KP, grp = lane / KP;
     const double* at = current_at(st, L, hst, H);
     const double* __restrict__ lnrho = B.lnrho;
@@ -516,33 +480,28 @@ __global__ void __launch_bounds__(HT) hmm_bwd_kernel(const ScanPlan sp, const do
     const double* __restrict__ alpha = B.alpha;
     const double* __restrict__ cs = B.ichat;                 // rho_i / c_i = rhohat_i * (1 / chat_i)
     const int64_t item = ((int64_t)blockIdx.x * HW + warp) * G + grp;
-    const int64_t nitems = MODE == 1 ? (int64_t)(sp.nch - 1) * K : sp.nch;
-    const int c = MODE == 1 ? 1 + (int)(item / K) : (int)item;          // basis runs: chunks 1 .. nch-1
-    const int j0 = MODE == 1 ? (int)(item % K) : 0;
+    const int c = (int)item;
     ChunkInfo ci{};
     if constexpr (SEQS) ci = chunk_info(sp, T, c);
-    // basis runs only for chunks preceded by another chunk of the same sequence
-    const bool live = item < nitems && !(SEQS && MODE == 1 && ci.i0 == ci.s0), mine = live && kk < K;
+    const bool live = item < sp.nch, mine = live && kk < K;
     if (SEQS && !__any_sync(0xffffffffu, live)) return;
-    double arow[KP], srow[BASIS ? 1 : KP];
+    double arow[KP], srow[KP];
 #pragma unroll
     for (int k = 0; k < KP; ++k) arow[k] = (mine && k < K) ? at[kk * K + k] : 0.0;
-    if constexpr (!BASIS) {
 #pragma unroll
-        for (int k = 0; k < KP; ++k) srow[k] = 0.0;
-    }
+    for (int k = 0; k < KP; ++k) srow[k] = 0.0;
     const int64_t i0 = SEQS ? ci.i0 : (int64_t)c * sp.L;
     const int64_t i1 = (SEQS ? ci.i1 : (i0 + sp.L < sp.n ? i0 + sp.L : sp.n)) - 1;   // last element of the chunk
     const int nst = SEQS ? warp_steps(live, ci) : sp.L;
     double b = 0.0;
-    if (SEQS && MODE == 0 && ci.i1 == ci.s1) b = mine ? 1.0 : 0.0;       // a sequence ends (:939)
-    else if (mine) b = MODE == 1 ? (kk == j0 ? 1.0 : 0.0) : B.vb[(int64_t)c * K + kk];
-    double slog = 0.0, gl = 0.0;
+    if (SEQS && ci.i1 == ci.s1) b = mine ? 1.0 : 0.0;                   // a sequence ends (:939)
+    else if (mine) b = B.vb[(int64_t)c * K + kk];
+    double gl = 0.0;
     // loads run two steps ahead, exp / reciprocal one step ahead of the dependent chain (which runs through b only)
-    auto LR = [&](int64_t i) { return (!BASIS && mine && i >= i0) ? lnrho[i * K + kk] : 0.0; };
+    auto LR = [&](int64_t i) { return (mine && i >= i0) ? lnrho[i * K + kk] : 0.0; };
     auto RH = [&](int64_t i) { return (mine && i >= i0) ? rhohat[i * K + kk] : 0.0; };
     auto CI = [&](int64_t i) { return (live && i >= i0) ? cs[i] : 1.0; };
-    auto AL = [&](int64_t i) { return (!BASIS && mine && i >= 0) ? alpha[i * K + kk] : 0.0; };
+    auto AL = [&](int64_t i) { return (mine && i >= 0) ? alpha[i * K + kk] : 0.0; };
     double lr_c = LR(i1), rho_c = RH(i1), inv_c = CI(i1);
     double lr_n = LR(i1 - 1), rho_n = RH(i1 - 1), ci_n = CI(i1 - 1);
     double al_c = AL(i1), al_p = AL(i1 - 1), al_pp = AL(i1 - 2);
@@ -554,7 +513,7 @@ __global__ void __launch_bounds__(HT) hmm_bwd_kernel(const ScanPlan sp, const do
         lr_n = LR(i - 2); rho_n = RH(i - 2); ci_n = CI(i - 2);
         al_c = al_p; al_p = al_pp; al_pp = AL(i - 3);
         const double rb = on ? rho * b : 0.0;                          // rho_i[k] beta_i[k]
-        if (!BASIS && on) {
+        if (on) {
             const double g = al * b;                                   // :1014
             B.gamma[i * K + kk] = g;
             if (B.beta_out != nullptr) B.beta_out[i * K + kk] = b;
@@ -568,51 +527,28 @@ __global__ void __launch_bounds__(HT) hmm_bwd_kernel(const ScanPlan sp, const do
         double* line = lines[warp][s & 1];
         publish<KP>(line, lane, rb);
         const double dot = group_dot<KP>(line, grp * KP, arow);        // (A~ (rho o beta))[kk]
-        if constexpr (!BASIS) {
-            // alpha_{i-1}[kk] / c_i (:1017-1018); xi = 0 at a (sequence) start
-            const double f = (on && (SEQS ? i > ci.s0 : i >= 1)) ? aprev * inv : 0.0;
-            const double2* p = reinterpret_cast<const double2*>(line + grp * KP);
+        // alpha_{i-1}[kk] / c_i (:1017-1018); xi = 0 at a (sequence) start
+        const double f = (on && (SEQS ? i > ci.s0 : i >= 1)) ? aprev * inv : 0.0;
+        const double2* p = reinterpret_cast<const double2*>(line + grp * KP);
 #pragma unroll
-            for (int k2 = 0; k2 < KP / 2; ++k2) {
-                const double2 vv = p[k2];
-                srow[2 * k2] = fma(f, vv.x, srow[2 * k2]);
-                srow[2 * k2 + 1] = fma(f, vv.y, srow[2 * k2 + 1]);
-            }
+        for (int k2 = 0; k2 < KP / 2; ++k2) {
+            const double2 vv = p[k2];
+            srow[2 * k2] = fma(f, vv.x, srow[2 * k2]);
+            srow[2 * k2 + 1] = fma(f, vv.y, srow[2 * k2 + 1]);
         }
-        if (MODE == 1) {
-            // each step is already scaled by 1 / chat_i, so the vector is renormalised every 8 steps only; the result
-            // need not be normalised at the end (phase B' uses U e^{ls}, whatever the split between the two)
-            const double nb = dot * inv;
-            if ((s & 7) == 7) {
-                const double sum = group_sum<KP>(nb);
-                if (in) {
-                    if (sum > 0.0) { b = nb / sum; slog += log(sum); }
-                    else { b = 0.0; slog = -INFINITY; }                // impossible end state: zero response (see forward)
-                }
-            } else if (in) {
-                b = nb;
-            }
-        } else if (in) {
-            b = dot * inv;                                             // :1010-1011
-        }
+        if (in) b = dot * inv;                                         // :1010-1011
     }
-    if (MODE == 1) {
-        if (mine) B.tf[((int64_t)c * K + j0) * K + kk] = b;
-        if (live && kk == 0) B.ls[(int64_t)c * K + j0] = slog;
-    }
-    if constexpr (!BASIS) {
-        if (mine) {
+    if (mine) {
 #pragma unroll
-            for (int k = 0; k < KP; ++k)
-                if (k < K) B.ps[((int64_t)c * K + kk) * K + k] = srow[k];
-        }
-        const double t = group_sum<KP>(gl);
-        if (live && kk == 0) B.pgl[c] = t;
+        for (int k = 0; k < KP; ++k)
+            if (k < K) B.ps[((int64_t)c * K + kk) * K + k] = srow[k];
     }
+    const double t = group_sum<KP>(gl);
+    if (live && kk == 0) B.pgl[c] = t;
 }
 
-// Phase A / A' on the FP64 tensor pipe (K > 8).  The K basis runs of a chunk are ONE matrix recursion: with row j0 of S the
-// message vector started from unit vector j0,
+// Phase A / A' on the FP64 tensor pipe, for every K (K <= 8 runs as KP = 8, zero-padded).  The K basis runs of a chunk
+// are ONE matrix recursion: with row j0 of S the message vector started from unit vector j0,
 //     forward :  S <- (S . A~) o rho_i          (column scaling; `_hiddenmarkovnormal.py` :999-1004 applied to K vectors)
 //     backward:  S <- ((S o rho_i) . A~^T) / chat_i                                              (:1010-1011)
 // i.e. a right-multiplication by a CONSTANT matrix per step.  One warp owns one chunk and keeps S in DMMA accumulator
@@ -620,9 +556,10 @@ __global__ void __launch_bounds__(HT) hmm_bwd_kernel(const ScanPlan sp, const do
 // the next step: for fixed (kb, e) they form an 8 x 4 tile over the columns k = 8 kb + 2 q + e, a permuted k-block, and the
 // sum over k does not care about the order as long as the constant B fragments use the same rows — so there is no
 // layout conversion, no shuffle and no shared memory in the step: (KP/8)^3 * 2 DMMAs (128 at K = 32) + KP scalings.
-// The vector form above does the same 2 K^3 flops per element as K dependent mat-vec chains through shared memory
-// (12.4 of h2's 16.6 ms); this one is bound by the DMMA pipe.  Rows are renormalised every 8 steps (and at the end of a
-// forward chunk: phase B relies on rows summing to one), with the same zero-row rule as the vector kernels.
+// As K separate vector recursions the same 2 K^3 flops per element would be K dependent mat-vec chains through shared
+// memory; this form is bound by the DMMA pipe.  Rows are renormalised every 8 steps (and at the end of a forward chunk:
+// phase B relies on rows summing to one); a row whose sum is exactly zero (its start state is impossible) stays exactly
+// zero with log scale -inf, so it weighs nothing in phase B.
 template <int KP, bool FWD, bool SEQS>
 __global__ void __launch_bounds__(HT, KP >= 32 ? 1 : 4) hmm_basis_mma_kernel(const ScanPlan sp, const double* __restrict__ st, const Layout L,
                                                               const double* __restrict__ hst, const HmmLayout H,
@@ -903,11 +840,9 @@ static int64_t scan_ws_doubles(int K, int64_t n, int64_t nch) {
     return nch * KK + nch * K + nch * K + nch * KK + 2 * nch + 64 + n * K + 3 * n + 72 * (KK + 2 * K) + 2;
 }
 
-// Phase B of one direction: the single-CTA sweep, or (>= 4 groups of SEQ_GLEN steps) group matrices -> group sweep -> expansion
-static int hmm_two_level() {
-    static const int two_level = [] { const char* e = getenv("BGMM_HMM_TWO_LEVEL"); return (e == nullptr || atoi(e) != 0) ? 1 : 0; }();
-    return two_level;
-}
+// Phase B of one direction over nsteps chunk matrices: the single-CTA sweep, or (>= 4 groups of SEQ_GLEN steps) group
+// matrices -> group sweep -> expansion
+static bool two_level_sweep(int64_t nsteps) { return (nsteps + SEQ_GLEN - 1) / SEQ_GLEN >= 4; }
 
 // the sweep over chunks [cbase, cbase + nsteps] (cbase = 0 unless SEQS)
 template <int KP, bool FWD, bool SEQS>
@@ -915,11 +850,10 @@ static void launch_seq(const ScanPlan& sp, double* st, const Layout& L, double* 
                        const ScanBufs& B, size_t smem_seq, cudaStream_t stream, int cbase, int nsteps) {
     const int K = sp.K;
     const int ngroups = (nsteps + SEQ_GLEN - 1) / SEQ_GLEN;
-    const int two_level = hmm_two_level();
     SeqLevel lv{0, nsteps, ngroups, B.tf, B.ls, B.vb, nullptr, nullptr, nullptr};
     SeqRangeArg<SEQS> R{};
     if constexpr (SEQS) R = SeqRange{cbase, nullptr};
-    if (!two_level || ngroups < 4) {
+    if (!two_level_sweep(nsteps)) {
         hmm_seq_kernel<KP, FWD, SEQS><<<1, SEQ_T, smem_seq, stream>>>(sp, st, L, hst, H, force, lv, R);
         return;
     }
@@ -959,8 +893,7 @@ static int launch_scan(const ScanPlan& sp, double* st, const Layout& L, double* 
                        const int64_t* segs_dev) {
     constexpr int G = 32 / KP;
     const int per_cta = HW * G;
-    const int64_t nbasis = (int64_t)(sp.nch - 1) * sp.K;
-    const unsigned gb = (unsigned)((nbasis + per_cta - 1) / per_cta), gc = (unsigned)((sp.nch + per_cta - 1) / per_cta);
+    const unsigned gc = (unsigned)((sp.nch + per_cta - 1) / per_cta);
     const size_t smem_seq = (size_t)2 * seq_batch(sp.K) * (sp.K * sp.K + sp.K + 8) * sizeof(double);
     {   // per launch: the attribute is per device
         cudaError_t e = cudaFuncSetAttribute(hmm_seq_kernel<KP, true, SEQS>, cudaFuncAttributeMaxDynamicSharedMemorySize, 208 * 1024);
@@ -970,28 +903,20 @@ static int launch_scan(const ScanPlan& sp, double* st, const Layout& L, double* 
     }
     // boundary vectors: either {basis runs, sequential sweep} or {one warm-up window per chunk}; the device decides
     // (hmm_window) from the current A~, the kernels of the other branch return at once
-    const char* env_mma = getenv("BGMM_HMM_BASIS_MMA");                    // 0: the vector basis runs (tests compare the two)
-    const int basis_mma = (env_mma == nullptr || atoi(env_mma) != 0) ? 1 : 0;
-    const unsigned gm = (unsigned)((sp.nch - 1 + HW - 1) / HW);          // tensor-pipe basis runs: one warp per chunk
+    const unsigned gm = (unsigned)((sp.nch - 1 + HW - 1) / HW);          // basis runs: one warp per chunk
     // basis runs and sweeps only where a sequence has more than one chunk
     const bool multi = plan == nullptr ? sp.nch > 1 : plan[4] + plan[5] > 0;
-    if (multi) {
-        if (KP >= 2 && basis_mma) hmm_basis_mma_kernel<(KP >= 8 ? KP : 8), true, SEQS><<<gm, HT, 0, stream>>>(sp, st, L, hst, H, force, B, T);
-        else hmm_fwd_kernel<KP, 1, SEQS><<<gb, HT, 0, stream>>>(sp, st, L, hst, H, force, B, T);
-    }
+    if (multi) hmm_basis_mma_kernel<(KP >= 8 ? KP : 8), true, SEQS><<<gm, HT, 0, stream>>>(sp, st, L, hst, H, force, B, T);
     if (plan == nullptr) launch_seq<KP, true, false>(sp, st, L, hst, H, force, B, smem_seq, stream, 0, sp.nch - 1);
     else launch_seq_segs<KP, true>(sp, st, L, hst, H, force, B, smem_seq, stream, plan, segs_dev);
     hmm_window_kernel<KP, true, SEQS><<<gc, HT, 0, stream>>>(sp, st, L, hst, H, force, B, T);
-    hmm_fwd_kernel<KP, 0, SEQS><<<gc, HT, 0, stream>>>(sp, st, L, hst, H, force, B, T);
+    hmm_fwd_kernel<KP, SEQS><<<gc, HT, 0, stream>>>(sp, st, L, hst, H, force, B, T);
     hmm_cs_kernel<SEQS><<<sp.nch, 128, 0, stream>>>(sp, st, L, force, B, T);
-    if (multi) {
-        if (KP >= 2 && basis_mma) hmm_basis_mma_kernel<(KP >= 8 ? KP : 8), false, SEQS><<<gm, HT, 0, stream>>>(sp, st, L, hst, H, force, B, T);
-        else hmm_bwd_kernel<KP, 1, SEQS><<<gb, HT, 0, stream>>>(sp, st, L, hst, H, force, B, T);
-    }
+    if (multi) hmm_basis_mma_kernel<(KP >= 8 ? KP : 8), false, SEQS><<<gm, HT, 0, stream>>>(sp, st, L, hst, H, force, B, T);
     if (plan == nullptr) launch_seq<KP, false, false>(sp, st, L, hst, H, force, B, smem_seq, stream, 0, sp.nch - 1);
     else launch_seq_segs<KP, false>(sp, st, L, hst, H, force, B, smem_seq, stream, plan, segs_dev);
     hmm_window_kernel<KP, false, SEQS><<<gc, HT, 0, stream>>>(sp, st, L, hst, H, force, B, T);
-    hmm_bwd_kernel<KP, 0, SEQS><<<gc, HT, 0, stream>>>(sp, st, L, hst, H, force, B, T);
+    hmm_bwd_kernel<KP, SEQS><<<gc, HT, 0, stream>>>(sp, st, L, hst, H, force, B, T);
     const int nred = sp.K * sp.K + 2 + (SEQS ? sp.K : 0);
     hmm_reduce_kernel<SEQS><<<(nred + 31) / 32, 256, 0, stream>>>(sp, st, L, hst, H, force, B, T);
     return check_cuda(cudaGetLastError(), "hmm scan launch");
@@ -1083,7 +1008,7 @@ static int launch_emit_small_d(const void* x, int64_t n, int K, const double* st
 // D <= 8 and K <= 32: the thread-per-element kernel; otherwise -1 (the caller uses the large-regime E kernel)
 static int launch_emit_small(const void* x, int64_t n, int K, int D, const double* st, const Layout& L, int force,
                              double* lnrho, double* rhohat, double* rowmax, cudaStream_t s) {
-    if (K > 32 || getenv("BGMM_HMM_NO_SMALL_EMIT") != nullptr) return -1;
+    if (K > 32) return -1;
     switch (D) {
         case 1: return launch_emit_small_d<1>(x, n, K, st, L, force, lnrho, rhohat, rowmax, s);
         case 2: return launch_emit_small_d<2>(x, n, K, st, L, force, lnrho, rhohat, rowmax, s);
@@ -1354,15 +1279,14 @@ extern "C" int64_t bgmm_hmm_seq_plan(int64_t n, int64_t n_seqs, const int64_t* s
     int64_t* segs = sen + nch;
     int64_t* starts = segs + 2 * nseg;
     int64_t c = 0, ns = 0, nl = 0, nshort = 0;
-    const int two_level = hmm_two_level();
     for (int64_t q = 0; q < n_seqs; ++q) {
         const int64_t m = ((q + 1 < n_seqs ? seq_starts[q + 1] : n) - seq_starts[q] + L - 1) / L;
-        nshort += m > 1 && !(two_level && (m - 1 + SEQ_GLEN - 1) / SEQ_GLEN >= 4);
+        nshort += m > 1 && !two_level_sweep(m - 1);
     }
     for (int64_t q = 0; q < n_seqs; ++q) {
         const int64_t a = seq_starts[q], b = q + 1 < n_seqs ? seq_starts[q + 1] : n, m = (b - a + L - 1) / L;
         if (m > 1) {
-            const bool lng = two_level && (m - 1 + SEQ_GLEN - 1) / SEQ_GLEN >= 4;
+            const bool lng = two_level_sweep(m - 1);
             int64_t* sg = segs + 2 * (lng ? nshort + nl++ : ns++);
             sg[0] = c;
             sg[1] = m;

@@ -11,7 +11,6 @@
 // Cholesky factorisation for the inverse and the log-determinant (agrees to cond*eps, tested vs the oracle).
 #include "bgmm_common.cuh"
 #include <math.h>
-#include <stdlib.h>
 
 namespace bgmm {
 
@@ -859,11 +858,8 @@ __global__ void __launch_bounds__(256) hmm_trans_kernel(double* __restrict__ st,
     }
 }
 
-// D <= 32 runs the warp-synchronous kernel; BGMM_SMALL_WARP=0 in the environment keeps the block kernel (A/B measurements)
-static bool use_warp_kernel(int D) {
-    static const int on = [] { const char* e = getenv("BGMM_SMALL_WARP"); return (e == nullptr || atoi(e) != 0) ? 1 : 0; }();
-    return on != 0 && D <= 32;
-}
+// D <= 32 runs the warp-synchronous kernel; the block kernel is the path for larger D
+static bool use_warp_kernel(int D) { return D <= 32; }
 
 static cudaError_t launch_small_warp(int K, int D, cudaStream_t stream, double* state, const Layout& L, int mode, int max_itr,
                                      double tol, const CommDesc* cd, const double* hmm_vlx) {

@@ -204,9 +204,9 @@ def test_window_and_basis_paths_agree(lib_built, monkeypatch):
 
 
 @pytest.mark.parametrize("K,D,n", [(32, 3, 120_000), (12, 2, 90_000), (17, 4, 40_000), (8, 2, 200_000), (3, 2, 100_000), (5, 3, 60_000)])
-def test_tensor_pipe_basis_runs_match_the_vector_basis_runs(K, D, n, lib_built, monkeypatch):
-    """Phase A / A' as one DMMA matrix recursion per chunk (hmm_basis_mma_kernel, K > 8) against the K vector recursions
-    per chunk it replaces, and against the oracle: same fit.  The window shortcut is disabled so the basis path runs."""
+def test_basis_runs_match_the_oracle(K, D, n, lib_built, monkeypatch):
+    """Phase A / A' (hmm_basis_mma_kernel: the K basis runs of a chunk as one DMMA matrix recursion, K padded to 8 below 8)
+    against the oracle: same fit.  The window shortcut is disabled so the basis path runs."""
     from bayesml_b200.engine import HMMEngine
     from oracle.hmm_vb_oracle import OracleHMM
     rng = np.random.default_rng(K + D)
@@ -223,30 +223,25 @@ def test_tensor_pipe_basis_runs_match_the_vector_basis_runs(K, D, n, lib_built, 
     o.init_subsampling(x)
     init_m, init_winv = o.hn_m_vecs.copy(), o.hn_w_mats_inv.copy()
     monkeypatch.setenv("BGMM_HMM_WINDOW_CAP", "0")
-    out = {}
-    for mma in ("1", "0"):
-        monkeypatch.setenv("BGMM_HMM_BASIS_MMA", mma)
-        eng = HMMEngine(K, D)
-        eng.load_data(x)
-        eng.set_hmm_prior(o.h0_eta_vec, o.h0_zeta_vecs, o.h0_m_vecs, o.h0_kappas, o.h0_nus, o.h0_w_mats_inv, o.ln_b_h0_w_nus,
-                          o.ln_c_h0_eta_vec, o.ln_c_h0_zeta_vecs_sum)
-        eng.set_hmm_params(o.h0_eta_vec, o.h0_zeta_vecs, init_m, o.h0_kappas, o.h0_nus, init_winv)
-        hist, _ = eng.run(3, 0.0)
-        out[mma] = (np.asarray(hist), eng.fetch_params(), eng.gamma_buf.cpu().numpy(), eng.cs_buf.cpu().numpy())
-    assert out["1"][1]["window"] == 0
-    assert np.allclose(out["1"][0], out["0"][0], rtol=1e-11)
-    for key in ("ms", "zeta", "m", "winv", "ns"):
-        assert np.allclose(out["1"][1][key], out["0"][1][key], rtol=1e-9, atol=1e-12), key
-    assert np.allclose(out["1"][2], out["0"][2], rtol=1e-8, atol=1e-13)
-    assert np.allclose(out["1"][3], out["0"][3], rtol=1e-10)
+    eng = HMMEngine(K, D)
+    eng.load_data(x)
+    eng.set_hmm_prior(o.h0_eta_vec, o.h0_zeta_vecs, o.h0_m_vecs, o.h0_kappas, o.h0_nus, o.h0_w_mats_inv, o.ln_b_h0_w_nus,
+                      o.ln_c_h0_eta_vec, o.ln_c_h0_zeta_vecs_sum)
+    eng.set_hmm_params(o.h0_eta_vec, o.h0_zeta_vecs, init_m, o.h0_kappas, o.h0_nus, init_winv)
+    hist, _ = eng.run(3, 0.0)
+    hist, p = np.asarray(hist), eng.fetch_params()
+    assert p["window"] == 0
     o.e_step(x)
     o.calc_vl()
     ref = [o.vl]
     for _ in range(3):
         o.iterate(x)
         ref.append(o.vl)
-    assert _close(out["1"][0], ref), np.max(np.abs(out["1"][0] - ref) / np.abs(ref))
-    assert np.allclose(out["1"][2], o.gamma_vecs, rtol=1e-7, atol=1e-12)
+    assert _close(hist, ref), np.max(np.abs(hist - ref) / np.abs(ref))
+    for mine, name in (("ms", "ms"), ("zeta", "hn_zeta_vecs"), ("m", "hn_m_vecs"), ("winv", "hn_w_mats_inv"), ("ns", "ns")):
+        assert _close(p[mine], getattr(o, name)), mine
+    assert np.allclose(eng.gamma_buf.cpu().numpy(), o.gamma_vecs, rtol=1e-7, atol=1e-12)
+    assert _close(eng.cs_buf.cpu().numpy(), o.cs, rtol=1e-8)
 
 
 def test_viterbi_long_sequence_is_bit_identical_to_the_numpy_recursion(lib_built):
