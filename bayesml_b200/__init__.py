@@ -1,5 +1,6 @@
 """bayesml_b200 — B200-native variational-Bayes Gaussian mixture, drop-in for `bayesml.gaussianmixture.LearnModel`
-(and, sharing its kernels, `bayesml.hiddenmarkovnormal.LearnModel`).
+(and, sharing its kernels, `bayesml.hiddenmarkovnormal.LearnModel`; both modules also have the reference's `GenModel`, whose
+`gen_sample` can draw on the device).
 
     from bayesml_b200 import gaussianmixture
     model = gaussianmixture.LearnModel(c_num_classes=3, c_degree=2)

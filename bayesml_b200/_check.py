@@ -59,6 +59,17 @@ def float_vec_sum_1(val, val_name, exception_class):
     raise exception_class(val_name + " must be a 1-dimensional numpy.ndarray, and the sum of its elements must equal to 1.")
 
 
+def float_vecs_sum_1(val, val_name, exception_class):
+    """Numeric ndarray with ndim >= 1 whose sums along the last axis are each 1 within sqrt(eps) (the stacked form of
+    float_vec_sum_1)."""
+    if type(val) is np.ndarray and val.ndim >= 1 and np.all(np.abs(val.sum(axis=-1) - 1.0) <= np.sqrt(np.finfo(np.float64).eps)):
+        if np.issubdtype(val.dtype, np.integer):
+            return val.astype(float)
+        if np.issubdtype(val.dtype, np.floating):
+            return val
+    raise exception_class(val_name + " must be a numpy.ndarray whose ndim >= 1, and the sum along the last dimension must equal to 1.")
+
+
 def float_vecs(val, val_name, exception_class):
     """Numeric ndarray with ndim >= 1 (reference _check.py:203-209)."""
     if type(val) is np.ndarray and val.ndim >= 1:

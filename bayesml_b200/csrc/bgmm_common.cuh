@@ -159,6 +159,14 @@ __host__ __device__ inline HmmLayout make_hmm_layout(int K) {
     return H;
 }
 
+// Chunk length of the HMM scans and of the chain sampler: <= 4096 chunks (the length of their phase B), at least 32
+// elements each.
+__host__ __device__ inline int hmm_chunk_len(int64_t n) {
+    int64_t L = (n + 4095) / 4096;
+    if (L < 32) L = 32;
+    return (int)((L + 7) & ~int64_t(7));
+}
+
 // Entry test of every pass kernel: queued launches after convergence are no-ops (ctrl.done), and the feature-map kernels
 // stand down when bgmm_small has flagged the current parameter set as ill-conditioned (ctrl.robust): the DIRECT kernel
 // launched behind them does that pass.

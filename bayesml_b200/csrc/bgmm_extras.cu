@@ -79,25 +79,17 @@ __global__ void __launch_bounds__(256) dirichlet1_kernel(double* __restrict__ r,
     for (int j = 0; j < K; ++j) out[j] *= inv;
 }
 
-// GenModel.gen_sample on the device (/root/reference/bayesml/gaussianmixture/_gaussianmixture.py:241-264: a Python loop,
-// one `rng.choice` + one `rng.multivariate_normal` per sample): one thread per sample, class from the inverse CDF of pi,
-// x = mu_z + L_z eps with L_z = chol(Lambda_z^-1) and Box-Muller normals from Philox keyed by (seed, global row).
-__global__ void __launch_bounds__(128) gen_sample_kernel(double* __restrict__ x, int32_t* __restrict__ z, const int64_t n,
-                                                         const int K, const int D, const double* __restrict__ cdf,
-                                                         const double* __restrict__ mu, const double* __restrict__ chol,
-                                                         const unsigned long long seed, const int64_t row_offset) {
-    extern __shared__ double eps_s[];                           // [128][D + 1]: this thread's standard normals
-    const int64_t i = (int64_t)blockIdx.x * 128 + threadIdx.x;
-    if (i >= n) return;
-    const unsigned long long g = (unsigned long long)(row_offset + i);
-    const uint2 key = make_uint2((uint32_t)seed, (uint32_t)(seed >> 32));
-    double* eps = eps_s + threadIdx.x * (D + 1);
-    const uint4 v0 = philox4x32_10(make_uint4((uint32_t)g, (uint32_t)(g >> 32), 0u, 0x47454e53u), key);
-    const double u = uniform_open(v0.x, v0.y);
-    int k = 0;
-    while (k < K - 1 && u > cdf[k]) ++k;
+// One generated element: class k = pick(u) with u the uniform of Philox word 0 of the counter (g, 0, tag) under `key`,
+// then x[i] = mu_k + L_k eps (L_k = chol[k], lower [D][D]) with eps ~ N(0, I_D) by Box-Muller from words 1, 2, ... of
+// the same counter.  `eps` holds D doubles of this thread's scratch.  Returns k.
+template <class Pick>
+__device__ __forceinline__ int gauss_sample(double* __restrict__ x, const int64_t i, double* eps, const int D,
+                                            const double* __restrict__ mu, const double* __restrict__ chol,
+                                            const unsigned long long g, const uint2 key, const uint32_t tag, Pick pick) {
+    const uint4 v0 = philox4x32_10(make_uint4((uint32_t)g, (uint32_t)(g >> 32), 0u, tag), key);
+    const int k = pick(uniform_open(v0.x, v0.y));
     for (int j = 0; j < D; j += 2) {
-        const uint4 v = philox4x32_10(make_uint4((uint32_t)g, (uint32_t)(g >> 32), (uint32_t)(1 + (j >> 1)), 0x47454e53u), key);
+        const uint4 v = philox4x32_10(make_uint4((uint32_t)g, (uint32_t)(g >> 32), (uint32_t)(1 + (j >> 1)), tag), key);
         const double rad = sqrt(-2.0 * log(uniform_open(v.x, v.y))), ang = 6.283185307179586476925286766559 * uniform_open(v.z, v.w);
         double sn, cs;
         sincos(ang, &sn, &cs);
@@ -111,7 +103,175 @@ __global__ void __launch_bounds__(128) gen_sample_kernel(double* __restrict__ x,
         for (int b = 0; b <= a; ++b) acc = fma(L[a * D + b], eps[b], acc);
         x[i * D + a] = acc;
     }
-    z[i] = k;
+    return k;
+}
+
+// GenModel.gen_sample on the device (/root/reference/bayesml/gaussianmixture/_gaussianmixture.py:241-264: a Python loop,
+// one `rng.choice` + one `rng.multivariate_normal` per sample): one thread per sample, class from the inverse CDF of pi,
+// x = mu_z + L_z eps with L_z = chol(Lambda_z^-1) and Box-Muller normals from Philox keyed by (seed, global row).
+__global__ void __launch_bounds__(128) gen_sample_kernel(double* __restrict__ x, int32_t* __restrict__ z, const int64_t n,
+                                                         const int K, const int D, const double* __restrict__ cdf,
+                                                         const double* __restrict__ mu, const double* __restrict__ chol,
+                                                         const unsigned long long seed, const int64_t row_offset) {
+    extern __shared__ double eps_s[];                           // [128][D + 1]: this thread's standard normals
+    const int64_t i = (int64_t)blockIdx.x * 128 + threadIdx.x;
+    if (i >= n) return;
+    const unsigned long long g = (unsigned long long)(row_offset + i);
+    const uint2 key = make_uint2((uint32_t)seed, (uint32_t)(seed >> 32));
+    double* eps = eps_s + threadIdx.x * (D + 1);
+    z[i] = gauss_sample(x, i, eps, D, mu, chol, g, key, 0x47454e53u, [&](double u) {
+        int k = 0;
+        while (k < K - 1 && u > cdf[k]) ++k;
+        return k;
+    });
+}
+
+// ---- hidden-Markov chains (bgmm_hmm_gen_sample) ----
+// Element i of a chain is z_i = f_i(z_{i-1}) with f_i(s) = inverse CDF of row s of A at u_i, or at a sequence start the
+// constant map "inverse CDF of pi at u_i".  Maps on {0..K-1} compose associatively, so the chain is sampled exactly in
+// three phases over chunks of L elements:  A: per chunk, the composed map F_c (lane s of the chunk's warp runs the chunk
+// from state s);  B: one CTA sweeps the <= 4096 maps staged in shared memory, in_c = F_{c-1}(in_{c-1});  C: per chunk,
+// the run from in_c writes z.  u_i is Philox word 0 of (seed, i, HMM_GEN_TAG), so z does not depend on L.
+constexpr uint32_t HMM_GEN_TAG = 0x484d4d47u;                    // "HMMG"
+constexpr int HMM_GEN_MAX_CHUNKS = 4096;
+
+__host__ __device__ inline int pow2_ceil(int K) {
+    int p = 1;
+    while (p < K) p <<= 1;
+    return p;
+}
+
+// The (K + 1) inverse-CDF rows in shared memory, stride KP + 1 doubles (KP = pow2_ceil(K)): entry k < K - 1 is the running
+// max of cdf[r][0..k], every later entry +inf.  The running max does not change "the first k with u <= cdf[r][k]" (every
+// earlier entry is < u), makes the row sorted for a binary search, and k = K - 1 is the clamp of gen_sample_kernel.
+__device__ __forceinline__ void stage_cdf(double* tab, const double* __restrict__ cdf, const int K, const int KP) {
+    for (int e = threadIdx.x; e < (K + 1) * KP; e += blockDim.x) {
+        const int r = e / KP, k = e - r * KP;
+        double v = INFINITY;
+        if (k < K - 1) {
+            v = cdf[r * K];
+            for (int j = 1; j <= k; ++j) v = fmax(v, cdf[r * K + j]);
+        }
+        tab[r * (KP + 1) + k] = v;
+    }
+}
+
+__device__ __forceinline__ int inv_cdf(const double* row, const double u, const int KP) {
+    int k = 0;
+    for (int step = KP >> 1; step > 0; step >>= 1)
+        if (row[k + step - 1] < u) k += step;
+    return k;
+}
+
+// Phases A (WRITE_Z = false: maps[c][s] = F_c(s)) and C (WRITE_Z: z of chunk c from in[c]); one warp per chunk.  The
+// lanes draw the uniforms of 32 elements at a time and the chain steps through them by broadcast; `starts` (sorted,
+// starts[0] = 0) is searched once per chunk and then read 32 entries per batch into a bit mask of the batch's starts.
+template <bool WRITE_Z>
+__global__ void __launch_bounds__(256) hmm_chain_kernel(const int64_t n, const int K, const int KP, const int64_t L,
+                                                        const int nch, const double* __restrict__ cdf,
+                                                        const int64_t* __restrict__ starts, const int64_t n_seqs,
+                                                        const unsigned long long seed, uint8_t* __restrict__ maps,
+                                                        const uint8_t* __restrict__ in, int32_t* __restrict__ z) {
+    extern __shared__ double tab[];                             // [K + 1][KP + 1]
+    stage_cdf(tab, cdf, K, KP);
+    __syncthreads();
+    const int lane = threadIdx.x & 31;
+    const int c = blockIdx.x * 8 + (threadIdx.x >> 5);
+    if (c >= nch) return;
+    const uint2 key = make_uint2((uint32_t)seed, (uint32_t)(seed >> 32));
+    const int64_t b = (int64_t)c * L, e = min(n, b + L);
+    int64_t lo = 0, hi = n_seqs;                                // p = first sequence start >= b
+    while (lo < hi) {
+        const int64_t mid = (lo + hi) >> 1;
+        if (starts[mid] < b) lo = mid + 1; else hi = mid;
+    }
+    int64_t p = lo;
+    int s = WRITE_Z ? (int)in[c] : min(lane, K - 1);
+    for (int64_t base = b; base < e; base += 32) {
+        const unsigned long long g = (unsigned long long)(base + lane);
+        const uint4 v = philox4x32_10(make_uint4((uint32_t)g, (uint32_t)(g >> 32), 0u, HMM_GEN_TAG), key);
+        const double u_mine = uniform_open(v.x, v.y);
+        const int64_t st = p + lane < n_seqs ? starts[p + lane] : n;
+        const bool hit = st < base + 32;
+        const unsigned smask = __reduce_or_sync(0xffffffffu, hit ? 1u << (int)(st - base) : 0u);
+        p += __popc(__ballot_sync(0xffffffffu, hit));
+        const int cnt = (int)min((int64_t)32, e - base);
+        int zi = 0;
+        for (int j = 0; j < cnt; ++j) {
+            const double u = __shfl_sync(0xffffffffu, u_mine, j);
+            s = inv_cdf(tab + ((smask >> j) & 1u ? 0 : s + 1) * (KP + 1), u, KP);
+            if (WRITE_Z && lane == j) zi = s;
+        }
+        if (WRITE_Z && lane < cnt) z[base + lane] = zi;
+    }
+    if (!WRITE_Z && lane < K) maps[(int64_t)c * K + lane] = (uint8_t)s;
+}
+
+// Phase B in one CTA of 1024 threads, on maps staged in shared memory (a chain of dependent global loads would cost one
+// L2 round trip per chunk): the nch maps are cut into nseg segments; thread (seg, s) composes its segment's maps from s,
+// thread 0 sweeps the nseg segment maps, and thread seg then writes in[c] along its segment.
+__global__ void __launch_bounds__(1024) hmm_chain_sweep_kernel(const uint8_t* __restrict__ maps, const int nch, const int K,
+                                                               const int nseg, uint8_t* __restrict__ in) {
+    extern __shared__ uint4 sweep_s[];
+    uint8_t* mp = reinterpret_cast<uint8_t*>(sweep_s);          // [nch][K] padded to 16 bytes | [nseg][K] | [nseg]
+    const int mbytes = (nch * K + 15) & ~15;
+    uint8_t* segm = mp + mbytes;
+    uint8_t* segin = segm + nseg * K;
+    for (int o = threadIdx.x; o < mbytes / 16; o += blockDim.x) sweep_s[o] = reinterpret_cast<const uint4*>(maps)[o];
+    __syncthreads();
+    const int t = threadIdx.x, sl = (nch + nseg - 1) / nseg;
+    const int seg = t / K, s0 = t - seg * K;
+    if (seg < nseg) {
+        int s = s0;
+        for (int c = seg * sl; c < min(nch, seg * sl + sl); ++c) s = mp[c * K + s];
+        segm[seg * K + s0] = (uint8_t)s;
+    }
+    __syncthreads();
+    if (t == 0) {
+        int s = 0;                                              // chunk 0 begins with a sequence start: any state
+        for (int q = 0; q < nseg; ++q) {
+            segin[q] = (uint8_t)s;
+            s = segm[q * K + s];
+        }
+    }
+    __syncthreads();
+    if (t < nseg) {
+        int s = segin[t];
+        for (int c = t * sl; c < min(nch, t * sl + sl); ++c) {
+            in[c] = (uint8_t)s;
+            s = mp[c * K + s];
+        }
+    }
+}
+
+// Emission: one thread per element, x_i = mu_{z_i} + L_{z_i} eps_i (64 threads: [64][D + 1] doubles of scratch, D <= 256).
+__global__ void __launch_bounds__(64) hmm_emit_kernel(double* __restrict__ x, const int32_t* __restrict__ z, const int64_t n,
+                                                      const int D, const double* __restrict__ mu,
+                                                      const double* __restrict__ chol, const unsigned long long seed) {
+    extern __shared__ double eps_s[];
+    const int64_t i = (int64_t)blockIdx.x * 64 + threadIdx.x;
+    if (i >= n) return;
+    const uint2 key = make_uint2((uint32_t)seed, (uint32_t)(seed >> 32));
+    gauss_sample(x, i, eps_s + threadIdx.x * (D + 1), D, mu, chol, (unsigned long long)i, key, HMM_GEN_TAG,
+                 [&](double) { return (int)z[i]; });
+}
+
+// Workspace of bgmm_hmm_gen_sample (bytes, 256-aligned parts): starts [n_seqs] int64 | maps [nch][K] | in [nch].
+struct HmmGenWs {
+    int64_t nch, starts, maps, in, total;
+};
+inline int64_t align256(int64_t v) { return (v + 255) & ~int64_t(255); }
+inline bool hmm_gen_ws(int K, int64_t n, int64_t n_seqs, int64_t chunk_len, HmmGenWs& w) {
+    if (K <= 0 || K > 32 || n < 0) return false;
+    const int64_t L = chunk_len == 0 ? hmm_chunk_len(n) : chunk_len;
+    if (L <= 0) return false;
+    w.nch = (n + L - 1) / L;
+    if (w.nch > HMM_GEN_MAX_CHUNKS) return false;
+    w.starts = 0;
+    w.maps = align256((n_seqs > 1 ? n_seqs : 1) * 8);
+    w.in = w.maps + align256(w.nch * K);
+    w.total = w.in + align256(w.nch);
+    return true;
 }
 
 }  // namespace bgmm
@@ -135,6 +295,76 @@ extern "C" int bgmm_gen_sample(double* x_out, int32_t* z_out, int64_t n, int K, 
     gen_sample_kernel<<<(unsigned)((n + 127) / 128), 128, smem, (cudaStream_t)stream>>>(x_out, z_out, n, K, D, cdf, mu, chol,
                                                                                         (unsigned long long)seed, row_offset);
     return check_cuda(cudaGetLastError(), "gen_sample_kernel launch");
+}
+
+extern "C" int64_t bgmm_hmm_gen_workspace_bytes(int K, int64_t n, int64_t n_seqs, int64_t chunk_len) {
+    HmmGenWs w;
+    return hmm_gen_ws(K, n, n_seqs, chunk_len, w) ? w.total : 0;
+}
+
+extern "C" int bgmm_hmm_gen_sample(double* x_out, int32_t* z_out, int64_t n, int K, int D, const double* cdf, const double* mu,
+                                   const double* chol, const int64_t* seq_starts, int64_t n_seqs, uint64_t seed,
+                                   int64_t chunk_len, void* workspace, void* stream) {
+    HmmGenWs w;
+    if (seq_starts == nullptr || n_seqs < 1) n_seqs = 1;
+    if (n < 0 || K <= 0 || K > 32 || D <= 0 || D > 256 || chunk_len < 0 || cdf == nullptr || mu == nullptr ||
+        chol == nullptr || ((x_out == nullptr || z_out == nullptr || workspace == nullptr) && n > 0)) {
+        set_error("bgmm_hmm_gen_sample: bad argument (n=%lld K=%d D=%d; K <= 32, D <= 256)", (long long)n, K, D);
+        return BGMM_EINVAL;
+    }
+    if (!hmm_gen_ws(K, n, n_seqs, chunk_len, w)) {
+        set_error("bgmm_hmm_gen_sample: chunk_len=%lld gives more than %d chunks of n=%lld", (long long)chunk_len,
+                  HMM_GEN_MAX_CHUNKS, (long long)n);
+        return BGMM_EINVAL;
+    }
+    if (seq_starts != nullptr && n_seqs > 1) {
+        bool ok = seq_starts[0] == 0 && n_seqs <= n;
+        for (int64_t q = 1; ok && q < n_seqs; ++q) ok = seq_starts[q] > seq_starts[q - 1] && seq_starts[q] < n;
+        if (!ok) {
+            set_error("bgmm_hmm_gen_sample: seq_starts must begin with 0, increase strictly and stay below n=%lld",
+                      (long long)n);
+            return BGMM_EINVAL;
+        }
+    }
+    if (n == 0) return BGMM_OK;
+    cudaStream_t st = (cudaStream_t)stream;
+    uint8_t* ws = static_cast<uint8_t*>(workspace);
+    int64_t* starts = reinterpret_cast<int64_t*>(ws + w.starts);
+    int rc = n_seqs > 1 ? check_cuda(cudaMemcpyAsync(starts, seq_starts, sizeof(int64_t) * n_seqs, cudaMemcpyHostToDevice, st),
+                                     "cudaMemcpyAsync(seq_starts)")
+                        : check_cuda(cudaMemsetAsync(starts, 0, sizeof(int64_t), st), "cudaMemsetAsync(seq_starts)");
+    if (rc) return rc;
+    const int KP = pow2_ceil(K), nch = (int)w.nch;
+    const int64_t L = chunk_len == 0 ? hmm_chunk_len(n) : chunk_len;
+    const size_t tab_smem = sizeof(double) * (K + 1) * (KP + 1);
+    const unsigned grid = (unsigned)((nch + 7) / 8);
+    uint8_t* maps = ws + w.maps;
+    uint8_t* in = ws + w.in;
+    hmm_chain_kernel<false><<<grid, 256, tab_smem, st>>>(n, K, KP, L, nch, cdf, starts, n_seqs, (unsigned long long)seed,
+                                                         maps, nullptr, nullptr);
+    if ((rc = check_cuda(cudaGetLastError(), "hmm_chain_kernel<maps> launch"))) return rc;
+    int nseg = 1;
+    while ((nseg + 1) * (nseg + 1) <= nch) ++nseg;              // ~sqrt(nch) segments of ~sqrt(nch) maps
+    nseg = min(nseg, 1024 / K);
+    const size_t sweep_smem = (size_t)((nch * K + 15) & ~15) + (size_t)nseg * (K + 1);
+    if (sweep_smem > 48 * 1024) {
+        rc = check_cuda(cudaFuncSetAttribute(hmm_chain_sweep_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sweep_smem),
+                        "cudaFuncSetAttribute(hmm_chain_sweep_kernel)");
+        if (rc) return rc;
+    }
+    hmm_chain_sweep_kernel<<<1, 1024, sweep_smem, st>>>(maps, nch, K, nseg, in);
+    if ((rc = check_cuda(cudaGetLastError(), "hmm_chain_sweep_kernel launch"))) return rc;
+    hmm_chain_kernel<true><<<grid, 256, tab_smem, st>>>(n, K, KP, L, nch, cdf, starts, n_seqs, (unsigned long long)seed,
+                                                        nullptr, in, z_out);
+    if ((rc = check_cuda(cudaGetLastError(), "hmm_chain_kernel<z> launch"))) return rc;
+    const size_t emit_smem = sizeof(double) * 64 * (size_t)(D + 1);
+    if (emit_smem > 48 * 1024) {
+        rc = check_cuda(cudaFuncSetAttribute(hmm_emit_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)emit_smem),
+                        "cudaFuncSetAttribute(hmm_emit_kernel)");
+        if (rc) return rc;
+    }
+    hmm_emit_kernel<<<(unsigned)((n + 63) / 64), 64, emit_smem, st>>>(x_out, z_out, n, D, mu, chol, (unsigned long long)seed);
+    return check_cuda(cudaGetLastError(), "hmm_emit_kernel launch");
 }
 
 extern "C" int bgmm_pred_logdensity(const double* lnrho, int64_t n, int K, const double* acst, const double* ck,

@@ -42,13 +42,6 @@ struct ScanPlan {
 };
 
 
-// Chunk length: <= 4096 chunks (the length of the sequential phase B), at least 32 elements each.
-__host__ __device__ inline int hmm_chunk_len(int64_t n) {
-    int64_t L = (n + 4095) / 4096;
-    if (L < 32) L = 32;
-    return (int)((L + 7) & ~int64_t(7));
-}
-
 template <int KP>
 __device__ __forceinline__ double group_sum(double v) {
 #pragma unroll

@@ -20,7 +20,14 @@ inside a sequence), E ln p(z) / E ln q(z) take gamma summed over the sequence st
 sequence.  The per-element arrays keep their (N, K) / (N,) shapes over the concatenated rows.  `lengths=None` and
 `lengths=[N]` are the single-sequence path.
 
-Additive, defaulted options (they do not exist in the reference): `device`, `lengths`.
+`GenModel` is the reference's generative model (pi ~ Dir(h_eta_vec), every row of A ~ Dir(h_zeta_vecs[k]), (mu_k,
+Lambda_k) ~ Gauss-Wishart, z a Markov chain, x ~ N(mu_z, Lambda_z^-1)).  `gen_sample(n)` is the reference's per-element
+loop with `self.rng`; `gen_sample(n, device="cuda:i")` draws the same distribution on the device (bgmm_hmm_gen_sample:
+the chain sampled exactly by composing per-element transition maps over chunks, counter-based Philox, NOT numpy's
+stream; c_num_classes <= 32 and c_degree <= 256 there, no CPU fallback).
+
+Additive, defaulted options (they do not exist in the reference): `device`, `lengths` (of `LearnModel.update_posterior`,
+`LearnModel.estimate_latent_vars` and `GenModel.gen_sample`), `as_numpy` (of `GenModel.gen_sample`).
 """
 import warnings
 
@@ -36,7 +43,9 @@ from .gaussianmixture import _LazyDeviceArray
 
 MAX_NUM_CLASSES, MAX_DEGREE = 32, 128        # limits of the device path (bgmm_hmm_supported)
 
-__all__ = ["LearnModel"]
+GEN_MAX_NUM_CLASSES, GEN_MAX_DEGREE = 32, 256   # limits of the device sampler (bgmm_hmm_gen_sample)
+
+__all__ = ["GenModel", "LearnModel"]
 
 _HN_NAMES = ("hn_eta_vec", "hn_zeta_vecs", "hn_m_vecs", "hn_kappas", "hn_nus", "hn_w_mats", "hn_w_mats_inv")
 _LAZY = ("_ln_rho", "alpha_vecs", "beta_vecs", "gamma_vecs", "_cs")
@@ -52,6 +61,229 @@ def _lazy_property(name):
         getattr(self, slot).set_host(value)
 
     return property(getter, setter)
+
+
+def _inverse_cdf_table(pi_vec, a_mat):
+    """The (K + 1, K) inverse-CDF table of bgmm_hmm_gen_sample: row 0 for pi, row 1 + s for row s of A.  Each row is the
+    cumulative sum of its probabilities with the entry of its last positive-probability state set to 2.0; state k is
+    drawn for u in (0, 1) as the first k with u <= row[k], so a zero-probability state is never drawn, even when the
+    rounded cumulative sum ends below 1 and u falls above it."""
+    p = np.vstack([pi_vec[np.newaxis, :], a_mat])
+    cdf = np.cumsum(p, axis=1)
+    last = p.shape[1] - 1 - np.argmax(p[:, ::-1] > 0, axis=1)
+    cdf[np.arange(p.shape[0]), last] = 2.0
+    return cdf
+
+
+class GenModel(base.Generative):
+    """The stochastic data generative model of the Bayesian hidden Markov model with Gaussian emissions: pi ~
+    Dir(h_eta_vec), a_mat[k] ~ Dir(h_zeta_vecs[k]), (mu_k, Lambda_k) ~ Gauss-Wishart(h_m_vecs, h_kappas, h_nus, h_w_mats),
+    z_0 ~ Cat(pi), z_i ~ Cat(a_mat[z_{i-1}]), x_i ~ N(mu_{z_i}, Lambda_{z_i}^-1).  Same constructor, parameters and
+    methods as the reference class.
+
+    Parameters
+    ----------
+    c_num_classes, c_degree : int
+        number of hidden states K and data dimension D (positive)
+    pi_vec, a_mat, mu_vecs, lambda_mats : optional (keyword only)
+        parameters; defaults 1/K, 1/K, 0, I
+    h_eta_vec, h_zeta_vecs, h_m_vecs, h_kappas, h_nus, h_w_mats : optional (keyword only)
+        hyperparameters of the prior; defaults 1/2, 1/2, 0, 1, D, I (those of LearnModel's h0_*)
+    seed : {None, int}
+        seed of `numpy.random.default_rng`
+
+    `gen_sample(n)` is the reference's per-element loop (`rng.choice` + `rng.multivariate_normal`); `gen_sample(n,
+    device="cuda:0")` draws the same distribution on the device (bgmm_hmm_gen_sample; counter-based Philox, NOT numpy's
+    stream) and can leave the sample there (`as_numpy=False`)."""
+
+    def __init__(self, c_num_classes, c_degree, *, pi_vec=None, a_mat=None, mu_vecs=None, lambda_mats=None,
+                 h_eta_vec=None, h_zeta_vecs=None, h_m_vecs=None, h_kappas=None, h_nus=None, h_w_mats=None, seed=None):
+        self.c_degree = _check.pos_int(c_degree, 'c_degree', ParameterFormatError)
+        self.c_num_classes = _check.pos_int(c_num_classes, 'c_num_classes', ParameterFormatError)
+        self.rng = np.random.default_rng(seed)
+        K, D = self.c_num_classes, self.c_degree
+        self.pi_vec = np.ones(K) / K
+        self.a_mat = np.ones((K, K)) / K
+        self.mu_vecs = np.zeros((K, D))
+        self.lambda_mats = np.tile(np.eye(D), (K, 1, 1))
+        self.h_eta_vec = np.ones(K) / 2
+        self.h_zeta_vecs = np.ones((K, K)) / 2
+        self.h_m_vecs = np.zeros((K, D))
+        self.h_kappas = np.ones(K)
+        self.h_nus = np.ones(K) * D
+        self.h_w_mats = np.tile(np.eye(D), (K, 1, 1))
+        self.set_params(pi_vec, a_mat, mu_vecs, lambda_mats)
+        self.set_h_params(h_eta_vec, h_zeta_vecs, h_m_vecs, h_kappas, h_nus, h_w_mats)
+
+    def get_constants(self):
+        """{"c_num_classes", "c_degree"}."""
+        return {"c_num_classes": self.c_num_classes, "c_degree": self.c_degree}
+
+    def _shape(self, arr, name, shape):
+        if arr.shape != shape:
+            raise ParameterFormatError(f"{name}.shape must be {shape} (c_num_classes = {self.c_num_classes}, "
+                                       f"c_degree = {self.c_degree}): {name}.shape = {arr.shape}")
+
+    def set_h_params(self, h_eta_vec=None, h_zeta_vecs=None, h_m_vecs=None, h_kappas=None, h_nus=None, h_w_mats=None):
+        """Set the hyperparameters of the prior (arrays broadcast to their attribute's shape)."""
+        D = self.c_degree
+        if h_eta_vec is not None:
+            _check.pos_floats(h_eta_vec, 'h_eta_vec', ParameterFormatError)
+            self.h_eta_vec[:] = h_eta_vec
+        if h_zeta_vecs is not None:
+            _check.pos_floats(h_zeta_vecs, 'h_zeta_vecs', ParameterFormatError)
+            self.h_zeta_vecs[:] = h_zeta_vecs
+        if h_m_vecs is not None:
+            _check.float_vecs(h_m_vecs, 'h_m_vecs', ParameterFormatError)
+            if h_m_vecs.shape[-1] != D:
+                raise ParameterFormatError("h_m_vecs.shape[-1] must coincide with self.c_degree: "
+                                           f"h_m_vecs.shape[-1] = {h_m_vecs.shape[-1]}, self.c_degree = {D}")
+            self.h_m_vecs[:] = h_m_vecs
+        if h_kappas is not None:
+            _check.pos_floats(h_kappas, 'h_kappas', ParameterFormatError)
+            self.h_kappas[:] = h_kappas
+        if h_nus is not None:
+            _check.pos_floats(h_nus, 'h_nus', ParameterFormatError)
+            if np.any(h_nus <= D - 1):
+                raise ParameterFormatError("All the values of h_nus must be greater than self.c_degree - 1: "
+                                           f"self.c_degree = {D}, h_nus = {h_nus}")
+            self.h_nus[:] = h_nus
+        if h_w_mats is not None:
+            _check.pos_def_sym_mats(h_w_mats, 'h_w_mats', ParameterFormatError)
+            if h_w_mats.shape[-1] != D:
+                raise ParameterFormatError("h_w_mats.shape[-1] must coincide with self.c_degree: "
+                                           f"h_w_mats.shape[-1] = {h_w_mats.shape[-1]}, self.c_degree = {D}")
+            self.h_w_mats[:] = h_w_mats
+        return self
+
+    def get_h_params(self):
+        """Live references to the hyperparameters."""
+        return {"h_eta_vec": self.h_eta_vec, "h_zeta_vecs": self.h_zeta_vecs, "h_m_vecs": self.h_m_vecs,
+                "h_kappas": self.h_kappas, "h_nus": self.h_nus, "h_w_mats": self.h_w_mats}
+
+    def gen_params(self):
+        """Draw pi ~ Dir(h_eta_vec), then every row of A ~ Dir(h_zeta_vecs[k]), then (Lambda_k, mu_k) for every k as
+        `gaussianmixture.GenModel.gen_params` does, all from `self.rng`."""
+        self.pi_vec[:] = self.rng.dirichlet(self.h_eta_vec)
+        for k in range(self.c_num_classes):
+            self.a_mat[k] = self.rng.dirichlet(self.h_zeta_vecs[k])
+        for k in range(self.c_num_classes):
+            self.lambda_mats[k] = ss_wishart.rvs(df=self.h_nus[k], scale=self.h_w_mats[k], random_state=self.rng)
+            self.mu_vecs[k] = self.rng.multivariate_normal(mean=self.h_m_vecs[k],
+                                                           cov=np.linalg.inv(self.h_kappas[k] * self.lambda_mats[k]))
+        return self
+
+    def set_params(self, pi_vec=None, a_mat=None, mu_vecs=None, lambda_mats=None):
+        """Set the parameters of the sampling distribution: pi_vec (K,) and every row of a_mat (K, K) non-negative and
+        summing to 1, mu_vecs (K, D), lambda_mats (K, D, D) positive-definite symmetric."""
+        K, D = self.c_num_classes, self.c_degree
+        if pi_vec is not None:
+            _check.float_vec_sum_1(pi_vec, 'pi_vec', ParameterFormatError)
+            self._shape(pi_vec, 'pi_vec', (K,))
+            if np.any(pi_vec < 0):
+                raise ParameterFormatError(f"pi_vec must be non-negative: pi_vec = {pi_vec}")
+            self.pi_vec[:] = pi_vec
+        if a_mat is not None:
+            _check.float_vecs_sum_1(a_mat, 'a_mat', ParameterFormatError)
+            self._shape(a_mat, 'a_mat', (K, K))
+            if np.any(a_mat < 0):
+                raise ParameterFormatError(f"a_mat must be non-negative: a_mat = {a_mat}")
+            self.a_mat[:] = a_mat
+        if mu_vecs is not None:
+            _check.float_vecs(mu_vecs, 'mu_vecs', ParameterFormatError)
+            self._shape(mu_vecs, 'mu_vecs', (K, D))
+            self.mu_vecs[:] = mu_vecs
+        if lambda_mats is not None:
+            _check.pos_def_sym_mats(lambda_mats, 'lambda_mats', ParameterFormatError)
+            self._shape(lambda_mats, 'lambda_mats', (K, D, D))
+            self.lambda_mats[:] = lambda_mats
+        return self
+
+    def get_params(self):
+        """Live references to pi_vec, a_mat, mu_vecs, lambda_mats."""
+        return {"pi_vec": self.pi_vec, "a_mat": self.a_mat, "mu_vecs": self.mu_vecs, "lambda_mats": self.lambda_mats}
+
+    def gen_sample(self, sample_length, *, lengths=None, device=None, as_numpy=True):
+        """Generate a sample -> (x (sample_length, c_degree) float64, z (sample_length, c_num_classes) one-hot int).
+
+        device=None: the reference's loop with `self.rng`: z_0 = rng.choice(K, p=pi_vec), then x_0 =
+        rng.multivariate_normal(mu[z_0], Lambda[z_0]^-1); for i >= 1, z_i = rng.choice(K, p=a_mat[z_{i-1}]), then that
+        element's multivariate_normal.
+        lengths : optional (extension, keyword only) 1-D sequence of positive ints summing to sample_length: that many
+            independent sequences, concatenated, each starting from pi.  On the host the loop above runs once per
+            sequence in order, so lengths=[sample_length] is exactly lengths=None.
+        device="cuda:i": one call of bgmm_hmm_gen_sample (same distribution, its own counter-based stream seeded by one
+            `self.rng.integers` draw; c_num_classes <= 32, c_degree <= 256, else ParameterFormatError); with
+            as_numpy=False, x (float64) and the state indices z (int32, NOT one-hot) stay on the device as torch tensors.
+        """
+        _check.pos_int(sample_length, 'sample_length', DataFormatError)
+        starts = LearnModel._seq_starts(lengths, sample_length)
+        K, D = self.c_num_classes, self.c_degree
+        cov = np.linalg.inv(self.lambda_mats)
+        if device is None:
+            z = np.zeros((sample_length, K), dtype=int)
+            x = np.empty((sample_length, D))
+            first = np.zeros(sample_length, dtype=bool)
+            first[0 if starts is None else starts] = True
+            k = 0
+            for i in range(sample_length):
+                k = self.rng.choice(K, p=self.pi_vec if first[i] else self.a_mat[k])
+                z[i, k] = 1
+                x[i] = self.rng.multivariate_normal(mean=self.mu_vecs[k], cov=cov[k])
+            return x, z
+        if K > GEN_MAX_NUM_CLASSES or D > GEN_MAX_DEGREE:
+            raise ParameterFormatError(
+                f"gen_sample on the device supports c_num_classes <= {GEN_MAX_NUM_CLASSES} and c_degree <= "
+                f"{GEN_MAX_DEGREE} (got {K}, {D}); there is no CPU fallback")
+        import torch
+        from . import _lib
+        lib = _lib.load()
+        dev = torch.device(device)
+        seed = int(self.rng.integers(0, 2 ** 63 - 1))
+        n_seqs = 1 if starts is None else starts.size
+        starts_ptr = None if starts is None else starts.ctypes.data
+        with torch.cuda.device(dev):
+            consts = [torch.as_tensor(np.ascontiguousarray(a, dtype=np.float64)).to(dev)
+                      for a in (_inverse_cdf_table(self.pi_vec, self.a_mat), self.mu_vecs, np.linalg.cholesky(cov))]
+            x_dev = torch.empty((sample_length, D), dtype=torch.float64, device=dev)
+            z_dev = torch.empty(sample_length, dtype=torch.int32, device=dev)
+            ws = torch.empty(lib.bgmm_hmm_gen_workspace_bytes(K, sample_length, n_seqs, 0), dtype=torch.uint8, device=dev)
+            _lib.check(lib.bgmm_hmm_gen_sample(x_dev.data_ptr(), z_dev.data_ptr(), sample_length, K, D,
+                                               consts[0].data_ptr(), consts[1].data_ptr(), consts[2].data_ptr(),
+                                               starts_ptr, n_seqs, seed, 0, ws.data_ptr(),
+                                               torch.cuda.current_stream(dev).cuda_stream), "bgmm_hmm_gen_sample")
+            if not as_numpy:
+                torch.cuda.current_stream(dev).synchronize()
+                return x_dev, z_dev
+            return x_dev.cpu().numpy(), np.eye(K, dtype=int)[z_dev.cpu().numpy()]
+
+    def save_sample(self, filename, sample_length):
+        """gen_sample, then np.savez_compressed(filename, x=x, z=z)."""
+        x, z = self.gen_sample(sample_length)
+        np.savez_compressed(filename, x=x, z=z)
+
+    def visualize_model(self, sample_length=200):
+        """Print the parameters and plot a sample (x against time for c_degree 1, the plane for c_degree 2, coloured by
+        state) for c_degree <= 2; needs matplotlib."""
+        if self.c_degree > 2:
+            raise ParameterFormatError("if c_degree > 2, it is impossible to visualize the model by this function.")
+        print(f"pi_vec:\n {self.pi_vec}")
+        print(f"a_mat:\n {self.a_mat}")
+        print(f"mu_vecs:\n {self.mu_vecs}")
+        print(f"lambda_mats:\n {self.lambda_mats}")
+        import matplotlib.pyplot as plt
+        sample, z = self.gen_sample(sample_length)
+        states = z.argmax(axis=1)
+        fig, axes = plt.subplots()
+        if self.c_degree == 1:
+            axes.plot(np.arange(sample_length), sample[:, 0], color="gray", linewidth=0.5)
+            axes.scatter(np.arange(sample_length), sample[:, 0], c=states, cmap="tab10")
+            axes.set_xlabel("time"); axes.set_ylabel("x")
+        else:
+            axes.plot(sample[:, 0], sample[:, 1], color="gray", linewidth=0.5)
+            axes.scatter(sample[:, 0], sample[:, 1], c=states, cmap="tab10")
+            axes.set_xlabel("x[0]"); axes.set_ylabel("x[1]")
+        plt.show()
 
 
 class LearnModel(base.Posterior, base.PredictiveMixin):

@@ -233,6 +233,26 @@ int bgmm_dirichlet1(double* r_out, int64_t n, int K, uint64_t seed, int64_t row_
  *   the global row index row_offset + i).  Same distribution as the reference, NOT numpy's random stream.  D <= 256. */
 int bgmm_gen_sample(double* x_out, int32_t* z_out, int64_t n, int K, int D, const double* cdf, const double* mu,
                     const double* chol, uint64_t seed, int64_t row_offset, void* stream);
+/* bgmm_hmm_gen_sample: `hiddenmarkovnormal.GenModel.gen_sample` on the device: z_out[n] (int32 state indices) is a Markov
+ *   chain, z_0 ~ pi and z_i ~ A[z_{i-1}], restarting from pi at every sequence start; x_out[n][D] = mu[z] + chol[z] eps as in
+ *   bgmm_gen_sample.  Same distribution as the host loop, NOT numpy's random stream.  K <= 32, D <= 256.
+ *   cdf[(K+1)][K] (device): row 0 the inverse-CDF table of pi, row 1 + s that of row s of A.  Each row is the cumulative
+ *   sum of its probabilities with the entry of its LAST positive-probability state set to 2.0; state k is drawn for
+ *   uniform u in (0, 1) as the first k with u <= cdf[row][k].  A zero-probability state is then never drawn, even when the
+ *   rounded cumulative sum ends below 1 and u falls above it.
+ *   seq_starts[n_seqs] (HOST, int64): first rows of the sequences, starting with 0, strictly increasing, below n; NULL or
+ *   n_seqs = 1 for one sequence.  It is copied into the workspace with cudaMemcpyAsync (a pinned array must stay valid
+ *   until the stream reaches the copy).
+ *   Philox4x32-10 keyed by `seed`, counter = (global element index, word, own tag): word 0 gives the state's uniform, words
+ *   1.. the normals, so the sample does not depend on the chunking or on how the rows are split into sequences.
+ *   The chain is sampled exactly by composing the per-element transition maps over chunks of chunk_len elements (0 = the
+ *   default, at most 4096 chunks; a chunk_len giving more than 4096 chunks is BGMM_EINVAL); the result does not depend on
+ *   chunk_len.  workspace: bgmm_hmm_gen_workspace_bytes(K, n, n_seqs, chunk_len) bytes of device memory (0 for a bad
+ *   argument). */
+int64_t bgmm_hmm_gen_workspace_bytes(int K, int64_t n, int64_t n_seqs, int64_t chunk_len);
+int bgmm_hmm_gen_sample(double* x_out, int32_t* z_out, int64_t n, int K, int D, const double* cdf, const double* mu,
+                        const double* chol, const int64_t* seq_starts, int64_t n_seqs, uint64_t seed, int64_t chunk_len,
+                        void* workspace, void* stream);
 
 /* ---- 5th-generation tensor cores (fp32 mode) ----
  * bgmm_tc_selftest: D[128][N] = A[128][Kd] . B[N][Kd]^T with tcgen05.mma kind::tf32 (operands staged in shared memory in the
