@@ -9,7 +9,7 @@ _PKG_DIR = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(_PKG_DIR, "libbgmm.so")
 
 # constants mirrored from include/bgmm.h (checked against bgmm_abi_version at load time)
-ABI_VERSION = 4
+ABI_VERSION = 5
 F64, F32 = 0, 1
 PASS_AUTO, PASS_SIMPLE, PASS_DMMA, PASS_F32, PASS_LARGE, PASS_DIRECT, PASS_TF32 = 0, 1, 2, 3, 4, 5, 6
 SMALL_FEATURES, SMALL_ITERATE, SMALL_STATS = 0, 1, 2
@@ -45,6 +45,8 @@ def load():
     lib.bgmm_abi_version.argtypes = []
     lib.bgmm_last_error.restype = ctypes.c_char_p
     lib.bgmm_last_error.argtypes = []
+    lib.bgmm_launch_count.restype = i64
+    lib.bgmm_launch_count.argtypes = []
     lib.bgmm_robust_threshold.restype = f64
     lib.bgmm_robust_threshold.argtypes = []
     lib.bgmm_set_robust_threshold.restype = f64

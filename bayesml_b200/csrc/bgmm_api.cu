@@ -8,6 +8,7 @@
 namespace bgmm {
 
 static thread_local char g_err[512] = "";
+thread_local int64_t g_launches = 0;
 static double g_robust_threshold = 2.0e4;
 
 double robust_threshold() { return g_robust_threshold; }
@@ -96,6 +97,7 @@ extern "C" double bgmm_set_robust_threshold(double t) {
     return old;
 }
 extern "C" const char* bgmm_last_error(void) { return g_err; }
+extern "C" int64_t bgmm_launch_count(void) { return g_launches; }
 
 extern "C" int bgmm_layout(int K, int D, int hist_len, int64_t* off, int64_t* poff) {
     if (K <= 0 || D <= 0 || hist_len < 1 || off == nullptr || poff == nullptr) {
@@ -141,9 +143,9 @@ extern "C" int bgmm_colsum(const void* x, int64_t n, int D, int dtype, double* o
     const int64_t stride = colsum_stride(D), total = n * D;
     const int grid = (int)((stride + PREP_THREADS - 1) / PREP_THREADS);
     cudaStream_t s = (cudaStream_t)stream;
-    if (dtype == BGMM_F64) colsum_partial_kernel<double><<<grid, PREP_THREADS, 0, s>>>((const double*)x, total, stride, ws);
-    else colsum_partial_kernel<float><<<grid, PREP_THREADS, 0, s>>>((const float*)x, total, stride, ws);
-    colsum_final_kernel<<<D, 32, 0, s>>>(ws, stride, D, out);
+    if (dtype == BGMM_F64) launch(colsum_partial_kernel<double>, grid, PREP_THREADS, 0, s, (const double*)x, total, stride, ws);
+    else launch(colsum_partial_kernel<float>, grid, PREP_THREADS, 0, s, (const float*)x, total, stride, ws);
+    launch(colsum_final_kernel, D, 32, 0, s, ws, stride, D, out);
     return check_cuda(cudaGetLastError(), "bgmm_colsum launch");
 }
 
@@ -159,13 +161,13 @@ extern "C" int bgmm_center(const void* x, int dtype_in, void* y, int dtype_out, 
     const int grid = (int)(grid64 < 148 * 16 ? grid64 : 148 * 16);
     cudaStream_t s = (cudaStream_t)stream;
     if (dtype_in == BGMM_F64 && dtype_out == BGMM_F64)
-        center_kernel<double, double><<<grid, PREP_THREADS, 0, s>>>((const double*)x, (double*)y, total, D, c);
+        launch(center_kernel<double, double>, grid, PREP_THREADS, 0, s, (const double*)x, (double*)y, total, D, c);
     else if (dtype_in == BGMM_F64 && dtype_out == BGMM_F32)
-        center_kernel<double, float><<<grid, PREP_THREADS, 0, s>>>((const double*)x, (float*)y, total, D, c);
+        launch(center_kernel<double, float>, grid, PREP_THREADS, 0, s, (const double*)x, (float*)y, total, D, c);
     else if (dtype_in == BGMM_F32 && dtype_out == BGMM_F32)
-        center_kernel<float, float><<<grid, PREP_THREADS, 0, s>>>((const float*)x, (float*)y, total, D, c);
+        launch(center_kernel<float, float>, grid, PREP_THREADS, 0, s, (const float*)x, (float*)y, total, D, c);
     else if (dtype_in == BGMM_F32 && dtype_out == BGMM_F64)
-        center_kernel<float, double><<<grid, PREP_THREADS, 0, s>>>((const float*)x, (double*)y, total, D, c);
+        launch(center_kernel<float, double>, grid, PREP_THREADS, 0, s, (const float*)x, (double*)y, total, D, c);
     else { set_error("bgmm_center: bad dtype"); return BGMM_EINVAL; }
     return check_cuda(cudaGetLastError(), "bgmm_center launch");
 }

@@ -189,6 +189,25 @@ __device__ __forceinline__ void pdl_trigger() { asm volatile("griddepcontrol.lau
 __device__ __forceinline__ void pdl_wait() { asm volatile("griddepcontrol.wait;" ::: "memory"); }
 bool pdl_enabled();
 
+// Kernels launched from this host thread (bgmm_launch_count).  Every kernel of libbgmm is launched through launch() or
+// launch_pdl(), which count it, so the library, not its callers, knows what each entry point launched.
+extern thread_local int64_t g_launches;
+
+template <typename... KArgs, typename... Args>
+inline cudaError_t launch_counted(const cudaLaunchConfig_t& cfg, void (*kern)(KArgs...), Args... args) {
+    const cudaError_t e = cudaLaunchKernelEx(&cfg, kern, static_cast<KArgs>(args)...);
+    if (e == cudaSuccess) ++g_launches;
+    return e;
+}
+
+// A plain launch: no attributes, the kernel starts once its predecessor on the stream has completed.
+template <typename... KArgs, typename... Args>
+inline cudaError_t launch(void (*kern)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t stream, Args... args) {
+    cudaLaunchConfig_t cfg = {};
+    cfg.gridDim = grid; cfg.blockDim = block; cfg.dynamicSmemBytes = smem; cfg.stream = stream;
+    return launch_counted(cfg, kern, args...);
+}
+
 template <typename... KArgs, typename... Args>
 inline cudaError_t launch_pdl(void (*kern)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t stream, Args... args) {
     cudaLaunchConfig_t cfg = {};
@@ -198,7 +217,7 @@ inline cudaError_t launch_pdl(void (*kern)(KArgs...), dim3 grid, dim3 block, siz
     attr[0].val.programmaticStreamSerializationAllowed = 1;
     cfg.attrs = attr;
     cfg.numAttrs = pdl_enabled() ? 1 : 0;
-    return cudaLaunchKernelEx(&cfg, kern, static_cast<KArgs>(args)...);
+    return launch_counted(cfg, kern, args...);
 }
 
 // Publication of freshly reduced statistics to the peers (bgmm_comm.cu), executed by the LAST CTA of a reduction after its

@@ -292,8 +292,8 @@ extern "C" int bgmm_gen_sample(double* x_out, int32_t* z_out, int64_t n, int K, 
                             "cudaFuncSetAttribute(gen_sample_kernel)");
         if (rc) return rc;
     }
-    gen_sample_kernel<<<(unsigned)((n + 127) / 128), 128, smem, (cudaStream_t)stream>>>(x_out, z_out, n, K, D, cdf, mu, chol,
-                                                                                        (unsigned long long)seed, row_offset);
+    launch(gen_sample_kernel, (unsigned)((n + 127) / 128), 128, smem, (cudaStream_t)stream, x_out, z_out, n, K, D, cdf, mu, chol,
+           (unsigned long long)seed, row_offset);
     return check_cuda(cudaGetLastError(), "gen_sample_kernel launch");
 }
 
@@ -340,8 +340,8 @@ extern "C" int bgmm_hmm_gen_sample(double* x_out, int32_t* z_out, int64_t n, int
     const unsigned grid = (unsigned)((nch + 7) / 8);
     uint8_t* maps = ws + w.maps;
     uint8_t* in = ws + w.in;
-    hmm_chain_kernel<false><<<grid, 256, tab_smem, st>>>(n, K, KP, L, nch, cdf, starts, n_seqs, (unsigned long long)seed,
-                                                         maps, nullptr, nullptr);
+    launch(hmm_chain_kernel<false>, grid, 256, tab_smem, st, n, K, KP, L, nch, cdf, starts, n_seqs, (unsigned long long)seed,
+           maps, nullptr, nullptr);
     if ((rc = check_cuda(cudaGetLastError(), "hmm_chain_kernel<maps> launch"))) return rc;
     int nseg = 1;
     while ((nseg + 1) * (nseg + 1) <= nch) ++nseg;              // ~sqrt(nch) segments of ~sqrt(nch) maps
@@ -352,10 +352,10 @@ extern "C" int bgmm_hmm_gen_sample(double* x_out, int32_t* z_out, int64_t n, int
                         "cudaFuncSetAttribute(hmm_chain_sweep_kernel)");
         if (rc) return rc;
     }
-    hmm_chain_sweep_kernel<<<1, 1024, sweep_smem, st>>>(maps, nch, K, nseg, in);
+    launch(hmm_chain_sweep_kernel, 1, 1024, sweep_smem, st, maps, nch, K, nseg, in);
     if ((rc = check_cuda(cudaGetLastError(), "hmm_chain_sweep_kernel launch"))) return rc;
-    hmm_chain_kernel<true><<<grid, 256, tab_smem, st>>>(n, K, KP, L, nch, cdf, starts, n_seqs, (unsigned long long)seed,
-                                                        nullptr, in, z_out);
+    launch(hmm_chain_kernel<true>, grid, 256, tab_smem, st, n, K, KP, L, nch, cdf, starts, n_seqs, (unsigned long long)seed,
+           nullptr, in, z_out);
     if ((rc = check_cuda(cudaGetLastError(), "hmm_chain_kernel<z> launch"))) return rc;
     const size_t emit_smem = sizeof(double) * 64 * (size_t)(D + 1);
     if (emit_smem > 48 * 1024) {
@@ -363,7 +363,7 @@ extern "C" int bgmm_hmm_gen_sample(double* x_out, int32_t* z_out, int64_t n, int
                         "cudaFuncSetAttribute(hmm_emit_kernel)");
         if (rc) return rc;
     }
-    hmm_emit_kernel<<<(unsigned)((n + 63) / 64), 64, emit_smem, st>>>(x_out, z_out, n, D, mu, chol, (unsigned long long)seed);
+    launch(hmm_emit_kernel, (unsigned)((n + 63) / 64), 64, emit_smem, st, x_out, z_out, n, D, mu, chol, (unsigned long long)seed);
     return check_cuda(cudaGetLastError(), "hmm_emit_kernel launch");
 }
 
@@ -375,7 +375,7 @@ extern "C" int bgmm_pred_logdensity(const double* lnrho, int64_t n, int K, const
         return BGMM_EINVAL;
     }
     if (n == 0) return BGMM_OK;
-    pred_logdensity_kernel<<<(unsigned)((n + 7) / 8), 256, 0, (cudaStream_t)stream>>>(lnrho, n, K, acst, ck, hk, nuk, out);
+    launch(pred_logdensity_kernel, (unsigned)((n + 7) / 8), 256, 0, (cudaStream_t)stream, lnrho, n, K, acst, ck, hk, nuk, out);
     return check_cuda(cudaGetLastError(), "pred_logdensity_kernel launch");
 }
 
@@ -385,7 +385,7 @@ extern "C" int bgmm_dirichlet1(double* r_out, int64_t n, int K, uint64_t seed, i
         return BGMM_EINVAL;
     }
     if (n == 0) return BGMM_OK;
-    dirichlet1_kernel<<<(unsigned)((n + 255) / 256), 256, 0, (cudaStream_t)stream>>>(r_out, n, K, (unsigned long long)seed,
-                                                                                     row_offset);
+    launch(dirichlet1_kernel, (unsigned)((n + 255) / 256), 256, 0, (cudaStream_t)stream, r_out, n, K, (unsigned long long)seed,
+           row_offset);
     return check_cuda(cudaGetLastError(), "dirichlet1_kernel launch");
 }

@@ -847,18 +847,18 @@ static void launch_seq(const ScanPlan& sp, double* st, const Layout& L, double* 
     SeqRangeArg<SEQS> R{};
     if constexpr (SEQS) R = SeqRange{cbase, nullptr};
     if (!two_level_sweep(nsteps)) {
-        hmm_seq_kernel<KP, FWD, SEQS><<<1, SEQ_T, smem_seq, stream>>>(sp, st, L, hst, H, force, lv, R);
+        launch(hmm_seq_kernel<KP, FWD, SEQS>, 1, SEQ_T, smem_seq, stream, sp, st, L, hst, H, force, lv, R);
         return;
     }
     double* tg = B.seq2;                                   // [ngroups][K][K]
     double* lsg = tg + (int64_t)72 * K * K;                // [ngroups][K]
     double* vbg = lsg + (int64_t)72 * K;                   // [ngroups + 1][K]
     lv.mode = 1; lv.tg = tg; lv.lsg = lsg;
-    hmm_seq_kernel<KP, FWD, SEQS><<<dim3(ngroups, K), SEQ_T, smem_seq, stream>>>(sp, st, L, hst, H, force, lv, R);
+    launch(hmm_seq_kernel<KP, FWD, SEQS>, dim3(ngroups, K), SEQ_T, smem_seq, stream, sp, st, L, hst, H, force, lv, R);
     SeqLevel l2{2, ngroups - 1, ngroups, tg, lsg, vbg, nullptr, nullptr, nullptr};   // the last group's matrix is not needed
-    hmm_seq_kernel<KP, FWD, SEQS><<<1, SEQ_T, smem_seq, stream>>>(sp, st, L, hst, H, force, l2, SeqRangeArg<SEQS>{});   // group level: cbase 0
+    launch(hmm_seq_kernel<KP, FWD, SEQS>, 1, SEQ_T, smem_seq, stream, sp, st, L, hst, H, force, l2, SeqRangeArg<SEQS>{});   // group level: cbase 0
     lv.mode = 3; lv.tg = nullptr; lv.lsg = nullptr; lv.vbg = vbg;
-    hmm_seq_kernel<KP, FWD, SEQS><<<ngroups, SEQ_T, smem_seq, stream>>>(sp, st, L, hst, H, force, lv, R);
+    launch(hmm_seq_kernel<KP, FWD, SEQS>, ngroups, SEQ_T, smem_seq, stream, sp, st, L, hst, H, force, lv, R);
 }
 
 // Phase B of one direction over several sequences: sequences of one chunk need none; the others are swept in parallel
@@ -872,8 +872,8 @@ static void launch_seq_segs(const ScanPlan& sp, double* st, const Layout& L, dou
     const int64_t* segs = plan + 8 + 3 * plan[3] + 1;
     if (nshort > 0) {
         SeqLevel lv{0, 0, 0, B.tf, B.ls, B.vb, nullptr, nullptr, nullptr};
-        hmm_seq_kernel<KP, FWD, true><<<(unsigned)nshort, SEQ_T, smem_seq, stream>>>(sp, st, L, hst, H, force, lv,
-                                                                                     SeqRange{0, segs_dev});
+        launch(hmm_seq_kernel<KP, FWD, true>, (unsigned)nshort, SEQ_T, smem_seq, stream, sp, st, L, hst, H, force, lv,
+               SeqRange{0, segs_dev});
     }
     for (int64_t q = nshort; q < nshort + nlong; ++q)
         launch_seq<KP, FWD, true>(sp, st, L, hst, H, force, B, smem_seq, stream, (int)segs[2 * q], (int)segs[2 * q + 1] - 1);
@@ -899,19 +899,19 @@ static int launch_scan(const ScanPlan& sp, double* st, const Layout& L, double* 
     const unsigned gm = (unsigned)((sp.nch - 1 + HW - 1) / HW);          // basis runs: one warp per chunk
     // basis runs and sweeps only where a sequence has more than one chunk
     const bool multi = plan == nullptr ? sp.nch > 1 : plan[4] + plan[5] > 0;
-    if (multi) hmm_basis_mma_kernel<(KP >= 8 ? KP : 8), true, SEQS><<<gm, HT, 0, stream>>>(sp, st, L, hst, H, force, B, T);
+    if (multi) launch(hmm_basis_mma_kernel<(KP >= 8 ? KP : 8), true, SEQS>, gm, HT, 0, stream, sp, st, L, hst, H, force, B, T);
     if (plan == nullptr) launch_seq<KP, true, false>(sp, st, L, hst, H, force, B, smem_seq, stream, 0, sp.nch - 1);
     else launch_seq_segs<KP, true>(sp, st, L, hst, H, force, B, smem_seq, stream, plan, segs_dev);
-    hmm_window_kernel<KP, true, SEQS><<<gc, HT, 0, stream>>>(sp, st, L, hst, H, force, B, T);
-    hmm_fwd_kernel<KP, SEQS><<<gc, HT, 0, stream>>>(sp, st, L, hst, H, force, B, T);
-    hmm_cs_kernel<SEQS><<<sp.nch, 128, 0, stream>>>(sp, st, L, force, B, T);
-    if (multi) hmm_basis_mma_kernel<(KP >= 8 ? KP : 8), false, SEQS><<<gm, HT, 0, stream>>>(sp, st, L, hst, H, force, B, T);
+    launch(hmm_window_kernel<KP, true, SEQS>, gc, HT, 0, stream, sp, st, L, hst, H, force, B, T);
+    launch(hmm_fwd_kernel<KP, SEQS>, gc, HT, 0, stream, sp, st, L, hst, H, force, B, T);
+    launch(hmm_cs_kernel<SEQS>, sp.nch, 128, 0, stream, sp, st, L, force, B, T);
+    if (multi) launch(hmm_basis_mma_kernel<(KP >= 8 ? KP : 8), false, SEQS>, gm, HT, 0, stream, sp, st, L, hst, H, force, B, T);
     if (plan == nullptr) launch_seq<KP, false, false>(sp, st, L, hst, H, force, B, smem_seq, stream, 0, sp.nch - 1);
     else launch_seq_segs<KP, false>(sp, st, L, hst, H, force, B, smem_seq, stream, plan, segs_dev);
-    hmm_window_kernel<KP, false, SEQS><<<gc, HT, 0, stream>>>(sp, st, L, hst, H, force, B, T);
-    hmm_bwd_kernel<KP, SEQS><<<gc, HT, 0, stream>>>(sp, st, L, hst, H, force, B, T);
+    launch(hmm_window_kernel<KP, false, SEQS>, gc, HT, 0, stream, sp, st, L, hst, H, force, B, T);
+    launch(hmm_bwd_kernel<KP, SEQS>, gc, HT, 0, stream, sp, st, L, hst, H, force, B, T);
     const int nred = sp.K * sp.K + 2 + (SEQS ? sp.K : 0);
-    hmm_reduce_kernel<SEQS><<<(nred + 31) / 32, 256, 0, stream>>>(sp, st, L, hst, H, force, B, T);
+    launch(hmm_reduce_kernel<SEQS>, (nred + 31) / 32, 256, 0, stream, sp, st, L, hst, H, force, B, T);
     return check_cuda(cudaGetLastError(), "hmm scan launch");
 }
 
@@ -993,8 +993,8 @@ static int launch_emit_small_d(const void* x, int64_t n, int K, const double* st
     const size_t smem = (size_t)8 * (32 * (K | 1) + 32) * sizeof(double);
     cudaError_t e = cudaFuncSetAttribute(hmm_emit_small_kernel<D>, cudaFuncAttributeMaxDynamicSharedMemorySize, 80 * 1024);
     if (e != cudaSuccess) return check_cuda(e, "cudaFuncSetAttribute(hmm_emit_small)");
-    hmm_emit_small_kernel<D><<<(unsigned)g, 256, smem, s>>>(static_cast<const double*>(x), n, K, st, L, force, lnrho, rhohat,
-                                                           rowmax);
+    launch(hmm_emit_small_kernel<D>, (unsigned)g, 256, smem, s, static_cast<const double*>(x), n, K, st, L, force, lnrho, rhohat,
+           rowmax);
     return check_cuda(cudaGetLastError(), "hmm_emit_small launch");
 }
 
@@ -1188,11 +1188,11 @@ extern "C" int bgmm_hmm_viterbi_seqs(int64_t n, int K, const double* lnrho, cons
     }
     cudaStream_t s = (cudaStream_t)stream;
     const unsigned g = (unsigned)((n_seqs + 3) / 4);
-    if (K <= 2) hmm_viterbi_seqs_kernel<2><<<g, 128, 0, s>>>(n, K, n_seqs, seq_starts, lnrho, lnpi, lna, omega, phi, path);
-    else if (K <= 4) hmm_viterbi_seqs_kernel<4><<<g, 128, 0, s>>>(n, K, n_seqs, seq_starts, lnrho, lnpi, lna, omega, phi, path);
-    else if (K <= 8) hmm_viterbi_seqs_kernel<8><<<g, 128, 0, s>>>(n, K, n_seqs, seq_starts, lnrho, lnpi, lna, omega, phi, path);
-    else if (K <= 16) hmm_viterbi_seqs_kernel<16><<<g, 128, 0, s>>>(n, K, n_seqs, seq_starts, lnrho, lnpi, lna, omega, phi, path);
-    else hmm_viterbi_seqs_kernel<32><<<g, 128, 0, s>>>(n, K, n_seqs, seq_starts, lnrho, lnpi, lna, omega, phi, path);
+    if (K <= 2) launch(hmm_viterbi_seqs_kernel<2>, g, 128, 0, s, n, K, n_seqs, seq_starts, lnrho, lnpi, lna, omega, phi, path);
+    else if (K <= 4) launch(hmm_viterbi_seqs_kernel<4>, g, 128, 0, s, n, K, n_seqs, seq_starts, lnrho, lnpi, lna, omega, phi, path);
+    else if (K <= 8) launch(hmm_viterbi_seqs_kernel<8>, g, 128, 0, s, n, K, n_seqs, seq_starts, lnrho, lnpi, lna, omega, phi, path);
+    else if (K <= 16) launch(hmm_viterbi_seqs_kernel<16>, g, 128, 0, s, n, K, n_seqs, seq_starts, lnrho, lnpi, lna, omega, phi, path);
+    else launch(hmm_viterbi_seqs_kernel<32>, g, 128, 0, s, n, K, n_seqs, seq_starts, lnrho, lnpi, lna, omega, phi, path);
     return check_cuda(cudaGetLastError(), "viterbi_seqs launch");
 }
 
@@ -1213,7 +1213,7 @@ extern "C" int bgmm_hmm_viterbi(int64_t n, int K, const double* lnrho, const dou
     do {                                                                                                               \
         e = cudaFuncSetAttribute(hmm_viterbi_fwd_kernel<KP>, cudaFuncAttributeMaxDynamicSharedMemorySize, 160 * 1024);  \
         if (e != cudaSuccess) return check_cuda(e, "cudaFuncSetAttribute(viterbi_fwd)");                                \
-        hmm_viterbi_fwd_kernel<KP><<<1, SEQ_T, smem_f, s>>>(n, K, lnrho, lnpi, lna, omega, phi);                         \
+        launch(hmm_viterbi_fwd_kernel<KP>, 1, SEQ_T, smem_f, s, n, K, lnrho, lnpi, lna, omega, phi);                     \
     } while (0)
     if (K <= 2) BGMM_VIT(2);
     else if (K <= 4) BGMM_VIT(4);
@@ -1221,7 +1221,7 @@ extern "C" int bgmm_hmm_viterbi(int64_t n, int K, const double* lnrho, const dou
     else if (K <= 16) BGMM_VIT(16);
     else BGMM_VIT(32);
 #undef BGMM_VIT
-    hmm_viterbi_back_kernel<<<1, SEQ_T, smem_b, s>>>(n, K, omega, phi, path);
+    launch(hmm_viterbi_back_kernel, 1, SEQ_T, smem_b, s, n, K, omega, phi, path);
     return check_cuda(cudaGetLastError(), "viterbi launch");
 }
 

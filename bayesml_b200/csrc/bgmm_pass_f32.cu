@@ -491,9 +491,9 @@ int launch_pass_f32(const PassArgs& a, int K, int D, int dtype, cudaStream_t str
         const int64_t want = ((a.n + 1) / 2 + F32_THREADS - 1) / F32_THREADS;
         int64_t cap = (int64_t)sms * occ;
         if (cap > 1024) cap = 1024;
-        pass_f32x2_kernel<<<(int)(want < 1 ? 1 : (want < cap ? want : cap)), F32_THREADS, 0, stream>>>(a, L);
+        launch(pass_f32x2_kernel, (int)(want < 1 ? 1 : (want < cap ? want : cap)), F32_THREADS, 0, stream, a, L);
     }
-#define BGMM_F32_CASE(d, o) if (D == d && out == o) pass_f32_kernel<d, o><<<f32_grid<d, o>(a.n), F32_THREADS, 0, stream>>>(a, L, packed);
+#define BGMM_F32_CASE(d, o) if (D == d && out == o) launch(pass_f32_kernel<d, o>, f32_grid<d, o>(a.n), F32_THREADS, 0, stream, a, L, packed);
     BGMM_F32_CASE(1, false) BGMM_F32_CASE(1, true) BGMM_F32_CASE(2, false) BGMM_F32_CASE(2, true)
     BGMM_F32_CASE(3, false) BGMM_F32_CASE(3, true)
 #undef BGMM_F32_CASE

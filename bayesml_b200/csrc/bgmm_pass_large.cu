@@ -515,9 +515,9 @@ static int launch_large_t(const PassArgs& a, const Layout& L, int which, cudaStr
                               4 * sizeof(uint64_t) + sizeof(unsigned short) * (size_t)nchunk_e * LG_CW + 128;
         cudaError_t e = cudaFuncSetAttribute(e_large_kernel<KB, GB>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_e);
         if (e != cudaSuccess) return check_cuda(e, "cudaFuncSetAttribute(e_large)");
-        coef_pack_kernel<KB><<<nchunk_e, LG_THREADS, 0, stream>>>(a.state, L, packed, a.force, a.ignore_robust);
-        feat_table_kernel<<<(nchunk_e * LG_CW + 255) / 256, 256, 0, stream>>>(ftab, L.D, L.P, nchunk_e * LG_CW);
-        e_large_kernel<KB, GB><<<grid_e, LG_ETHREADS, smem_e, stream>>>(a, L, ews, packed, ftab);
+        launch(coef_pack_kernel<KB>, nchunk_e, LG_THREADS, 0, stream, a.state, L, packed, a.force, a.ignore_robust);
+        launch(feat_table_kernel, (nchunk_e * LG_CW + 255) / 256, 256, 0, stream, ftab, L.D, L.P, nchunk_e * LG_CW);
+        launch(e_large_kernel<KB, GB>, grid_e, LG_ETHREADS, smem_e, stream, a, L, ews, packed, ftab);
     }
     if (which & 2) {
         constexpr int RP = (8 * KB < 16) ? 16 : 8 * KB;
@@ -525,7 +525,7 @@ static int launch_large_t(const PassArgs& a, const Layout& L, int which, cudaStr
                               2 * sizeof(uint64_t) + 128;
         cudaError_t e = cudaFuncSetAttribute(m_large_kernel<KB>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_m);
         if (e != cudaSuccess) return check_cuda(e, "cudaFuncSetAttribute(m_large)");
-        m_large_kernel<KB><<<dim3(n_chunks, nsplit), LG_THREADS, smem_m, stream>>>(a, L, ews, grid_e, nsplit);
+        launch(m_large_kernel<KB>, dim3(n_chunks, nsplit), LG_THREADS, smem_m, stream, a, L, ews, grid_e, nsplit);
         launch_reduce_partials(a, L, nsplit, stream);
     }
     return check_cuda(cudaGetLastError(), "pass_large launch");
@@ -611,7 +611,7 @@ int launch_pass_batched(const void* x, int64_t n, int K, int D, const BatchDesc&
         return BGMM_ENOSUP;
     }
     const Layout Ls = make_layout(Ke, D, 1), Lm = make_layout(K, D, 1);
-    batch_gather_kernel<<<Ke, 128, 0, stream>>>(bd, sup, Ls, Lm, Kp);
+    launch(batch_gather_kernel, Ke, 128, 0, stream, bd, sup, Ls, Lm, Kp);
     PassArgs a{x, n, sup, workspace, r_scratch, nullptr, nullptr, nullptr, 0, 0};
     a.ignore_robust = 1;                                        // a flagged member is redone by its own DIRECT pass (caller)
     const int rc = launch_pass_large_part(a, Ke, D, BGMM_F64, 3, stream, Kp / 8);
@@ -619,7 +619,7 @@ int launch_pass_batched(const void* x, int64_t n, int K, int D, const BatchDesc&
     int grid_e, n_chunks, nsplit;
     large_plan(Ke, D, n, grid_e, n_chunks, nsplit);
     const double* ews = workspace + (int64_t)large_max_split(D) * Ls.stats_len;
-    batch_scatter_kernel<<<bd.R * (K + 1), 128, 0, stream>>>(bd, sup, Ls, Lm, Kp, ews, grid_e, (double)n);
+    launch(batch_scatter_kernel, bd.R * (K + 1), 128, 0, stream, bd, sup, Ls, Lm, Kp, ews, grid_e, (double)n);
     return check_cuda(cudaGetLastError(), "pass_batched launch");
 }
 

@@ -907,13 +907,13 @@ extern "C" int bgmm_hmm_small(int K, int D, double* state, double* hst, int mode
                             "cudaFuncSetAttribute(small_kernel)");
         if (rc) return rc;
     }
-    if (mode != BGMM_SMALL_STATS) hmm_trans_kernel<<<1, 256, 0, (cudaStream_t)stream>>>(state, L, hst, H, mode);
+    if (mode != BGMM_SMALL_STATS) launch(hmm_trans_kernel, 1, 256, 0, (cudaStream_t)stream, state, L, hst, H, mode);
     if (use_warp_kernel(D))
         return check_cuda(launch_small_warp(K, D, (cudaStream_t)stream, state, L, mode, max_itr, tol, nullptr,
                                             (const double*)(hst + H.vlx)), "hmm small (warp) launch");
     const int nt = D <= 16 ? 32 : (D <= 32 ? 64 : (D <= 64 ? 128 : 256));
-    small_kernel<<<K, nt, smem, (cudaStream_t)stream>>>(state, L, mode, max_itr, tol, nullptr, hst + H.vlx,
-                                                        robust_threshold());
+    launch(small_kernel, K, nt, smem, (cudaStream_t)stream, state, L, mode, max_itr, tol, nullptr, hst + H.vlx,
+           robust_threshold());
     return check_cuda(cudaGetLastError(), "hmm small launch");
 }
 

@@ -128,6 +128,6 @@ extern "C" int bgmm_tc_selftest(const float* A, const float* B, float* D, int N,
     const size_t smem = sizeof(float) * (size_t)(128 + N) * Kd + 128 + 1024;
     cudaError_t e = cudaFuncSetAttribute(tc_selftest_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     if (e != cudaSuccess) return check_cuda(e, "cudaFuncSetAttribute(tc_selftest)");
-    tc_selftest_kernel<<<1, 128, smem, (cudaStream_t)stream>>>(A, B, D, N, Kd, a_mn_major, b_mn_major);
+    launch(tc_selftest_kernel, 1, 128, smem, (cudaStream_t)stream, A, B, D, N, Kd, a_mn_major, b_mn_major);
     return check_cuda(cudaGetLastError(), "tc_selftest_kernel launch");
 }

@@ -68,11 +68,9 @@ class VBEngine:
         self.n_global = 0
         self.center = np.zeros(self.D)
         self.timing = {} if os.environ.get("BAYESML_B200_TIMING") else None
-        self.passes = 0                       # bgmm_pass calls
-        self.kernel_launches = 0              # kernels launched by this engine (pass + reduction + publish + small ...)
+        self.kernel_launches = 0              # kernels libbgmm launched for this engine's calls (_call)
         self._pending = None
         self.failed = False
-        self.small_launches = 0
         with torch.cuda.device(self.device):
             self.workspace = torch.empty(int(self.lib.bgmm_workspace_doubles(self.K, self.D)), dtype=torch.float64,
                                          device=self.device)
@@ -95,8 +93,7 @@ class VBEngine:
         base, handle = ctypes.c_void_p(), ctypes.create_string_buffer(64)
         with torch.cuda.device(self.device):
             try:
-                _lib.check(lib.bgmm_comm_alloc(lib.bgmm_comm_block_doubles(self.K, self.D), ctypes.byref(base), handle),
-                           "bgmm_comm_alloc")
+                self._call(lib.bgmm_comm_alloc, lib.bgmm_comm_block_doubles(self.K, self.D), ctypes.byref(base), handle)
             except RuntimeError:
                 ok = 0
             handles = [None] * world
@@ -149,6 +146,14 @@ class VBEngine:
 
     def phase(self, name):
         return _Phase(self, name)
+
+    def _call(self, fn, *args):
+        """One libbgmm call that returns a status code: raise RuntimeError on failure, and add the kernels the library
+        launched for it to kernel_launches."""
+        n0 = self.lib.bgmm_launch_count()
+        rc = fn(*args)
+        self.kernel_launches += self.lib.bgmm_launch_count() - n0
+        _lib.check(rc, fn.__name__)
 
     # ------------------------------------------------------------------ buffers
     def _alloc_state(self, hist_len):
@@ -218,8 +223,8 @@ class VBEngine:
             n = raw.shape[0]
             self.n_local = int(n)
             colsum = torch.zeros(D + 1, dtype=torch.float64, device=self.device)
-            _lib.check(self.lib.bgmm_colsum(raw.data_ptr(), n, D, raw_code, colsum.data_ptr(),
-                                            self.workspace.data_ptr(), self._stream()), "bgmm_colsum")
+            self._call(self.lib.bgmm_colsum, raw.data_ptr(), n, D, raw_code, colsum.data_ptr(), self.workspace.data_ptr(),
+                       self._stream())
             colsum[D] = float(n)
             if self.group is not None:
                 torch.distributed.all_reduce(colsum, group=self.group)
@@ -243,8 +248,8 @@ class VBEngine:
                 out = raw          # our own upload buffer: centre in place
             else:
                 out = torch.empty((n, D), dtype=self.x_torch_dtype, device=self.device)
-            _lib.check(self.lib.bgmm_center(raw.data_ptr(), raw_code, out.data_ptr(), self.x_code, n, D,
-                                            cview.data_ptr(), self._stream()), "bgmm_center")
+            self._call(self.lib.bgmm_center, raw.data_ptr(), raw_code, out.data_ptr(), self.x_code, n, D, cview.data_ptr(),
+                       self._stream())
             self.x = out
             self.r_dev = self.lnrho_dev = self.argmax_dev = None
             # the tcgen05 fp32-mode kernels keep r (float32, [n][K]) and their operand image in the workspace
@@ -279,10 +284,8 @@ class VBEngine:
 
     def _small(self, mode, max_itr, tol):
         comm = self.comm_desc.data_ptr() if (self.comm_desc is not None and mode != _lib.SMALL_FEATURES) else 0
-        _lib.check(self.lib.bgmm_small(self.K, self.D, self.state.data_ptr(), mode, int(max_itr), float(tol),
-                                       self.hist_len, comm, self._stream()), "bgmm_small")
-        self.small_launches += 1
-        self.kernel_launches += 1
+        self._call(self.lib.bgmm_small, self.K, self.D, self.state.data_ptr(), mode, int(max_itr), float(tol), self.hist_len,
+                   comm, self._stream())
 
     def _pass(self, r_out=None, lnrho_out=None, argmax_out=None, r_in=None, force=0, r_in_variant=_lib.PASS_SIMPLE):
         self.pass_only(r_out, lnrho_out, argmax_out, r_in, force, r_in_variant)
@@ -297,15 +300,9 @@ class VBEngine:
             if self._r_scratch is None or self._r_scratch.shape[0] != self.n_local:
                 self._r_scratch = torch.empty((self.n_local, self.K), dtype=torch.float64, device=self.device)
             r_out = self._r_scratch
-        _lib.check(self.lib.bgmm_pass(ptr(self.x), self.n_local, self.K, self.D, self.x_code, self.state.data_ptr(),
-                                      self.workspace.data_ptr(), ptr(r_out), ptr(lnrho_out), ptr(argmax_out),
-                                      ptr(r_in), self.variant if r_in is None else r_in_variant, force, 0,
-                                      self._stream()), "bgmm_pass")
-        self.passes += 1
-        resolved = self.lib.bgmm_pass_resolve(self.K, self.D, self.x_code, self.variant, int(r_in is not None))
-        self.kernel_launches += {_lib.PASS_DMMA: 2, _lib.PASS_LARGE: 5, _lib.PASS_TF32: 4}.get(resolved, 1)
-        if r_in is None and resolved != _lib.PASS_DIRECT and self.lib.bgmm_robust_threshold() < float("inf"):
-            self.kernel_launches += 1           # the conditioning guard: DIRECT kernel behind the feature-map kernel(s)
+        self._call(self.lib.bgmm_pass, ptr(self.x), self.n_local, self.K, self.D, self.x_code, self.state.data_ptr(),
+                   self.workspace.data_ptr(), ptr(r_out), ptr(lnrho_out), ptr(argmax_out), ptr(r_in),
+                   self.variant if r_in is None else r_in_variant, force, 0, self._stream())
 
     def exchange(self, force=0):
         """The per-iteration exchange of the statistics between row shards.  Peer memory: nothing to launch — bgmm_pass has
@@ -440,10 +437,8 @@ class VBEngine:
             acst = self._pview(cur, "acst", K)
             consts = torch.as_tensor(np.ascontiguousarray(np.stack([ck, hk, nuk]), dtype=np.float64)).to(self.device)
             out = torch.empty(n, dtype=torch.float64, device=self.device)
-            _lib.check(self.lib.bgmm_pred_logdensity(lnrho.data_ptr(), n, K, acst.data_ptr(), consts[0].data_ptr(),
-                                                     consts[1].data_ptr(), consts[2].data_ptr(), out.data_ptr(),
-                                                     self._stream()), "bgmm_pred_logdensity")
-            self.kernel_launches += 1
+            self._call(self.lib.bgmm_pred_logdensity, lnrho.data_ptr(), n, K, acst.data_ptr(), consts[0].data_ptr(),
+                       consts[1].data_ptr(), consts[2].data_ptr(), out.data_ptr(), self._stream())
             return out.cpu().numpy()
 
     def draw_dirichlet1(self, seed, row_offset=0):
@@ -451,9 +446,8 @@ class VBEngine:
         global row index) -> device tensor."""
         with torch.cuda.device(self.device):
             r = torch.empty((self.n_local, self.K), dtype=torch.float64, device=self.device)
-            _lib.check(self.lib.bgmm_dirichlet1(r.data_ptr(), self.n_local, self.K, int(seed) & (2 ** 64 - 1), int(row_offset),
-                                                self._stream()), "bgmm_dirichlet1")
-            self.kernel_launches += 1
+            self._call(self.lib.bgmm_dirichlet1, r.data_ptr(), self.n_local, self.K, int(seed) & (2 ** 64 - 1), int(row_offset),
+                       self._stream())
         return r
 
     def refine_smats(self):
@@ -494,12 +488,8 @@ class RestartBatch:
         R = len(members)
         ptrs = (ctypes.c_void_p * R)(*[m.state.data_ptr() for m in members])
         with torch.cuda.device(lead.device):
-            _lib.check(self.lib.bgmm_pass_batched(lead.x.data_ptr(), lead.n_local, lead.K, lead.D, R, ptrs,
-                                                  self.super_state.data_ptr(), self.workspace.data_ptr(),
-                                                  self.r_scratch.data_ptr(), lead._stream()), "bgmm_pass_batched")
-        lead.passes += 1
-        # gather + coefficient image + feature table + E + M + reduction + scatter (+ one guard launch per member)
-        lead.kernel_launches += 7 + (R if self.lib.bgmm_robust_threshold() < float("inf") else 0)
+            lead._call(self.lib.bgmm_pass_batched, lead.x.data_ptr(), lead.n_local, lead.K, lead.D, R, ptrs,
+                       self.super_state.data_ptr(), self.workspace.data_ptr(), self.r_scratch.data_ptr(), lead._stream())
 
     def step(self, members, max_itr=None, tol=None):
         """One VB iteration (:863-869) of every engine in `members`."""
@@ -584,37 +574,20 @@ class HMMEngine(VBEngine):
         self.set_params(eta, m, kappa, nu, winv)
 
     def _small(self, mode, max_itr, tol):
-        _lib.check(self.lib.bgmm_hmm_small(self.K, self.D, self.state.data_ptr(), self.hst.data_ptr(), mode, int(max_itr),
-                                           float(tol), self.hist_len, self._stream()), "bgmm_hmm_small")
-        self.small_launches += 1
-        self.kernel_launches += 1 if mode == _lib.SMALL_STATS else 2
+        self._call(self.lib.bgmm_hmm_small, self.K, self.D, self.state.data_ptr(), self.hst.data_ptr(), mode, int(max_itr),
+                   float(tol), self.hist_len, self._stream())
 
     def _pass(self, mode=_lib.HMM_FULL, force=0, beta_out=None):
         ptr = lambda t: 0 if t is None else t.data_ptr()  # noqa: E731
         if self.plan is not None:
-            _lib.check(self.lib.bgmm_hmm_pass_seqs(self.x.data_ptr(), self.n_local, self.K, self.D, self.state.data_ptr(),
-                                                   self.hst.data_ptr(), self.workspace.data_ptr(), ptr(self.scan_ws),
-                                                   ptr(self.lnrho_buf), ptr(self.alpha_buf), ptr(self.gamma_buf),
-                                                   ptr(self.cs_buf), ptr(beta_out), mode, force, self.plan.ctypes.data,
-                                                   self.plan_dev.data_ptr(), self._stream()), "bgmm_hmm_pass_seqs")
-            self.passes += 1
-            # emission (3) + per direction {window, chunk kernel} + c + reduction + statistics (2); with sequences of more
-            # than one chunk also the basis runs and the sweeps: one segmented launch for the short sequences, a
-            # two-level sweep (3 launches) for every long one
-            nshort, nlong = int(self.plan[4]), int(self.plan[5])
-            sweeps = (1 if nshort else 0) + 3 * nlong
-            multi = 2 + 2 * sweeps if nshort + nlong else 0
-            self.kernel_launches += (11 + multi) if mode == _lib.HMM_FULL else 2
+            self._call(self.lib.bgmm_hmm_pass_seqs, self.x.data_ptr(), self.n_local, self.K, self.D, self.state.data_ptr(),
+                       self.hst.data_ptr(), self.workspace.data_ptr(), ptr(self.scan_ws), ptr(self.lnrho_buf),
+                       ptr(self.alpha_buf), ptr(self.gamma_buf), ptr(self.cs_buf), ptr(beta_out), mode, force,
+                       self.plan.ctypes.data, self.plan_dev.data_ptr(), self._stream())
             return
-        _lib.check(self.lib.bgmm_hmm_pass(self.x.data_ptr(), self.n_local, self.K, self.D, self.state.data_ptr(),
-                                          self.hst.data_ptr(), self.workspace.data_ptr(), ptr(self.scan_ws),
-                                          ptr(self.lnrho_buf), ptr(self.alpha_buf), ptr(self.gamma_buf), ptr(self.cs_buf),
-                                          ptr(beta_out), mode, force, self._stream()), "bgmm_hmm_pass")
-        self.passes += 1
-        # emission (3) + per direction {basis runs (only with > 1 chunk), sweep, window, chunk kernel} + reduction +
-        # statistics (2); of the three boundary-vector kernels the device runs one branch, the others return at once
-        chunk = (max(32, -(-self.n_local // 4096)) + 7) // 8 * 8
-        self.kernel_launches += (11 + (4 if self.n_local > chunk else 2)) if mode == _lib.HMM_FULL else 2
+        self._call(self.lib.bgmm_hmm_pass, self.x.data_ptr(), self.n_local, self.K, self.D, self.state.data_ptr(),
+                   self.hst.data_ptr(), self.workspace.data_ptr(), ptr(self.scan_ws), ptr(self.lnrho_buf), ptr(self.alpha_buf),
+                   ptr(self.gamma_buf), ptr(self.cs_buf), ptr(beta_out), mode, force, self._stream())
 
     def begin(self, max_itr, tol, init=None):
         """Post-init E-step + ELBO (:1092-1101) and the first M-step.  `init` = (gamma [n][K], ms [K][K]) for the
@@ -672,25 +645,21 @@ class HMMEngine(VBEngine):
         -> (path [n] int64 numpy, omega [n][K] device tensor, phi [n][K] int32 device tensor)."""
         n, K = self.n_local, self.K
         with torch.cuda.device(self.device):
-            _lib.check(self.lib.bgmm_hmm_pass(self.x.data_ptr(), n, K, self.D, self.state.data_ptr(), self.hst.data_ptr(),
-                                              self.workspace.data_ptr(), 0, self.lnrho_buf.data_ptr(), 0, 0, 0, 0,
-                                              _lib.HMM_EMISSION_ONLY, 1, self._stream()), "bgmm_hmm_pass(emission)")
+            self._call(self.lib.bgmm_hmm_pass, self.x.data_ptr(), n, K, self.D, self.state.data_ptr(), self.hst.data_ptr(),
+                       self.workspace.data_ptr(), 0, self.lnrho_buf.data_ptr(), 0, 0, 0, 0, _lib.HMM_EMISSION_ONLY, 1,
+                       self._stream())
             lnpi = torch.as_tensor(np.ascontiguousarray(ln_pi_tilde, dtype=np.float64)).to(self.device)
             lna = torch.as_tensor(np.ascontiguousarray(ln_a_tilde, dtype=np.float64)).to(self.device)
             omega = torch.empty((n, K), dtype=torch.float64, device=self.device)
             phi = torch.empty((n, K), dtype=torch.int32, device=self.device)
             path = torch.empty(n, dtype=torch.int32, device=self.device)
             if self.plan is not None:
-                _lib.check(self.lib.bgmm_hmm_viterbi_seqs(n, K, self.lnrho_buf.data_ptr(), lnpi.data_ptr(), lna.data_ptr(),
-                                                          omega.data_ptr(), phi.data_ptr(), path.data_ptr(),
-                                                          self._seq_starts_dev().data_ptr(), self.seq_starts.size,
-                                                          self._stream()), "bgmm_hmm_viterbi_seqs")
-                self.kernel_launches += 4
+                self._call(self.lib.bgmm_hmm_viterbi_seqs, n, K, self.lnrho_buf.data_ptr(), lnpi.data_ptr(), lna.data_ptr(),
+                           omega.data_ptr(), phi.data_ptr(), path.data_ptr(), self._seq_starts_dev().data_ptr(),
+                           self.seq_starts.size, self._stream())
                 return path.cpu().numpy().astype(np.int64), omega, phi
-            _lib.check(self.lib.bgmm_hmm_viterbi(n, K, self.lnrho_buf.data_ptr(), lnpi.data_ptr(), lna.data_ptr(),
-                                                 omega.data_ptr(), phi.data_ptr(), path.data_ptr(), self._stream()),
-                       "bgmm_hmm_viterbi")
-            self.kernel_launches += 5
+            self._call(self.lib.bgmm_hmm_viterbi, n, K, self.lnrho_buf.data_ptr(), lnpi.data_ptr(), lna.data_ptr(),
+                       omega.data_ptr(), phi.data_ptr(), path.data_ptr(), self._stream())
             return path.cpu().numpy().astype(np.int64), omega, phi
 
     def final_pass(self):

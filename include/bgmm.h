@@ -33,7 +33,7 @@
 extern "C" {
 #endif
 
-#define BGMM_ABI_VERSION 4
+#define BGMM_ABI_VERSION 5
 
 /* dtype of X */
 #define BGMM_F64 0
@@ -140,6 +140,11 @@ enum {
 
 int bgmm_abi_version(void);
 const char* bgmm_last_error(void);
+/* Number of CUDA kernels libbgmm has launched from the calling host thread since the library was loaded (launches the
+ * runtime accepted; copies and memsets are not kernels).  The difference around a call is what that call launched,
+ * including kernels the device turns into no-ops (passes queued after convergence, the idle side of the conditioning
+ * guard).  A call rejected by its argument checks launches nothing. */
+int64_t bgmm_launch_count(void);
 
 /* Sizes.  offsets[BGMM_N_OFFSETS], param_offsets[BGMM_N_PARAM_OFFSETS] are HOST arrays. */
 int bgmm_layout(int K, int D, int hist_len, int64_t* offsets_host, int64_t* param_offsets_host);

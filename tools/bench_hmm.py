@@ -5,8 +5,9 @@
 
 One "step" = one VB iteration of `hiddenmarkovnormal.LearnModel.update_posterior` (_hiddenmarkovnormal.py:1104-1113):
 M-steps of q(mu, Lambda), q(pi), q(A); emission densities; forward / backward recursions; gamma, xi; statistics; ELBO +
-convergence test.  On the device: bgmm_hmm_pass + bgmm_hmm_small (14 kernels).  Synthetic sticky-chain data with
-Gaussian emissions; the sequence is larger than L2, so every iteration streams it from HBM.
+convergence test.  On the device: bgmm_hmm_pass + bgmm_hmm_small (`gpu_launches` / `steps` kernels per step, as counted
+by libbgmm).  Synthetic sticky-chain data with Gaussian emissions; the sequence is larger than L2, so every iteration
+streams it from HBM.
 
 `value` = N*K element*states per second with x resident in HBM; `e2e` = the same through the public API with a HOST
 array; `cpu_baseline` = the numpy oracle port of the reference's sequential recursions on a bounded sample.
