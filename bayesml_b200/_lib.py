@@ -9,13 +9,14 @@ _PKG_DIR = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(_PKG_DIR, "libbgmm.so")
 
 # constants mirrored from include/bgmm.h (checked against bgmm_abi_version at load time)
-ABI_VERSION = 5
+ABI_VERSION = 6
 F64, F32 = 0, 1
 PASS_AUTO, PASS_SIMPLE, PASS_DMMA, PASS_F32, PASS_LARGE, PASS_DIRECT, PASS_TF32 = 0, 1, 2, 3, 4, 5, 6
 SMALL_FEATURES, SMALL_ITERATE, SMALL_STATS = 0, 1, 2
 
 OFF_NAMES = ("center", "alpha0", "kappa0", "nu0", "m0", "w0inv", "lnb0", "lnc0", "params0", "params1", "stats",
              "ns", "xbar", "smats", "vlk", "vlterms", "vlhist", "ctrl", "total", "stats_len", "params_len", "pitch", "shift")
+STATS_ENTROPY, STATS_ROWS, STATS_FORMAT = 0, 1, 2       # tail slots of the statistics: stats[K * pitch + slot]
 POFF_NAMES = ("alpha", "kappa", "nu", "m", "winv", "w", "elnpi", "elndet", "lnb", "coef", "acst", "linv")
 CTRL_CUR, CTRL_ITER, CTRL_DONE, CTRL_CONVERGED, CTRL_TICKET, CTRL_PASS_TICKET, CTRL_ERROR, CTRL_SEQ, CTRL_ROBUST, CTRL_CRIT = range(10)
 CTRL_COMM_LO, CTRL_COMM_HI = 10, 11
@@ -60,7 +61,7 @@ def load():
     lib.bgmm_center.restype = i32
     lib.bgmm_center.argtypes = [vp, i32, vp, i32, i64, i32, vp, vp]
     lib.bgmm_pass.restype = i32
-    lib.bgmm_pass.argtypes = [vp, i64, i32, i32, i32, vp, vp, vp, vp, vp, vp, i32, i32, i32, vp]
+    lib.bgmm_pass.argtypes = [vp, i64, i32, i32, i32, vp, vp, vp, vp, vp, vp, i32, i32, vp]
     lib.bgmm_pass_batched.restype = i32
     lib.bgmm_pass_batched.argtypes = [vp, i64, i32, i32, i32, ctypes.POINTER(vp), vp, vp, vp, vp]
     lib.bgmm_batch_capacity.restype = i32
@@ -95,8 +96,6 @@ def load():
     lib.bgmm_comm_close.argtypes = [vp]
     lib.bgmm_comm_free.restype = i32
     lib.bgmm_comm_free.argtypes = [vp]
-    lib.bgmm_publish.restype = i32
-    lib.bgmm_publish.argtypes = [i32, i32, vp, vp, i32, vp]
     lib.bgmm_hmm_layout.restype = i32
     lib.bgmm_hmm_layout.argtypes = [i32, ctypes.POINTER(i64)]
     lib.bgmm_hmm_supported.restype = i32

@@ -202,7 +202,7 @@ extern "C" int bgmm_pass_batched(const void* x, int64_t n, int K, int D, int R, 
     if (g_robust_threshold < INFINITY) {
         // conditioning guard, per member: returns at once unless that member's ctrl.robust is set
         for (int i = 0; i < R && rc == 0; ++i) {
-            PassArgs a{x, n, bd.st[i], workspace, nullptr, nullptr, nullptr, nullptr, 0, 0};
+            PassArgs a{x, n, bd.st[i], workspace, nullptr, nullptr, nullptr, nullptr, 0};
             rc = launch_pass_simple(a, K, D, BGMM_F64, 1, s);
         }
     }
@@ -235,13 +235,13 @@ extern "C" int bgmm_pass_resolve(int K, int D, int dtype, int variant, int has_r
 
 extern "C" int bgmm_pass(const void* x, int64_t n, int K, int D, int dtype, double* state, double* workspace,
                          double* r_out, double* lnrho_out, int32_t* argmax_out, const double* r_in, int variant,
-                         int force, int accumulate, void* stream) {
+                         int force, void* stream) {
     if (K <= 0 || D <= 0 || n < 0 || state == nullptr || workspace == nullptr || (x == nullptr && n > 0) ||
         (dtype != BGMM_F64 && dtype != BGMM_F32)) {
         set_error("bgmm_pass: bad argument (n=%lld K=%d D=%d dtype=%d)", (long long)n, K, D, dtype);
         return BGMM_EINVAL;
     }
-    PassArgs a{x, n, state, workspace, r_out, lnrho_out, argmax_out, r_in, force & BGMM_FORCE, accumulate};
+    PassArgs a{x, n, state, workspace, r_out, lnrho_out, argmax_out, r_in, force & BGMM_FORCE};
     a.no_publish = (force & BGMM_FORCE_NO_PUBLISH) ? 1 : 0;
     cudaStream_t s = (cudaStream_t)stream;
     variant = bgmm_pass_resolve(K, D, dtype, variant, r_in != nullptr);

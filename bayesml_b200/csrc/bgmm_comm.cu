@@ -2,27 +2,15 @@
 //
 // The per-iteration collective of the row-sharded fit is an all-reduce of K*PITCH+8 doubles (41 KB at K=32, D=16) that
 // is followed immediately by bgmm_small.  Instead of an NCCL call between the two kernels, every rank PUBLISHES its
-// local statistics into an exchange block that its peers have mapped through CUDA IPC (bgmm_publish: copy + system
-// fence + a stamp written into every peer's flag array), and bgmm_small itself waits for the stamps and sums the
-// peers' blocks straight out of peer memory, in rank order — so the reduced values are bit-identical on every rank and
-// the transfer is fused into the consuming kernel (no extra launch, no ring/tree latency).
+// local statistics into an exchange block that its peers have mapped through CUDA IPC (the last CTA of every bgmm_pass's
+// reduction: copy + system fence + a stamp written into every peer's flag array, publish_stats in bgmm_common.cuh), and
+// bgmm_small itself waits for the stamps and sums the peers' blocks straight out of peer memory, in rank order — so the
+// reduced values are bit-identical on every rank and the transfer is fused into the kernels on either side (no extra
+// launch, no ring/tree latency).
 // Two exchange buffers (sequence parity) make the protocol safe without a second barrier: a rank can run at most one
 // exchange ahead of the slowest peer, because its next bgmm_small needs that peer's next stamp.
 #include "bgmm_common.cuh"
 #include <string.h>
-
-namespace bgmm {
-
-__global__ void __launch_bounds__(256) publish_kernel(double* __restrict__ st, const Layout L, const CommDesc* __restrict__ cd,
-                                                      const int force) {
-    pdl_trigger();
-    pdl_wait();
-    volatile int* ctrl = reinterpret_cast<volatile int*>(st + L.ctrl);
-    if (!force && ctrl[BGMM_CTRL_DONE]) return;
-    publish_block(st, L, cd);
-}
-
-}  // namespace bgmm
 
 using namespace bgmm;
 
@@ -59,13 +47,3 @@ extern "C" int bgmm_comm_open(const void* ipc_handle, void** ptr_out) {
 
 extern "C" int bgmm_comm_close(void* ptr) { return check_cuda(cudaIpcCloseMemHandle(ptr), "cudaIpcCloseMemHandle"); }
 extern "C" int bgmm_comm_free(void* base) { return check_cuda(cudaFree(base), "cudaFree(exchange block)"); }
-
-extern "C" int bgmm_publish(int K, int D, double* state, const void* comm_desc, int force, void* stream) {
-    if (K <= 0 || D <= 0 || state == nullptr || comm_desc == nullptr) {
-        set_error("bgmm_publish: bad argument");
-        return BGMM_EINVAL;
-    }
-    const Layout L = make_layout(K, D, 1);
-    return check_cuda(launch_pdl(publish_kernel, dim3(1), dim3(256), 0, (cudaStream_t)stream, state, L,
-                                 static_cast<const CommDesc*>(comm_desc), force), "publish_kernel launch");
-}

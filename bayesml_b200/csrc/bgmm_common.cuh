@@ -122,7 +122,7 @@ struct PassArgs {
     double* lnrho_out;
     int32_t* argmax_out;
     const double* r_in;
-    int force, accumulate;
+    int force;
     int no_publish = 0;   // 1: leave the peer-exchange block alone even if ctrl.comm is set (BGMM_FORCE_NO_PUBLISH)
     // conditioning guard (ctrl.ROBUST): 0 = feature-map kernel, returns at once when the flag is set (the DIRECT kernel
     // launched behind it does the pass); 1 = ignore the flag (given responsibilities, hidden-Markov path, forced variant)
@@ -220,14 +220,56 @@ inline cudaError_t launch_pdl(void (*kern)(KArgs...), dim3 grid, dim3 block, siz
     return launch_counted(cfg, kern, args...);
 }
 
-// Publication of freshly reduced statistics to the peers (bgmm_comm.cu), executed by the LAST CTA of a reduction after its
-// __threadfence(): copy STATS into the own exchange block, fence at system scope, stamp every peer, bump ctrl.seq.
-// `cd` comes from ctrl.comm (0: single GPU or NCCL exchange).
-__device__ __forceinline__ const CommDesc* comm_of(const volatile int* ctrl) {
+// ---- the end of a pass: hand its statistics over ----
+// Every pass leaves per-CTA partial statistics [grid][stats_len] in the workspace.  The CTA that finishes last (of the pass
+// kernel itself, or of reduce_partials_kernel behind it) sums them into state.STATS and, in a row-sharded fit, publishes
+// the result to the peers (bgmm_comm.cu), where the next bgmm_small picks it up.
+
+// Last-CTA election on ctrl.PASS_TICKET: true in every thread of the CTA that arrives last, which then sees the stores of
+// every other CTA.  That CTA resets the ticket for the next pass.
+__device__ __forceinline__ bool last_cta(volatile int* ctrl) {
+    __shared__ int is_last;
+    __threadfence();
+    __syncthreads();
+    if (threadIdx.x == 0) {
+        const int t = atomicAdd(const_cast<int*>(&ctrl[BGMM_CTRL_PASS_TICKET]), 1);
+        is_last = (t == (int)gridDim.x - 1);
+    }
+    __syncthreads();
+    if (!is_last) return false;
+    __threadfence();
+    if (threadIdx.x == 0) ctrl[BGMM_CTRL_PASS_TICKET] = 0;
+    return true;
+}
+
+// state.STATS = the sum of the gridDim.x partials in CTA order (deterministic), with the pass's row count and `format`
+// (BGMM_STATS_FORMAT: 1 = moments about state.SHIFT, 0 = about the centre) in the tail.
+__device__ __forceinline__ void sum_partials(const PassArgs& a, const Layout& L, double format) {
+    const int64_t len = L.stats_len, tail = (int64_t)L.K * L.pitch;
+    double* out = a.state + L.stats;
+    for (int64_t o = threadIdx.x; o < len; o += blockDim.x) {
+        double acc = 0.0;
+        for (int b = 0; b < (int)gridDim.x; ++b) acc += __ldcg(&a.workspace[(int64_t)b * len + o]);
+        if (o == tail + BGMM_STATS_ROWS) acc = (double)a.n;
+        if (o == tail + BGMM_STATS_FORMAT) acc = format;
+        out[o] = acc;
+    }
+}
+
+// The peer-exchange descriptor a pass publishes to: the one in ctrl.COMM unless the call set BGMM_FORCE_NO_PUBLISH.
+// nullptr: one GPU, or the caller exchanges state.STATS itself (NCCL).
+__device__ __forceinline__ const CommDesc* publish_target(const volatile int* ctrl, int no_publish) {
+    if (no_publish) return nullptr;
     const unsigned long long lo = (unsigned int)ctrl[BGMM_CTRL_COMM_LO], hi = (unsigned int)ctrl[BGMM_CTRL_COMM_HI];
     return reinterpret_cast<const CommDesc*>((hi << 32) | lo);
 }
-__device__ __forceinline__ void publish_block(double* __restrict__ st, const Layout& L, const CommDesc* cd) {
+
+// Run by the elected CTA once state.STATS holds the reduced statistics: copy them into the own exchange block, fence at
+// system scope, stamp every peer, bump ctrl.SEQ.  Nothing to do without a descriptor.
+__device__ __forceinline__ void publish_stats(double* __restrict__ st, const Layout& L, const CommDesc* cd) {
+    if (cd == nullptr) return;
+    __threadfence();
+    __syncthreads();
     volatile int* ctrl = reinterpret_cast<volatile int*>(st + L.ctrl);
     const int seq = ctrl[BGMM_CTRL_SEQ];
     const int64_t len = L.stats_len;
@@ -244,6 +286,13 @@ __device__ __forceinline__ void publish_block(double* __restrict__ st, const Lay
     }
     __syncthreads();
     if (threadIdx.x == 0) ctrl[BGMM_CTRL_SEQ] = seq + 1;
+}
+
+// The finish of a pass kernel that reduces its own partials (the simple, DIRECT and fp32 kernels).
+__device__ __forceinline__ void finish_pass(const PassArgs& a, const Layout& L, volatile int* ctrl, double format) {
+    if (!last_cta(ctrl)) return;
+    sum_partials(a, L, format);
+    publish_stats(a.state, L, publish_target(ctrl, a.no_publish));
 }
 
 // sum of `nparts` per-CTA partial statistics buffers (workspace) into state.STATS, fixed order (bgmm_pass_dmma.cu)

@@ -1321,7 +1321,7 @@ static int hmm_pass(const void* x, int64_t n, int K, int D, double* state, doubl
         const int rs = launch_emit_small(x, n, K, D, state, make_layout(K, D, 1), force, lnrho, nullptr, nullptr,
                                          (cudaStream_t)stream);
         if (rs != -1) return rs;
-        PassArgs ea{x, n, state, workspace, nullptr, lnrho, nullptr, nullptr, force, 0};
+        PassArgs ea{x, n, state, workspace, nullptr, lnrho, nullptr, nullptr, force};
         ea.ignore_robust = 1;                                    // the hidden-Markov path has no DIRECT kernel (DESIGN §2)
         ea.lnrho_only = 1;
         return launch_pass_large_part(ea, K, D, BGMM_F64, 1, (cudaStream_t)stream);
@@ -1333,7 +1333,7 @@ static int hmm_pass(const void* x, int64_t n, int K, int D, double* state, doubl
     cudaStream_t s = (cudaStream_t)stream;
     const Layout L = make_layout(K, D, 1);
     const HmmLayout H = make_hmm_layout(K);
-    PassArgs a{x, n, state, workspace, nullptr, lnrho, nullptr, nullptr, force, 0};
+    PassArgs a{x, n, state, workspace, nullptr, lnrho, nullptr, nullptr, force};
     a.ignore_robust = 1;
     int rc;
     if (mode == BGMM_HMM_FULL) {

@@ -381,7 +381,7 @@ pass_dmma_kernel(const PassArgs a, const Layout L) {
     ent = block_sum(ent, red);
     if (tid == 0) {
         double* part = a.workspace + (int64_t)blockIdx.x * len;
-        part[(int64_t)K * L.pitch] = ent;
+        part[(int64_t)K * L.pitch + BGMM_STATS_ENTROPY] = ent;
         for (int o = 1; o < 8; ++o) part[(int64_t)K * L.pitch + o] = 0.0;
     }
 }
@@ -389,20 +389,19 @@ pass_dmma_kernel(const PassArgs a, const Layout L) {
 // Cross-CTA reduction of the per-CTA partial statistics, fully parallel and in a fixed order (deterministic):
 // out[o] = sum_b ws[b][o].  A 256-thread CTA owns 32 outputs; its 8 warps each sum one slice of the partials (short
 // dependency chains, 256-byte coalesced loads) and warp 0 adds the 8 slice sums in slice order.
-// tail[1] of the statistics buffer is set to the local row count.  With a peer-exchange descriptor in ctrl.comm the last
-// CTA to finish (atomic ticket) publishes the reduced buffer to the peers (publish_block).
+// The tail of the statistics gets the local row count and format 0.  With a peer-exchange descriptor in ctrl.comm the last
+// CTA to finish publishes the reduced buffer to the peers.
 __global__ void __launch_bounds__(256) reduce_partials_kernel(const double* __restrict__ ws, const int nparts,
                                                               const int64_t len, double* __restrict__ st, const Layout L,
-                                                              const double rows, const int accumulate, const int force,
-                                                              const int ignore_robust, const int no_publish,
-                                                              const int crit_limit) {
+                                                              const double rows, const int force, const int ignore_robust,
+                                                              const int no_publish, const int crit_limit) {
     pdl_trigger();
     pdl_wait();
     volatile int* ctrl = reinterpret_cast<volatile int*>(st + L.ctrl);
     if (pass_skip(ctrl, force, ignore_robust, crit_limit)) return;
     double* __restrict__ out = st + L.stats;
-    const int64_t rows_slot = (int64_t)L.K * L.pitch + 1;
-    const CommDesc* cd = no_publish ? nullptr : comm_of(ctrl);
+    const int64_t tail = (int64_t)L.K * L.pitch;
+    const CommDesc* cd = publish_target(ctrl, no_publish);
     __shared__ double slice[8][32];
     const int lane = threadIdx.x & 31, sl = threadIdx.x >> 5;
     const int64_t o = (int64_t)blockIdx.x * 32 + lane;
@@ -424,31 +423,18 @@ __global__ void __launch_bounds__(256) reduce_partials_kernel(const double* __re
         double acc = 0.0;
 #pragma unroll
         for (int i = 0; i < 8; ++i) acc += slice[i][lane];
-        if (o == rows_slot) acc = rows;
-        if (o == rows_slot + 1) out[o] = 0.0;             // format marker: moments about the centre (feature-map kernels)
-        else out[o] = accumulate ? out[o] + acc : acc;
+        if (o == tail + BGMM_STATS_ROWS) acc = rows;
+        if (o == tail + BGMM_STATS_FORMAT) acc = 0.0;     // moments about the centre (feature-map kernels)
+        out[o] = acc;
     }
-    if (cd == nullptr) return;
-    // ---- last CTA publishes the reduced statistics to the peers ----
-    __shared__ int is_last;
-    __threadfence();
-    __syncthreads();
-    if (threadIdx.x == 0) {
-        const int t = atomicAdd(const_cast<int*>(&ctrl[BGMM_CTRL_PASS_TICKET]), 1);
-        is_last = (t == (int)gridDim.x - 1);
-    }
-    __syncthreads();
-    if (!is_last) return;
-    __threadfence();
-    if (threadIdx.x == 0) ctrl[BGMM_CTRL_PASS_TICKET] = 0;
-    publish_block(st, L, cd);
+    if (cd != nullptr && last_cta(ctrl)) publish_stats(st, L, cd);      // one GPU: no election
 }
 
 // ---- host side ----
 void launch_reduce_partials(const PassArgs& a, const Layout& L, int nparts, cudaStream_t stream) {
     const int64_t len = L.stats_len;
     launch_pdl(reduce_partials_kernel, dim3((unsigned)((len + 31) / 32)), dim3(256), 0, stream, (const double*)a.workspace,
-               nparts, len, a.state, L, (double)a.n, a.accumulate, a.force, a.ignore_robust, a.no_publish, a.crit_limit);
+               nparts, len, a.state, L, (double)a.n, a.force, a.ignore_robust, a.no_publish, a.crit_limit);
 }
 
 struct DmmaPlan {

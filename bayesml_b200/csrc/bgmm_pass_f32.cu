@@ -42,11 +42,10 @@ __device__ __forceinline__ float rcp_approx(float x) {
     return y;
 }
 
-// per-CTA partial from the per-warp float64 accumulators, then the last CTA (atomic ticket) reduces the partials in CTA
-// order and publishes them to the peers of a row-sharded fit
+// per-CTA partial from the per-warp float64 accumulators, then the finish of the pass (last CTA: sum in CTA order, publish)
 template <int P>
 __device__ __forceinline__ void f32_epilogue(const PassArgs& a, const Layout& L, volatile int* ctrl,
-                                             double (&wsum)[F32_THREADS / 32][F32_KMAX * P + 1], int& is_last) {
+                                             double (&wsum)[F32_THREADS / 32][F32_KMAX * P + 1]) {
     constexpr int NW = F32_THREADS / 32;
     const int K = L.K, tid = threadIdx.x;
     // ---- per-CTA partial (fp64, logical layout [K][pitch]) ----
@@ -63,35 +62,9 @@ __device__ __forceinline__ void f32_epilogue(const PassArgs& a, const Layout& L,
     if (tid == 0) {
         double v = 0.0;
         for (int w = 0; w < NW; ++w) v += wsum[w][F32_KMAX * P];
-        part[(int64_t)K * L.pitch] = v;
+        part[(int64_t)K * L.pitch + BGMM_STATS_ENTROPY] = v;
     }
-
-    // ---- last CTA reduces the partials in CTA order ----
-    __threadfence();
-    __syncthreads();
-    if (tid == 0) {
-        const int tk = atomicAdd(const_cast<int*>(&ctrl[BGMM_CTRL_PASS_TICKET]), 1);
-        is_last = (tk == (int)gridDim.x - 1);
-    }
-    __syncthreads();
-    if (!is_last) return;
-    __threadfence();
-    double* out = a.state + L.stats;
-    const double* ws = a.workspace;
-    for (int64_t o = tid; o < len; o += F32_THREADS) {
-        double s0 = 0.0;
-        for (int b = 0; b < (int)gridDim.x; ++b) s0 += __ldcg(&ws[(int64_t)b * len + o]);
-        if (o == (int64_t)K * L.pitch + 1) s0 = (double)a.n;
-        if (o == (int64_t)K * L.pitch + 2) { out[o] = 0.0; continue; }      // format marker: moments about the centre
-        out[o] = a.accumulate ? out[o] + s0 : s0;
-    }
-    if (tid == 0) ctrl[BGMM_CTRL_PASS_TICKET] = 0;
-    const CommDesc* cd = a.no_publish ? nullptr : comm_of(ctrl);
-    if (cd != nullptr) {                  // row-sharded fit: hand the reduced statistics to the peers (bgmm_comm.cu)
-        __threadfence();
-        __syncthreads();
-        publish_block(a.state, L, cd);
-    }
+    finish_pass(a, L, ctrl, 0.0);                 // moments about the centre
 }
 
 template <int D>
@@ -110,7 +83,6 @@ __global__ void __launch_bounds__(F32_THREADS) pass_f32_kernel(const PassArgs a,
     __shared__ F32Params<D> prm[F32_KMAX];
     __shared__ double wsum[NW][F32_KMAX * P + 1];
     __shared__ double red[40];
-    __shared__ int is_last;
     const int K = L.K, tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
     volatile int* ctrl = reinterpret_cast<volatile int*>(a.state + L.ctrl);
     if (pass_skip(ctrl, a.force, a.ignore_robust)) return;
@@ -315,7 +287,7 @@ __global__ void __launch_bounds__(F32_THREADS) pass_f32_kernel(const PassArgs a,
     flush();
     __syncthreads();
 
-    f32_epilogue<P>(a, L, ctrl, wsum, is_last);
+    f32_epilogue<P>(a, L, ctrl, wsum);
     (void)red;
 }
 
@@ -336,7 +308,6 @@ __global__ void __launch_bounds__(F32_THREADS, 2) pass_f32x2_kernel(const PassAr
     constexpr int D = 2, P = 6, NW = F32_THREADS / 32;
     __shared__ float cf[F32_KMAX][P];
     __shared__ double wsum[NW][F32_KMAX * P + 1];
-    __shared__ int is_last;
     const int K = L.K, tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
     volatile int* ctrl = reinterpret_cast<volatile int*>(a.state + L.ctrl);
     if (pass_skip(ctrl, a.force, a.ignore_robust)) return;
@@ -448,7 +419,7 @@ __global__ void __launch_bounds__(F32_THREADS, 2) pass_f32x2_kernel(const PassAr
     }
     flush();
     __syncthreads();
-    f32_epilogue<P>(a, L, ctrl, wsum, is_last);
+    f32_epilogue<P>(a, L, ctrl, wsum);
     (void)D;
 }
 

@@ -457,10 +457,10 @@ m_large_kernel(const PassArgs a, const Layout L, const double* __restrict__ ews,
     }
     if (cx == 0 && tid < 8) {
         double v = 0.0;
-        if (tid == 0 && ry == 0)
+        if (tid == BGMM_STATS_ENTROPY && ry == 0)
             for (int i = 0; i < n_ews; ++i) v += ews[(int64_t)i * 8];   // fixed order: deterministic (group 0; the other
                                                                         // groups of a batched pass are summed by batch_scatter)
-        part[(int64_t)K * L.pitch + tid] = v;
+        part[(int64_t)K * L.pitch + tid] = v;                           // the rest of the tail: 0
     }
 }
 
@@ -598,8 +598,8 @@ __global__ void __launch_bounds__(128) batch_scatter_kernel(const BatchDesc bd, 
         double v = 0.0;
         for (int i = 0; i < n_ews; ++i) v += ews[(int64_t)i * 8 + r];
         double* tail = st + Lm.stats + (int64_t)Lm.K * Lm.pitch;
-        tail[0] = v; tail[1] = rows; tail[2] = 0.0;
-        for (int o = 3; o < 8; ++o) tail[o] = 0.0;
+        tail[BGMM_STATS_ENTROPY] = v; tail[BGMM_STATS_ROWS] = rows; tail[BGMM_STATS_FORMAT] = 0.0;
+        for (int o = BGMM_STATS_FORMAT + 1; o < 8; ++o) tail[o] = 0.0;
     }
 }
 
@@ -612,7 +612,7 @@ int launch_pass_batched(const void* x, int64_t n, int K, int D, const BatchDesc&
     }
     const Layout Ls = make_layout(Ke, D, 1), Lm = make_layout(K, D, 1);
     launch(batch_gather_kernel, Ke, 128, 0, stream, bd, sup, Ls, Lm, Kp);
-    PassArgs a{x, n, sup, workspace, r_scratch, nullptr, nullptr, nullptr, 0, 0};
+    PassArgs a{x, n, sup, workspace, r_scratch, nullptr, nullptr, nullptr, 0};
     a.ignore_robust = 1;                                        // a flagged member is redone by its own DIRECT pass (caller)
     const int rc = launch_pass_large_part(a, Ke, D, BGMM_F64, 3, stream, Kp / 8);
     if (rc) return rc;

@@ -147,39 +147,8 @@ __global__ void __launch_bounds__(SIMPLE_THREADS) pass_simple_kernel(const PassA
         }
     }
     ent = block_sum(ent, scratch);
-    if (tid == 0) {
-        part[(int64_t)K * L.pitch] = ent;
-        part[(int64_t)K * L.pitch + 1] = 0.0;
-        part[(int64_t)K * L.pitch + 2] = 0.0;
-    }
-
-    // ---- last CTA reduces the per-CTA partials in CTA order (deterministic) ----
-    __shared__ int is_last;
-    __threadfence();
-    __syncthreads();
-    if (tid == 0) {
-        const int t = atomicAdd(const_cast<int*>(&ctrl[BGMM_CTRL_PASS_TICKET]), 1);
-        is_last = (t == (int)gridDim.x - 1);
-    }
-    __syncthreads();
-    if (!is_last) return;
-    __threadfence();
-    double* out = a.state + L.stats;
-    volatile const double* ws = a.workspace;
-    for (int64_t o = tid; o < len; o += SIMPLE_THREADS) {
-        double acc = 0.0;
-        for (int b = 0; b < (int)gridDim.x; ++b) acc += ws[(int64_t)b * len + o];
-        if (o == (int64_t)K * L.pitch + 1) acc = (double)a.n;
-        if (o == (int64_t)K * L.pitch + 2) acc = DIRECT ? 1.0 : 0.0;        // format marker: moments about state.SHIFT
-        out[o] = (a.accumulate && o != (int64_t)K * L.pitch + 2) ? out[o] + acc : acc;
-    }
-    if (tid == 0) ctrl[BGMM_CTRL_PASS_TICKET] = 0;
-    const CommDesc* cd = a.no_publish ? nullptr : comm_of(ctrl);
-    if (cd != nullptr) {                  // row-sharded fit: hand the reduced statistics to the peers (bgmm_comm.cu)
-        __threadfence();
-        __syncthreads();
-        publish_block(a.state, L, cd);
-    }
+    if (tid == 0) part[(int64_t)K * L.pitch + BGMM_STATS_ENTROPY] = ent;
+    finish_pass(a, L, ctrl, DIRECT ? 1.0 : 0.0);
 }
 
 static int simple_tile(int K, int D) {

@@ -839,7 +839,7 @@ pass_tf32_m_kernel(const PassArgs a, const Layout L, const float* __restrict__ r
     if (blockIdx.x == 0 && tid == 0) {
         double v = 0.0;
         for (int i = 0; i < n_ews; ++i) v += ews[i];              // fixed order: deterministic
-        part[(int64_t)K * L.pitch] = v;
+        part[(int64_t)K * L.pitch + BGMM_STATS_ENTROPY] = v;
     }
     tc::fence_before_sync();
     __syncthreads();

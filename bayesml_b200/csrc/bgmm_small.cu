@@ -80,7 +80,7 @@ __global__ void __launch_bounds__(256) small_kernel(double* __restrict__ st, con
     int world = 1;
     if (fused) {
         world = cd->world;
-        const int seq = ctrl[BGMM_CTRL_SEQ] - 1;                // the exchange published by the preceding bgmm_publish
+        const int seq = ctrl[BGMM_CTRL_SEQ] - 1;                // the exchange published by the preceding bgmm_pass
         const int64_t len = L.stats_len;
         if (tid < world) {
             const unsigned long long* flag = reinterpret_cast<const unsigned long long*>(cd->xchg[cd->rank] + 2 * len) +
@@ -109,16 +109,16 @@ __global__ void __launch_bounds__(256) small_kernel(double* __restrict__ st, con
     double crit_n = 1.0;                 // weight of this component in the conditioning criterion: min(N_k, 1)
     if (iterate || stats_only) {
         // ---- statistics of component k from the moments about the centre (feature-map kernels) or about
-        //      shift_k (DIRECT kernel; tail[2] > 0):  x_bar = shift + d_bar,  S = M2 / N - d_bar d_bar^T ----
+        //      shift_k (DIRECT kernel; format slot > 0):  x_bar = shift + d_bar,  S = M2 / N - d_bar d_bar^T ----
         const double* raw = st + L.stats + (int64_t)k * L.pitch;
         const double N = raw[0];
         crit_n = fmin(N, 1.0);
         double fmt;
         if (fused) {                                            // CTA 0 owns the tail: sum the format marker from the peers
             fmt = 0.0;
-            for (int r = 0; r < world; ++r) fmt += ld_peer(xb[r] + (int64_t)K * L.pitch + 2);
+            for (int r = 0; r < world; ++r) fmt += ld_peer(xb[r] + (int64_t)K * L.pitch + BGMM_STATS_FORMAT);
         } else {
-            fmt = st[L.stats + (int64_t)K * L.pitch + 2];
+            fmt = st[L.stats + (int64_t)K * L.pitch + BGMM_STATS_FORMAT];
         }
         const bool shifted = fmt > 0.5;
         const double* sh = st + L.shift + (int64_t)k * D;
@@ -367,7 +367,7 @@ __global__ void __launch_bounds__(256) small_kernel(double* __restrict__ st, con
         qpi += vk[j * 8 + 4]; qml += vk[j * 8 + 5]; asum += vk[j * 8 + 6];
     }
     ppi += st[L.lnc0];
-    double qz = -st[L.stats + (int64_t)K * L.pitch];                          // -sum r ln r (:704)
+    double qz = -st[L.stats + (int64_t)K * L.pitch + BGMM_STATS_ENTROPY];     // -sum r ln r (:704)
     qpi += -lgamma_ni(asum) + (asum - K) * digamma_pos(asum);                    // dirichlet entropy (:707)
     double extra = 0.0;
     if (hmm_vlx != nullptr) {      // hidden-Markov ELBO (_hiddenmarkovnormal.py:869-932): terms from hmm_trans_kernel
@@ -464,16 +464,16 @@ __global__ void __launch_bounds__(32) small_warp_kernel(double* __restrict__ st,
     double t_trs = 0.0, t_q1 = 0.0, t_q2 = 0.0, t_tr0 = 0.0;
     double kappa_c = 1.0, nu_c = 0.0, alpha_c = 1.0, elnpi_c = 0.0, elndet_c = 0.0, lnb_c = 0.0;
     if (iterate || stats_only) {
-        // ---- statistics of component k (moments about the centre, or about shift_k when tail[2] > 0) ----
+        // ---- statistics of component k (moments about the centre, or about shift_k when the format slot is > 0) ----
         const double* raw = st + L.stats + (int64_t)k * L.pitch;
         N = raw[0];
         crit_n = fmin(N, 1.0);
         double fmt;
         if (fused) {
             fmt = 0.0;
-            for (int r = 0; r < world; ++r) fmt += ld_peer(xb[r] + (int64_t)K * L.pitch + 2);
+            for (int r = 0; r < world; ++r) fmt += ld_peer(xb[r] + (int64_t)K * L.pitch + BGMM_STATS_FORMAT);
         } else {
-            fmt = st[L.stats + (int64_t)K * L.pitch + 2];
+            fmt = st[L.stats + (int64_t)K * L.pitch + BGMM_STATS_FORMAT];
         }
         const bool shifted = fmt > 0.5;
         const double* sh = st + L.shift + (int64_t)k * D;
@@ -726,7 +726,7 @@ __global__ void __launch_bounds__(32) small_warp_kernel(double* __restrict__ st,
     const double lg_asum = __shfl_sync(full, sf, 0), psi_as = __shfl_sync(full, sf, 1);
     if (lane != 0) return;
     ppi += st[L.lnc0];
-    double qz = -st[L.stats + (int64_t)K * L.pitch];                          // -sum r ln r (:704)
+    double qz = -st[L.stats + (int64_t)K * L.pitch + BGMM_STATS_ENTROPY];     // -sum r ln r (:704)
     qpi += -lg_asum + (asum - K) * psi_as;                                       // dirichlet entropy (:707)
     double extra = 0.0;
     if (hmm_vlx != nullptr) {

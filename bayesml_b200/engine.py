@@ -127,7 +127,7 @@ class VBEngine:
 
     def _write_comm_ptr(self):
         """ctrl.comm <- device address of the exchange descriptor: every bgmm_pass then publishes its statistics from the
-        last CTA of its reduction (no separate bgmm_publish launch)."""
+        last CTA of its reduction."""
         if self.comm_desc is not None:
             p = self.comm_desc.data_ptr()
             c = self.ctrl
@@ -302,7 +302,7 @@ class VBEngine:
             r_out = self._r_scratch
         self._call(self.lib.bgmm_pass, ptr(self.x), self.n_local, self.K, self.D, self.x_code, self.state.data_ptr(),
                    self.workspace.data_ptr(), ptr(r_out), ptr(lnrho_out), ptr(argmax_out), ptr(r_in),
-                   self.variant if r_in is None else r_in_variant, force, 0, self._stream())
+                   self.variant if r_in is None else r_in_variant, force, self._stream())
 
     def exchange(self, force=0):
         """The per-iteration exchange of the statistics between row shards.  Peer memory: nothing to launch — bgmm_pass has
@@ -422,7 +422,7 @@ class VBEngine:
         # False: moments about the global centre (feature-map kernels), s_mats carries an absolute error of
         # ~ eps * |x_bar_k - c|^2 (far below what the E-step's own rounding does to r, measured in tests/cond_sweep.py);
         # refine_smats() recomputes it in the two-pass centred form from the materialised r if that is ever wanted
-        out["centred"] = bool(host[self.off["stats"] + self.K * self.off["pitch"] + 2] > 0.5)
+        out["centred"] = bool(host[self.off["stats"] + self.K * self.off["pitch"] + _lib.STATS_FORMAT] > 0.5)
         return out
 
     def pred_log_density(self, ck, hk, nuk):

@@ -33,7 +33,7 @@
 extern "C" {
 #endif
 
-#define BGMM_ABI_VERSION 5
+#define BGMM_ABI_VERSION 6
 
 /* dtype of X */
 #define BGMM_F64 0
@@ -81,8 +81,7 @@ enum {
     BGMM_OFF_LNC0,           /* _ln_c_h0_alpha[1] (+pad)                                                     */
     BGMM_OFF_PARAMS0,        /* parameter set 0 (see BGMM_P_* below)                                         */
     BGMM_OFF_PARAMS1,        /* parameter set 1 (ping-pong)                                                  */
-    BGMM_OFF_STATS,          /* raw[K][PITCH] then tail[8]: tail[0] = sum_n sum_k r ln r, tail[1] = rows,
-                                tail[2] > 0: the moments are taken about state.SHIFT (DIRECT kernel), else about 0  */
+    BGMM_OFF_STATS,          /* raw[K][PITCH] then tail[8] (slots BGMM_STATS_* below)                        */
     BGMM_OFF_NS,             /* ns[K]                                                                        */
     BGMM_OFF_XBAR,           /* x_bar_vecs[K][D] (centred)                                                   */
     BGMM_OFF_SMATS,          /* s_mats[K][D][D]                                                              */
@@ -97,6 +96,13 @@ enum {
     BGMM_OFF_SHIFT,          /* shift[K][D] (centred frame): the point the DIRECT kernel takes its moments about
                                 (previous x_bar_k, or m_k before the first pass); maintained by bgmm_small        */
     BGMM_N_OFFSETS
+};
+
+/* slots of the statistics tail: state.STATS[K*PITCH + slot], written by every bgmm_pass, read by bgmm_small */
+enum {
+    BGMM_STATS_ENTROPY = 0,  /* sum_n sum_k r ln r                                                              */
+    BGMM_STATS_ROWS = 1,     /* rows the statistics were taken over                                             */
+    BGMM_STATS_FORMAT = 2    /* > 0: the moments are taken about state.SHIFT (DIRECT kernel), else about 0      */
 };
 
 /* sub-offsets inside one parameter set (written by bgmm_layout into `param_offsets`) */
@@ -126,15 +132,15 @@ enum {
     BGMM_CTRL_TICKET,     /* internal: last-CTA election for bgmm_small                             */
     BGMM_CTRL_PASS_TICKET,/* internal: last-CTA election for bgmm_pass                              */
     BGMM_CTRL_ERROR,      /* 1 -> a W^-1 was not positive definite (Cholesky failed)                */
-    BGMM_CTRL_SEQ,        /* number of peer-memory exchanges published so far (bgmm_publish)        */
+    BGMM_CTRL_SEQ,        /* number of peer-memory exchanges published so far                       */
     BGMM_CTRL_ROBUST,     /* 1 -> the current parameter set is ill-conditioned for the feature-map kernels:
                              bgmm_pass runs the DIRECT kernel (set by bgmm_small for every new parameter set)  */
     BGMM_CTRL_CRIT,       /* the conditioning criterion itself, ceil(min(crit, 2^30)), for kernels with their own limit
                              (the fp32 kernel takes the feature-map E-step up to 128)                                 */
     BGMM_CTRL_COMM_LO = 10, /* low / high 32 bits of the DEVICE address of the peer-exchange descriptor (see below), or 0.  */
     BGMM_CTRL_COMM_HI,    /* When set (by the caller, once), every bgmm_pass PUBLISHES the statistics it has just reduced
-                             (copy into the own exchange block + stamps, what bgmm_publish does) from the reduction's last
-                             CTA: no separate launch.  Suppressed per call with BGMM_FORCE_NO_PUBLISH.                 */
+                             (copy into the own exchange block + stamps) from the reduction's last CTA: no separate
+                             launch.  Suppressed per call with BGMM_FORCE_NO_PUBLISH.                                    */
     BGMM_N_CTRL = 16
 };
 
@@ -167,14 +173,13 @@ int bgmm_center(const void* x_raw, int dtype_in, void* x_out, int dtype_out, int
  *   optional (NULL inside the VB loop: r never touches HBM).
  *   r_in (optional, [n][K] float64): statistics of GIVEN responsibilities instead of the E-step
  *   (`_init_random_responsibility` :734-736); variant SIMPLE/AUTO: moments about the centre, DIRECT: about state.SHIFT
- *   (the reference's two-pass centred `s_mats`, :730-732, when SHIFT holds x_bar).  No-op when ctrl.done != 0 unless `force`.
- *   accumulate != 0: add to state.STATS instead of overwriting (row-chunked uploads). */
+ *   (the reference's two-pass centred `s_mats`, :730-732, when SHIFT holds x_bar).  No-op when ctrl.done != 0 unless `force`. */
 #define BGMM_FORCE 1            /* `force` bit 0: run although ctrl.done is set                                          */
 #define BGMM_FORCE_NO_PUBLISH 2 /* `force` bit 1: do not publish to the peer-exchange block (a pass that is not followed by
                                    a consuming bgmm_small, e.g. predictive densities of the local rows)                 */
 int bgmm_pass(const void* x, int64_t n, int K, int D, int dtype, double* state, double* workspace,
               double* r_out, double* lnrho_out, int32_t* argmax_out, const double* r_in,
-              int variant, int force, int accumulate, void* stream);
+              int variant, int force, void* stream);
 
 /* Conditioning guard of the feature-map kernels.  bgmm_small computes, for every new parameter set,
  *   crit = max_k min(N_k, 1) * (m_k - c)^T (nu_k W_k) (m_k - c)     (N_k = 1 before the first statistics exist)
@@ -270,17 +275,17 @@ int bgmm_tc_selftest(const float* A, const float* B, float* D, int N, int Kd, in
  * block  [2][stats_len] doubles | [2][BGMM_MAX_RANKS] uint64 stamps  allocated by bgmm_comm_alloc (cudaMalloc, zeroed)
  * and mapped by its peers through CUDA IPC (bgmm_comm_open on the 64-byte handle).  `comm_desc` is a DEVICE struct
  *   { int32 world; int32 rank; int64 reserved; double* xchg[BGMM_MAX_RANKS]; }   (xchg[rank] = own block)
- * built by the caller.  bgmm_publish (after bgmm_pass) copies state.STATS into the own block, fences at system scope and
- * stamps every peer; bgmm_small with comm_desc != NULL (modes ITERATE, STATS) waits for all stamps, sums the peers' blocks
- * in rank order (bit-identical result on every rank) and stores the sums back into state.STATS.  comm_desc == NULL:
- * state.STATS is used as is (single GPU, or all-reduced by the caller, e.g. ncclAllReduce). */
+ * built by the caller.  With its address in ctrl.COMM, the last CTA of every bgmm_pass's reduction copies state.STATS into
+ * the own block, fences at system scope and stamps every peer; bgmm_small with comm_desc != NULL (modes ITERATE, STATS)
+ * waits for all stamps, sums the peers' blocks in rank order (bit-identical result on every rank) and stores the sums back
+ * into state.STATS.  comm_desc == NULL: state.STATS is used as is (single GPU, or all-reduced by the caller, e.g.
+ * ncclAllReduce). */
 #define BGMM_MAX_RANKS 16
 int64_t bgmm_comm_block_doubles(int K, int D);
 int bgmm_comm_alloc(int64_t doubles, void** base_out, void* ipc_handle_out /* 64 bytes, host */);
 int bgmm_comm_open(const void* ipc_handle /* 64 bytes, host */, void** peer_ptr_out);
 int bgmm_comm_close(void* peer_ptr);
 int bgmm_comm_free(void* base);
-int bgmm_publish(int K, int D, double* state, const void* comm_desc, int force, void* stream);
 
 /* ---- hidden-Markov model with Gaussian emissions (SURVEY.md §8 f1) -----------------------------------------------
  * Replaces the VB loop body of /root/reference/bayesml/hiddenmarkovnormal/_hiddenmarkovnormal.py

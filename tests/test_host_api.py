@@ -14,11 +14,11 @@ from bayesml_b200._exceptions import CriteriaError, DataFormatError, ParameterFo
 from oracle.gmm_vb_oracle import OracleGMM
 
 
-def test_library_exports_every_declared_symbol(lib_built):
+def test_library_exports_every_symbol_the_header_declares(lib_built):
     header = open(os.path.join(ROOT, "include", "bgmm.h")).read()
     declared = set(re.findall(r"\b(bgmm_[a-z_]+)\s*\(", header))
     assert {"bgmm_pass", "bgmm_small", "bgmm_layout", "bgmm_colsum", "bgmm_center", "bgmm_workspace_doubles",
-            "bgmm_last_error", "bgmm_abi_version", "bgmm_publish", "bgmm_comm_alloc", "bgmm_comm_open", "bgmm_comm_close",
+            "bgmm_last_error", "bgmm_abi_version", "bgmm_comm_alloc", "bgmm_comm_open", "bgmm_comm_close",
             "bgmm_comm_free", "bgmm_comm_block_doubles", "bgmm_pass_supported"} <= declared
     lib = ctypes.CDLL(lib_built)
     for sym in declared:
@@ -43,15 +43,14 @@ def test_layout_is_consistent(lib_built):
         assert all(off2[k] == off[k] for k in keys[:-1])
 
 
-def test_bad_arguments_return_error_codes(lib_built):
+def test_host_entry_points_reject_bad_arguments(lib_built):
     lib = _lib.load()
     off = (ctypes.c_int64 * 32)()
     assert lib.bgmm_layout(0, 2, 4, off, off) == -1
     assert b"bgmm_layout" in lib.bgmm_last_error()
     assert lib.bgmm_small(3, 2, None, 0, 1, 0.0, 2, None, None) == -1
-    assert lib.bgmm_publish(3, 2, None, None, 0, None) == -1
     assert lib.bgmm_comm_block_doubles(32, 16) == 2 * (32 * 160 + 8) + 32
-    assert lib.bgmm_pass(None, 5, 3, 2, 0, None, None, None, None, None, None, 0, 0, 0, None) == -1
+    assert lib.bgmm_pass(None, 5, 3, 2, 0, None, None, None, None, None, None, 0, 0, None) == -1
     with pytest.raises(RuntimeError, match="bgmm"):
         _lib.check(-1, "bgmm_pass")
 

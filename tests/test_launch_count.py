@@ -24,7 +24,7 @@ def test_every_launch_goes_through_the_counted_helpers():
 def test_rejected_calls_launch_nothing(lib_built):
     lib = _lib.load()
     n0 = lib.bgmm_launch_count()
-    assert lib.bgmm_pass(None, 5, 0, 2, 0, None, None, None, None, None, None, 0, 0, 0, None) == -1          # K = 0
+    assert lib.bgmm_pass(None, 5, 0, 2, 0, None, None, None, None, None, None, 0, 0, None) == -1             # K = 0
     assert lib.bgmm_hmm_pass(None, 10, 3, 2, *([None] * 9), 0, 0, None) == -1                             # NULL buffers
     assert lib.bgmm_hmm_viterbi(10, 3, *([None] * 6), None) == -1
     assert lib.bgmm_small(3, 2, None, 0, 1, 0.0, 2, None, None) == -1
