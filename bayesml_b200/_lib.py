@@ -76,6 +76,10 @@ def load():
     lib.bgmm_hmm_gen_workspace_bytes.argtypes = [i32, i64, i64, i64]
     lib.bgmm_hmm_gen_sample.restype = i32
     lib.bgmm_hmm_gen_sample.argtypes = [vp, vp, i64, i32, i32, vp, vp, vp, vp, i64, ctypes.c_uint64, i64, vp, vp]
+    lib.bgmm_hmm_init_random_workspace_doubles.restype = i64
+    lib.bgmm_hmm_init_random_workspace_doubles.argtypes = [i32, i64]
+    lib.bgmm_hmm_init_random.restype = i32
+    lib.bgmm_hmm_init_random.argtypes = [i64, i32, ctypes.c_uint64, vp, vp, i64, vp, vp, vp, vp]
     lib.bgmm_tc_selftest.restype = i32
     lib.bgmm_tc_selftest.argtypes = [vp, vp, vp, i32, i32, i32, i32, vp]
     lib.bgmm_tf32_workspace_doubles.restype = i64

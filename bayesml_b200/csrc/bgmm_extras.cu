@@ -9,6 +9,8 @@
 //                         with numpy's PCG64 + ziggurat stream, 3.2e8 variates on the host at BASELINE config C2).  Counter-
 //                         based Philox4x32-10 keyed by (seed, global row): the draw of a row does not depend on how the rows
 //                         are sharded.  NOT the reference's random stream — an opt-in (`device_init=True`); same distribution.
+//   bgmm_hmm_init_random  the hidden-Markov `random_responsibility` initial state (gamma, sum xi, gamma at the sequence
+//                         starts) from Dirichlet(1_{K^2}) transition draws, Philox keyed by (seed, element); same opt-in.
 #include "bgmm_common.cuh"
 #include <math.h>
 
@@ -274,6 +276,167 @@ inline bool hmm_gen_ws(int K, int64_t n, int64_t n_seqs, int64_t chunk_len, HmmG
     return true;
 }
 
+// ---- hidden-Markov 'random_responsibility' initial state (bgmm_hmm_init_random) ----
+// Element i draws xt_i[j][k] (j, k < K), K^2 standard exponentials -ln u, and xi_i = xt_i / T_i with T_i the sum of all
+// K^2 entries: Dirichlet(1_{K^2}) as a K x K matrix.  Counter mapping: pair p = r * K + k (r < ceil(K / 2)) holds the
+// entries (2r, k) and (2r + 1, k); Philox4x32-10 of counter (i lo, i hi, p, HMM_INIT_TAG) under key (seed lo, seed hi)
+// gives (2r, k) from words (0, 1) and (2r + 1, k) from words (2, 3), which stay unused when 2r + 1 = K.
+// Rules (those of hiddenmarkovnormal._init_random_responsibility): gamma_i = column sums of xi_i, except at a sequence
+// start s, where gamma_s = row sums of xi_{s+1} (its sequence is longer than 1) or of xi_s (length 1); MS = sum of xi_i
+// over the elements that are not starts, G0 = sum of gamma over the starts.  n = 1: gamma_0 = row 0 of xt_0 normalised
+// by its own sum (K exponentials: Dirichlet(1_K)), MS = 0.
+// Layout: a group of KP lanes (KP = max(2, pow2_ceil(K))) per element, lane k of the group owns column k, so a warp
+// takes 32 / KP consecutive elements per step.  Every warp runs a fixed contiguous span of elements and keeps MS in KP
+// registers per lane; the per-block partials are summed in block order by hmm_init_finish_kernel.  The grid depends
+// only on (n, K), so the sums come out the same bits on every run and every GPU.  A start's xi_{s+1} is redrawn.
+constexpr uint32_t HMM_INIT_TAG = 0x484d4d49u;                   // "HMMI"
+constexpr int HMM_INIT_WARPS = 8;
+constexpr int HMM_INIT_MAX_BLOCKS = 1024;
+
+struct HmmInitGrid {
+    int KP, nblk;
+    int64_t span;                                               // elements per warp, a multiple of 32 / KP
+};
+inline bool hmm_init_grid(int K, int64_t n, HmmInitGrid& g) {
+    if (K < 1 || K > 32 || n < 1) return false;
+    g.KP = K <= 2 ? 2 : pow2_ceil(K);
+    const int64_t per = 32 / g.KP, steps = (n + per - 1) / per;
+    g.nblk = (int)min((int64_t)HMM_INIT_MAX_BLOCKS, (steps + HMM_INIT_WARPS - 1) / HMM_INIT_WARPS);
+    const int64_t warps = (int64_t)g.nblk * HMM_INIT_WARPS;
+    g.span = (steps + warps - 1) / warps * per;
+    return true;
+}
+
+// 1 / t for a positive normal t, within an ulp of the rounded quotient: the reciprocal estimate and two Newton steps,
+// without the slow-path call of the IEEE division (a call makes ptxas spill values that live across it)
+__device__ __forceinline__ double recip_pos(const double t) {
+    double r;
+    asm("rcp.approx.ftz.f64 %0, %1;" : "=d"(r) : "d"(t));
+    r = fma(r, fma(-t, r, 1.0), r);
+    return fma(r, fma(-t, r, 1.0), r);
+}
+
+template <int KP>
+__device__ __forceinline__ double group_sum(double v) {         // over the KP lanes of a group; every lane gets the sum
+#pragma unroll
+    for (int o = KP / 2; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
+    return v;
+}
+
+// Column k of xt_i into e[0..K-1] (zeros beyond K, and in lanes k >= K); returns its sum.
+template <int KP>
+__device__ __forceinline__ double init_draw(double (&e)[KP], const unsigned long long i, const int K, const int k,
+                                            const uint2 key) {
+    double col = 0.0;
+#pragma unroll
+    for (int r = 0; r < KP / 2; ++r) {
+        e[2 * r] = e[2 * r + 1] = 0.0;
+        if (2 * r < K && k < K) {
+            const uint4 v = philox4x32_10(make_uint4((uint32_t)i, (uint32_t)(i >> 32), (uint32_t)(r * K + k), HMM_INIT_TAG), key);
+            e[2 * r] = -log(uniform_open(v.x, v.y));
+            if (2 * r + 1 < K) e[2 * r + 1] = -log(uniform_open(v.z, v.w));
+        }
+    }
+#pragma unroll
+    for (int j = 0; j < KP; ++j) col += e[j];
+    return col;
+}
+
+template <int KP>
+__global__ void __launch_bounds__(HMM_INIT_WARPS * 32) hmm_init_random_kernel(const int64_t n, const int K,
+                                                                             const unsigned long long seed,
+                                                                             const int64_t* __restrict__ starts,
+                                                                             const int64_t n_seqs, const int64_t span,
+                                                                             double* __restrict__ gamma,
+                                                                             double* __restrict__ part) {
+    constexpr int G = 32 / KP;                                  // elements per warp step
+    __shared__ double red[KP * KP + KP];
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, g = lane / KP, k = lane % KP;
+    const uint2 key = make_uint2((uint32_t)seed, (uint32_t)(seed >> 32));
+    const int64_t b = min(n, ((int64_t)blockIdx.x * HMM_INIT_WARPS + warp) * span), e = min(n, b + span);
+    // starts == NULL: one sequence, start 0
+    auto start = [&](int64_t q) { return q >= n_seqs ? INT64_MAX : starts != nullptr ? starts[q] : (int64_t)0; };
+    int64_t lo = 0, hi = n_seqs;                                // p = first sequence start >= b
+    while (lo < hi) {
+        const int64_t mid = (lo + hi) >> 1;
+        if (start(mid) < b) lo = mid + 1; else hi = mid;
+    }
+    int64_t p = lo;
+    double acc[KP], g0 = 0.0;
+#pragma unroll
+    for (int j = 0; j < KP; ++j) acc[j] = 0.0;
+    for (int64_t base = b; base < e; base += G) {
+        // bit t of smask: element base + t is a sequence start (t <= G, so the start after the last element is seen)
+        const int64_t st = start(p + lane);
+        const unsigned smask = __reduce_or_sync(0xffffffffu, st <= base + G ? 1u << (int)(st - base) : 0u);
+        p += __popc(__ballot_sync(0xffffffffu, st < base + G));
+        const int64_t i = base + g;
+        const bool valid = i < e, first = valid && ((smask >> g) & 1u);
+        double ev[KP];
+        const double col = init_draw<KP>(ev, (unsigned long long)i, K, k, key);
+        double inv = recip_pos(group_sum<KP>(col));
+        if (valid && !first) {
+#pragma unroll
+            for (int j = 0; j < KP; ++j) acc[j] += ev[j] * inv;
+            if (k < K) gamma[i * K + k] = col * inv;
+        }
+        if (__any_sync(0xffffffffu, first)) {                   // warp-uniform: every lane takes part in the shuffles
+            const bool redraw = first && !(i + 1 == n || ((smask >> (g + 1)) & 1u));
+            const double col1 = redraw ? init_draw<KP>(ev, (unsigned long long)(i + 1), K, k, key) : 0.0;
+            const double t1 = group_sum<KP>(col1);
+            if (redraw) inv = recip_pos(t1);
+            double row = 0.0, row0 = 0.0;
+#pragma unroll
+            for (int j = 0; j < KP; ++j) {
+                const double s = group_sum<KP>(ev[j]);
+                if (k == j) row = s;
+                if (j == 0) row0 = s;
+            }
+            const double gm = n == 1 ? ev[0] * recip_pos(row0) : row * inv;
+            if (first && k < K) {
+                gamma[i * K + k] = gm;
+                g0 += gm;
+            }
+        }
+    }
+    // the warp's groups, then the block's warps in order
+#pragma unroll
+    for (int j = 0; j < KP; ++j)
+        for (int o = KP; o < 32; o <<= 1) acc[j] += __shfl_xor_sync(0xffffffffu, acc[j], o);
+    for (int o = KP; o < 32; o <<= 1) g0 += __shfl_xor_sync(0xffffffffu, g0, o);
+    for (int w = 0; w < HMM_INIT_WARPS; ++w) {
+        if (warp == w && lane < K) {
+#pragma unroll
+            for (int j = 0; j < KP; ++j)
+                if (j < K) red[j * K + lane] = (w == 0 ? 0.0 : red[j * K + lane]) + acc[j];
+            red[K * K + lane] = (w == 0 ? 0.0 : red[K * K + lane]) + g0;
+        }
+        __syncthreads();
+    }
+    const int len = K * K + K;
+    for (int t = threadIdx.x; t < len; t += blockDim.x) part[(int64_t)blockIdx.x * len + t] = red[t];
+}
+
+// MS, G0 = the per-block partials summed in block order; SC = 0.
+__global__ void __launch_bounds__(128) hmm_init_finish_kernel(const double* __restrict__ part, const int nblk, const int K,
+                                                              double* __restrict__ ms, double* __restrict__ g0,
+                                                              double* __restrict__ sc) {
+    const int len = K * K + K, t = blockIdx.x * 128 + threadIdx.x;
+    if (t < 8) sc[t] = 0.0;
+    if (t >= len) return;
+    double s = 0.0;
+    for (int blk = 0; blk < nblk; ++blk) s += part[(int64_t)blk * len + t];
+    if (t < K * K) ms[t] = s; else g0[t - K * K] = s;
+}
+
+template <int KP>
+int launch_hmm_init_random(const HmmInitGrid& gr, int64_t n, int K, unsigned long long seed, const int64_t* starts,
+                           int64_t n_seqs, double* gamma, double* part, cudaStream_t st) {
+    launch(hmm_init_random_kernel<KP>, (unsigned)gr.nblk, HMM_INIT_WARPS * 32, 0, st, n, K, seed, starts, n_seqs, gr.span,
+           gamma, part);
+    return check_cuda(cudaGetLastError(), "hmm_init_random_kernel launch");
+}
+
 }  // namespace bgmm
 
 using namespace bgmm;
@@ -365,6 +528,49 @@ extern "C" int bgmm_hmm_gen_sample(double* x_out, int32_t* z_out, int64_t n, int
     }
     launch(hmm_emit_kernel, (unsigned)((n + 63) / 64), 64, emit_smem, st, x_out, z_out, n, D, mu, chol, (unsigned long long)seed);
     return check_cuda(cudaGetLastError(), "hmm_emit_kernel launch");
+}
+
+extern "C" int64_t bgmm_hmm_init_random_workspace_doubles(int K, int64_t n) {
+    HmmInitGrid gr;
+    return hmm_init_grid(K, n, gr) ? (int64_t)gr.nblk * (K * K + K) : 0;
+}
+
+extern "C" int bgmm_hmm_init_random(int64_t n, int K, uint64_t seed, const int64_t* seq_starts_host,
+                                    const int64_t* seq_starts, int64_t n_seqs, double* gamma, double* hst, double* workspace,
+                                    void* stream) {
+    HmmInitGrid gr;
+    if (!hmm_init_grid(K, n, gr) || n_seqs < 1 || gamma == nullptr || hst == nullptr || workspace == nullptr ||
+        (n_seqs > 1 && (seq_starts_host == nullptr || seq_starts == nullptr || n_seqs > n))) {
+        set_error("bgmm_hmm_init_random: bad argument (n=%lld K=%d n_seqs=%lld; n >= 1, 1 <= K <= 32, 1 <= n_seqs <= n)",
+                  (long long)n, K, (long long)n_seqs);
+        return BGMM_EINVAL;
+    }
+    if (n_seqs > 1) {
+        bool ok = seq_starts_host[0] == 0;
+        for (int64_t q = 1; ok && q < n_seqs; ++q) ok = seq_starts_host[q] > seq_starts_host[q - 1] && seq_starts_host[q] < n;
+        if (!ok) {
+            set_error("bgmm_hmm_init_random: seq_starts must begin with 0, increase strictly and stay below n=%lld",
+                      (long long)n);
+            return BGMM_EINVAL;
+        }
+    } else {
+        seq_starts = nullptr;
+    }
+    cudaStream_t st = (cudaStream_t)stream;
+    const unsigned long long s = (unsigned long long)seed;
+    int rc;
+    switch (gr.KP) {
+        case 2: rc = launch_hmm_init_random<2>(gr, n, K, s, seq_starts, n_seqs, gamma, workspace, st); break;
+        case 4: rc = launch_hmm_init_random<4>(gr, n, K, s, seq_starts, n_seqs, gamma, workspace, st); break;
+        case 8: rc = launch_hmm_init_random<8>(gr, n, K, s, seq_starts, n_seqs, gamma, workspace, st); break;
+        case 16: rc = launch_hmm_init_random<16>(gr, n, K, s, seq_starts, n_seqs, gamma, workspace, st); break;
+        default: rc = launch_hmm_init_random<32>(gr, n, K, s, seq_starts, n_seqs, gamma, workspace, st); break;
+    }
+    if (rc) return rc;
+    const HmmLayout H = make_hmm_layout(K);
+    launch(hmm_init_finish_kernel, (unsigned)((K * K + K + 127) / 128), 128, 0, st, (const double*)workspace, gr.nblk, K,
+           hst + H.ms, hst + H.g0, hst + H.sc);
+    return check_cuda(cudaGetLastError(), "hmm_init_finish_kernel launch");
 }
 
 extern "C" int bgmm_pred_logdensity(const double* lnrho, int64_t n, int K, const double* acst, const double* ck,

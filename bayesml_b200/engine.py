@@ -589,20 +589,40 @@ class HMMEngine(VBEngine):
                    self.hst.data_ptr(), self.workspace.data_ptr(), ptr(self.scan_ws), ptr(self.lnrho_buf), ptr(self.alpha_buf),
                    ptr(self.gamma_buf), ptr(self.cs_buf), ptr(beta_out), mode, force, self._stream())
 
+    def draw_random_init(self, seed):
+        """The 'random_responsibility' initial state drawn on the device (bgmm_hmm_init_random, Philox keyed by `seed`
+        and the element index): gamma into gamma_buf, sum xi into hst.MS, gamma summed over the sequence starts into
+        hst.G0, hst.SC zeroed.  Over the sequences of set_sequences when it was given some."""
+        n, K = self.n_local, self.K
+        with torch.cuda.device(self.device):
+            ws = torch.empty(int(self.lib.bgmm_hmm_init_random_workspace_doubles(K, n)), dtype=torch.float64,
+                             device=self.device)
+            starts_host = starts_dev = None
+            n_seqs = 1
+            if self.plan is not None:
+                starts_host, starts_dev = self.seq_starts.ctypes.data, self._seq_starts_dev().data_ptr()
+                n_seqs = self.seq_starts.size
+            self._call(self.lib.bgmm_hmm_init_random, n, K, int(seed) & (2 ** 64 - 1), starts_host, starts_dev, n_seqs,
+                       self.gamma_buf.data_ptr(), self.hst.data_ptr(), ws.data_ptr(), self._stream())
+
     def begin(self, max_itr, tol, init=None):
-        """Post-init E-step + ELBO (:1092-1101) and the first M-step.  `init` = (gamma [n][K], ms [K][K]) for the
-        'random_responsibility' initialisation (:944-952): the statistics of the given gamma / xi, with ln rho = 0
-        and c = 1 as `_init_fb_params` (:934-942) leaves them."""
+        """Post-init E-step + ELBO (:1092-1101) and the first M-step.  `init` for the 'random_responsibility'
+        initialisation (:944-952): (gamma [n][K], ms [K][K]) drawn on the host, or an int, the seed of the device draw
+        (draw_random_init); then the statistics of that gamma / xi, with ln rho = 0 and c = 1 as `_init_fb_params`
+        (:934-942) leaves them."""
         self._max_itr, self._tol, self._launched = int(max_itr), float(tol), 0
         with torch.cuda.device(self.device):
             self._alloc_state(self._max_itr + 1)
             if init is not None:
-                gamma, ms = init
-                self.gamma_buf.copy_(torch.as_tensor(np.ascontiguousarray(gamma, dtype=np.float64)))
-                self._put(self._hview("ms", self.K * self.K), ms)
-                g0 = gamma[0] if self.seq_starts is None else gamma[self.seq_starts].sum(axis=0)
-                self._put(self._hview("g0", self.K), g0)
-                self._hview("sc", 8).zero_()
+                if isinstance(init, int):
+                    self.draw_random_init(init)
+                else:
+                    gamma, ms = init
+                    self.gamma_buf.copy_(torch.as_tensor(np.ascontiguousarray(gamma, dtype=np.float64)))
+                    self._put(self._hview("ms", self.K * self.K), ms)
+                    g0 = gamma[0] if self.seq_starts is None else gamma[self.seq_starts].sum(axis=0)
+                    self._put(self._hview("g0", self.K), g0)
+                    self._hview("sc", 8).zero_()
                 self._pass(mode=_lib.HMM_STATS_FROM_GAMMA, force=1)
             else:
                 self._pass()

@@ -26,8 +26,10 @@ loop with `self.rng`; `gen_sample(n, device="cuda:i")` draws the same distributi
 the chain sampled exactly by composing per-element transition maps over chunks, counter-based Philox, NOT numpy's
 stream; c_num_classes <= 32 and c_degree <= 256 there, no CPU fallback).
 
-Additive, defaulted options (they do not exist in the reference): `device`, `lengths` (of `LearnModel.update_posterior`,
-`LearnModel.estimate_latent_vars` and `GenModel.gen_sample`), `as_numpy` (of `GenModel.gen_sample`).
+Additive, defaulted options (they do not exist in the reference): `device`, `device_init` (of `LearnModel`: draw the
+'random_responsibility' initial state on the device, bgmm_hmm_init_random: same distribution, NOT numpy's random
+stream), `lengths` (of `LearnModel.update_posterior`, `LearnModel.estimate_latent_vars` and `GenModel.gen_sample`),
+`as_numpy` (of `GenModel.gen_sample`).
 """
 import warnings
 
@@ -298,10 +300,13 @@ class LearnModel(base.Posterior, base.PredictiveMixin):
     seed : {None, int}
         seed of `numpy.random.default_rng` used by the initialisations
     device : optional (extension) CUDA device of the fit
+    device_init : bool, optional (extension, default False) draw the 'random_responsibility' initial state on the
+        device: one `self.rng.integers` value per restart seeds a counter-based generator (bgmm_hmm_init_random).  The
+        numbers differ from numpy's; the distribution and the rules of `_init_random_responsibility` are the same
     """
 
     def __init__(self, c_num_classes, c_degree, *, h0_eta_vec=None, h0_zeta_vecs=None, h0_m_vecs=None, h0_kappas=None,
-                 h0_nus=None, h0_w_mats=None, seed=None, device=None):
+                 h0_nus=None, h0_w_mats=None, seed=None, device=None, device_init=False):
         self.c_degree = _check.pos_int(c_degree, 'c_degree', ParameterFormatError)
         self.c_num_classes = _check.pos_int(c_num_classes, 'c_num_classes', ParameterFormatError)
         self.rng = np.random.default_rng(seed)
@@ -313,6 +318,7 @@ class LearnModel(base.Posterior, base.PredictiveMixin):
                 f"bayesml_b200.hiddenmarkovnormal supports c_num_classes <= {MAX_NUM_CLASSES} and c_degree <= {MAX_DEGREE} "
                 f"(got {K}, {D}); there is no CPU fallback")
         self._device = device
+        self._device_init = bool(device_init)
         self._engine_obj = None
 
         # prior hyperparameters and their constants (:531-543)
@@ -603,7 +609,12 @@ class LearnModel(base.Posterior, base.PredictiveMixin):
         Several sequences (`starts`, their first rows): the same single draw `rng.dirichlet(np.ones(K**2), n)`; every
         row gets gamma = xi.sum(axis=1), then at every sequence start s, gamma_s = xi_{s+1}.sum(axis=1) (row sums of the
         K x K matrix) when that sequence is longer than 1, or the row sums of its own drawn xi_s for a sequence of
-        length 1; then xi_s = 0.  With one sequence this is the reference's rule."""
+        length 1; then xi_s = 0.  With one sequence this is the reference's rule.
+
+        `device_init=True`: -> one int from `self.rng`, the seed with which the engine draws the same rules on the device
+        (bgmm_hmm_init_random) when the restart runs; nothing n-sized is made on the host."""
+        if self._device_init:
+            return int(self.rng.integers(0, 2 ** 63 - 1))
         K = self.c_num_classes
         gamma = np.ones([n, K]) / K
         xi_sum = np.zeros([K, K])
@@ -658,7 +669,9 @@ class LearnModel(base.Posterior, base.PredictiveMixin):
 
         Nothing else consumes `self.rng` between the restarts (:1087-1100), so all initial states are drawn first (the
         same random stream as the reference's sequential loop) while x is uploaded; the restarts then run one after the
-        other on the device and the reference's selection rule (:1114) and progress text are applied in order.
+        other on the device and the reference's selection rule (:1114) and progress text are applied in order.  With
+        `device_init=True` a 'random_responsibility' restart's initial state is kept as its seed and drawn on the device
+        when the restart runs.
         """
         x = self._check_x(x)
         starts = self._seq_starts(lengths, x.shape[0])

@@ -263,6 +263,25 @@ int64_t bgmm_hmm_gen_workspace_bytes(int K, int64_t n, int64_t n_seqs, int64_t c
 int bgmm_hmm_gen_sample(double* x_out, int32_t* z_out, int64_t n, int K, int D, const double* cdf, const double* mu,
                         const double* chol, const int64_t* seq_starts, int64_t n_seqs, uint64_t seed, int64_t chunk_len,
                         void* workspace, void* stream);
+/* bgmm_hmm_init_random: the 'random_responsibility' initial state of `hiddenmarkovnormal.LearnModel` (`_init_random_
+ *   responsibility`) drawn on the device, ready for bgmm_hmm_pass(_seqs) in mode BGMM_HMM_STATS_FROM_GAMMA: gamma[n][K],
+ *   hst.MS = sum of xi_i over the elements that are not sequence starts, hst.G0 = gamma summed over the sequence starts,
+ *   hst.SC = 0 (hst: the bgmm_hmm_layout block).  Same distribution as the host rule, NOT numpy's random stream.
+ *   Element i draws xt_i[j][k] (j, k < K) as K^2 standard exponentials -ln u, and xi_i = xt_i / (sum of its K^2 entries),
+ *   i.e. Dirichlet(1_{K^2}).  u comes from Philox4x32-10 keyed by `seed` (key = seed low, high 32 bits) at counter
+ *   (i low, i high, p, 0x484d4d49): pair p = r * K + k (r < ceil(K/2)) gives entry (2r, k) from words 0, 1 and entry
+ *   (2r + 1, k) from words 2, 3 (unused when 2r + 1 = K), u = ((w_hi << 32 | w_lo) >> 11) + 0.5) / 2^53 as in
+ *   bgmm_dirichlet1.  An element's draw does not depend on how the rows are split into sequences.
+ *   Rules: gamma_i = column sums sum_j xi_i[j][.], except at every sequence start s: gamma_s = row sums sum_k xi_{s+1}[.][k]
+ *   when its sequence is longer than 1, else the row sums of xi_s.  One sequence of n = 1: gamma_0 = row 0 of xt_0 divided
+ *   by its sum (Dirichlet(1_K)), MS = 0.
+ *   seq_starts[n_seqs] (device) and seq_starts_host[n_seqs] (the same values on the host; the checks read it): first rows
+ *   of the sequences, starting with 0, strictly increasing, below n; n_seqs = 1 (pointers ignored, may be NULL) for one
+ *   sequence.  K <= 32.  MS and G0 are summed in an order fixed by (n, K): a re-run gives the same bits.
+ *   workspace: bgmm_hmm_init_random_workspace_doubles(K, n) doubles (0 for a bad argument). */
+int64_t bgmm_hmm_init_random_workspace_doubles(int K, int64_t n);
+int bgmm_hmm_init_random(int64_t n, int K, uint64_t seed, const int64_t* seq_starts_host, const int64_t* seq_starts,
+                         int64_t n_seqs, double* gamma, double* hst, double* workspace, void* stream);
 
 /* ---- 5th-generation tensor cores (fp32 mode) ----
  * bgmm_tc_selftest: D[128][N] = A[128][Kd] . B[N][Kd]^T with tcgen05.mma kind::tf32 (operands staged in shared memory in the
