@@ -22,7 +22,10 @@ def _data(n, d, k, seed):
     return mu[z] + np.einsum("nij,nj->ni", chol[z], rng.normal(size=(n, d)))
 
 
-@pytest.mark.parametrize("shape", [(7001, 32, 16, 4), (5000, 24, 5, 3), (4000, 40, 8, 8), (3000, 20, 27, 2)])
+# (n, D, K, R); the last two: e_large_kernel<2, 1> (R = 2 restarts of K <= 8: num_init = 2, or a remainder batch) and
+# e_large_kernel<4, 2> (R = 2, K 9-16)
+@pytest.mark.parametrize("shape", [(7001, 32, 16, 4), (5000, 24, 5, 3), (4000, 40, 8, 8), (3000, 20, 27, 2), (5000, 24, 5, 2),
+                                   (5000, 20, 16, 2)])
 def test_batched_pass_equals_member_passes(shape):
     import torch
     from bayesml_b200 import _lib, gaussianmixture

@@ -123,7 +123,14 @@ def test_update_posterior_end_to_end(name, lib_built):
         assert _close(model.ms, g["latent_ms_after"], rtol=1e-8)
 
 
-@pytest.mark.parametrize("shape", [(20000, 4, 5, 3), (9000, 16, 32, 2), (50000, 3, 17, 2), (3000, 40, 9, 2), (777, 2, 1, 3)])
+@pytest.mark.parametrize("shape", [(20000, 4, 5, 3), (9000, 16, 32, 2), (50000, 3, 17, 2), (3000, 40, 9, 2), (777, 2, 1, 3),
+                                   # the limits K = 32 and D = 128 (bgmm_hmm_small's 256-thread block kernel with more than 48 KiB
+                                   # of shared memory); D = 64 and 33: the last and first D of its 128-thread block kernel.  Enough
+                                   # rows that the reference is defined: its subsampling initialisation takes each covariance from
+                                   # sqrt(n) rows and it evaluates rho = exp(ln rho) unshifted, so with too few rows some element
+                                   # has every component below exp(-745) and its forward recursion is NaN (at (3000, 128, 32),
+                                   # (20000, 128, 32) and (4000, 64, 5)).
+                                   (40000, 128, 32, 2), (6000, 64, 5, 2), (6000, 33, 17, 2)])
 def test_against_oracle_larger_shapes(shape, lib_built):
     """Seeded sticky-chain data at sizes the oracle finishes in seconds; many chunks, K not a power of two."""
     from bayesml_b200.engine import HMMEngine

@@ -208,7 +208,12 @@ def test_sequential_update_wrappers():
 
 
 @pytest.mark.parametrize("variant", ["simple", "auto", "large"])
-@pytest.mark.parametrize("shape", [(20000, 16, 32), (50000, 2, 8), (5000, 32, 16), (3000, 7, 5), (4099, 16, 13), (20000, 40, 12)])
+# D = 33 and 65: the first D of bgmm_small's 128- and 256-thread block kernel; D = 17 (K 9-16) and D = 13 (K 17-32): the
+# 3-stage Phi ring and SP = 128 blocks of the fused DMMA kernel, through whole fits.  D = 65 with 12000 rows: at 4000 the
+# fit is ill-determined at this bar (the oracle against itself, X perturbed by 1e-15 relative, moves W^-1 by up to 1.7e-7
+# and r by up to 3e-6 after 6 iterations); at 12000 that spread is 1.5e-12
+@pytest.mark.parametrize("shape", [(20000, 16, 32), (50000, 2, 8), (5000, 32, 16), (3000, 7, 5), (4099, 16, 13), (20000, 40, 12),
+                                   (6000, 33, 4), (12000, 65, 3), (9000, 17, 12), (9000, 13, 20)])
 def test_larger_shapes_against_oracle_and_elbo_monotone(shape, variant, monkeypatch):
     """Seeded synthetic mixtures at sizes the oracle finishes in seconds: trajectory parity from identical init, and
     the reference's own stated test criterion — the ELBO never decreases (doc/devdoc/vb_method.md:184-194)."""
@@ -285,14 +290,20 @@ def test_fp32_mode_against_fp64_oracle(shape, packed, monkeypatch):
     assert clear.mean() > 0.99
 
 
-@pytest.mark.parametrize("variant", ["auto", "simple"])
-def test_high_dimension_shape(variant, monkeypatch):
+@pytest.mark.parametrize("shape,variant", [pytest.param((3000, 128, 64), v, id=v) for v in ("auto", "simple")] +
+                         [pytest.param((n, d, k), v, id=f"d{d}-k{k}-{v}") for n, d, k in [(2000, 160, 4), (2000, 144, 5)]
+                          for v in ("auto", "simple", "direct")])
+def test_high_dimension_shape(shape, variant, monkeypatch):
     """BASELINE config C4's shape class (D=128, K=64) at a size the oracle finishes in seconds: exercises the
-    per-component kernel with a 128x128 Cholesky in shared memory and the large-regime (auto) / generic pass kernels."""
+    per-component kernel with a 128x128 Cholesky in shared memory and the large-regime (auto) / generic pass kernels.
+    Above D = 128 (up to MAX_DEGREE = 160) only the SIMPLE and DIRECT pass kernels exist (auto resolves to SIMPLE) and
+    bgmm_small runs 256 threads with up to 208 KiB of shared memory.  D = 144 with K = 5: with K = 3 two components split
+    one cluster and the fit is ill-determined at the 1e-9 bar (the oracle against itself, X perturbed by 1e-15 relative,
+    differs by up to 1.2e-6 in W^-1 after 3 iterations); with K = 5 that spread is below 7e-10."""
     monkeypatch.setenv("BAYESML_B200_PASS_VARIANT", variant)
     from bayesml_b200 import gaussianmixture
     from oracle.gmm_vb_oracle import OracleGMM, fit
-    n, d, k = 3000, 128, 64
+    n, d, k = shape
     rng = np.random.default_rng(9)
     x = rng.normal(size=(n, d)) + 3.0 * rng.normal(size=(k, d))[rng.integers(0, k, size=n)]
     m = gaussianmixture.LearnModel(k, d, seed=1)
@@ -302,7 +313,7 @@ def test_high_dimension_shape(variant, monkeypatch):
         m.update_posterior(x, max_itr=3, num_init=1, tolerance=0.0)
     fit(o, x, max_itr=3, num_init=1, tolerance=0.0)
     _close(m.vl, o.vl, what="vl")
-    for f in ("hn_alpha_vec", "hn_m_vecs", "hn_nus", "hn_w_mats_inv", "ns", "x_bar_vecs"):
+    for f in ("hn_alpha_vec", "hn_m_vecs", "hn_kappas", "hn_nus", "hn_w_mats_inv", "ns", "x_bar_vecs"):
         _close(getattr(m, f), getattr(o, f), what=f)
     assert np.array_equal(np.argmax(m.r_vecs, axis=1), np.argmax(o.r_vecs, axis=1))
 

@@ -78,6 +78,9 @@ def test_constructor_and_validation():
         gaussianmixture.LearnModel(3, 2, h0_w_mats=np.array([[1.0, 2.0], [2.0, 1.0]]))  # not positive definite
     with pytest.raises(ParameterFormatError):
         gaussianmixture.LearnModel(3, 2, h0_alpha_vec=np.array([1.0, -1.0, 1.0]))
+    assert gaussianmixture.LearnModel(2, gaussianmixture.MAX_DEGREE).c_degree == 160
+    with pytest.raises(ParameterFormatError, match="c_degree <= 160"):
+        gaussianmixture.LearnModel(2, 161)                                         # bgmm_small's D x D in shared memory
     with pytest.raises(DataFormatError):
         m.update_posterior(np.zeros((5, 3)))
     with pytest.raises(DataFormatError):
