@@ -85,6 +85,19 @@ __device__ __forceinline__ double block_sum(double v, double* scratch) {
     return scratch[32];
 }
 
+// Block-wide max (fmax, so the order does not matter); result valid in every thread.  `scratch` as for block_sum.
+__device__ __forceinline__ double block_max(double v, double* scratch) {
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, nwarp = (blockDim.x + 31) >> 5;
+    for (int o = 16; o > 0; o >>= 1) v = fmax(v, __shfl_xor_sync(0xffffffffu, v, o));
+    __syncthreads();  // protect scratch from a previous call
+    if (lane == 0) scratch[warp] = v;
+    __syncthreads();
+    v = scratch[0];
+    for (int w = 1; w < nwarp; ++w) v = fmax(v, scratch[w]);
+    __syncthreads();
+    return v;
+}
+
 // Device-resident descriptor of the peer-memory exchange (bgmm_comm.cu); mirrors the layout documented in bgmm.h.
 struct CommDesc {
     int world, rank;
